@@ -1221,6 +1221,23 @@ static cudaError_t ensure_dyn_smem(const void* func, size_t bytes) {
     if (e == cudaSuccess) g_smem_done.emplace_back(dev, func);
     return e;
 }
+// grid of a persistent kernel: as many CTAs as fit on every SM (at most cta_cap per SM when cta_cap > 0), at most one per item
+template <typename Kernel>
+static int persistent_grid(Kernel kern, int nt, size_t smem, int cta_cap, long long n_items, const char* name, unsigned& grid) {
+    IDL_CUDA_CHECK(ensure_dyn_smem((const void*)kern, smem));
+    int per_sm = 0;
+    IDL_CUDA_CHECK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, nt, smem));
+    if (per_sm < 1) return set_error(IDL_ECUDA, "%s kernel does not fit on an SM", name);
+    if (cta_cap > 0 && per_sm > cta_cap) per_sm = cta_cap;   // the caller wants room left on every SM (a concurrent stream)
+    const long long g = (long long)sm_count() * per_sm;
+    grid = (unsigned)(g < n_items ? g : n_items);   // (callers return early when there are no items)
+    return IDL_OK;
+}
+// grid of a 256-thread grid-stride elementwise kernel over n elements: one thread per element, at most 16 CTAs per SM
+static unsigned elementwise_grid(long long n) {
+    const long long grid = (n + 255) / 256, cap = (long long)sm_count() * 16;
+    return (unsigned)(grid < cap ? grid : cap);
+}
 
 // ---------------------------------------------------------------------------------------
 // K6: index maps of a count matrix (SURVEY §8f rank 4): FCGR order (kmers.pyx:53-123),
@@ -1297,46 +1314,68 @@ constexpr size_t WS_RSCALE = WS_GTAB + sizeof(uint32_t) * RNG_BLOCK * MAX_TABS;
 constexpr size_t WS_PROF = WS_RSCALE + sizeof(float) * 4096;
 constexpr size_t WS_TOTAL = WS_PROF + 8 * 16;  // 16 phase counters (development builds)
 
-template <int K, int NT, int OUT>
-static int launch_profiles(const ProfParams& p, const Plan& plan, cudaStream_t st, int* grid_out = nullptr) {
+// the instantiation of a kernel template for an output kind (nullptr for an unknown kind)
+template <typename Kernel>
+static Kernel kernel_for_out(int out_kind, Kernel stats, Kernel counts_i32, Kernel freq_f32, Kernel std_f32, Kernel freq_f64) {
+    static_assert(IDL_OUT_COUNTS_I32 == 0 && IDL_OUT_FREQ_F32 == 1 && IDL_OUT_STD_F32 == 2 && IDL_OUT_FREQ_F64 == 3 && OUT_STATS == 4, "by_kind order");
+    const Kernel by_kind[] = {counts_i32, freq_f32, std_f32, freq_f64, stats};
+    return out_kind >= 0 && out_kind <= OUT_STATS ? by_kind[out_kind] : nullptr;
+}
+
+template <int K, int NT>
+static int launch_profiles(const ProfParams& p, const Plan& plan, int out_kind, cudaStream_t st, int* grid_out) {
+    const auto kern = kernel_for_out(out_kind, profiles_kernel<K, NT, OUT_STATS>, profiles_kernel<K, NT, IDL_OUT_COUNTS_I32>, profiles_kernel<K, NT, IDL_OUT_FREQ_F32>,
+                                     profiles_kernel<K, NT, IDL_OUT_STD_F32>, profiles_kernel<K, NT, IDL_OUT_FREQ_F64>);
+    if (!kern) return set_error(IDL_EINVAL, "unknown out_kind%s %lld", "", out_kind);
     const size_t smem = sizeof(ProfSmem<K, NT>);
-    auto kern = profiles_kernel<K, NT, OUT>;
-    IDL_CUDA_CHECK(ensure_dyn_smem((const void*)kern, smem));
-    int per_sm = 0;
-    IDL_CUDA_CHECK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, NT, smem));
-    if (per_sm < 1) return set_error(IDL_ECUDA, "profiles kernel does not fit on an SM%s", "");
-    if (p.cta_cap > 0 && per_sm > p.cta_cap) per_sm = p.cta_cap;   // the caller wants room left on every SM (a concurrent stream)
-    long long grid = (long long)sm_count() * per_sm;
-    if (grid > p.n_items) grid = p.n_items;
-    if (grid < 1) grid = 1;
+    unsigned grid = 0;
+    if (const int rc = persistent_grid(kern, NT, smem, p.cta_cap, p.n_items, "profiles", grid); rc != IDL_OK) return rc;
     if (grid_out) *grid_out = (int)grid;
-    kern<<<(unsigned)grid, NT, smem, st>>>(p, plan); note_launch();
+    kern<<<grid, NT, smem, st>>>(p, plan); note_launch();
     IDL_CUDA_CHECK(cudaGetLastError());
     return IDL_OK;
 }
 
-template <int K, int NT>
-static int dispatch_out(const ProfParams& p, const Plan& plan, int out_kind, cudaStream_t st, int* grid_out = nullptr) {
-    switch (out_kind) {
-        case OUT_STATS: return launch_profiles<K, NT, OUT_STATS>(p, plan, st, grid_out);
-        case IDL_OUT_COUNTS_I32: return launch_profiles<K, NT, IDL_OUT_COUNTS_I32>(p, plan, st);
-        case IDL_OUT_FREQ_F32: return launch_profiles<K, NT, IDL_OUT_FREQ_F32>(p, plan, st);
-        case IDL_OUT_STD_F32: return launch_profiles<K, NT, IDL_OUT_STD_F32>(p, plan, st);
-        case IDL_OUT_FREQ_F64: return launch_profiles<K, NT, IDL_OUT_FREQ_F64>(p, plan, st);
-    }
-    return set_error(IDL_EINVAL, "unknown out_kind%s %lld", "", out_kind);
-}
-
 static int dispatch_k(const ProfParams& p, const Plan& plan, int k, int out_kind, cudaStream_t st, int* grid_out = nullptr) {
     switch (k) {
-        case 1: return dispatch_out<1, 64>(p, plan, out_kind, st, grid_out);
-        case 2: return dispatch_out<2, 64>(p, plan, out_kind, st, grid_out);
-        case 3: return dispatch_out<3, 64>(p, plan, out_kind, st, grid_out);
-        case 4: return dispatch_out<4, 128>(p, plan, out_kind, st, grid_out);
-        case 5: return dispatch_out<5, 256>(p, plan, out_kind, st, grid_out);
-        case 6: return dispatch_out<6, 512>(p, plan, out_kind, st, grid_out);
+        case 1: return launch_profiles<1, 64>(p, plan, out_kind, st, grid_out);
+        case 2: return launch_profiles<2, 64>(p, plan, out_kind, st, grid_out);
+        case 3: return launch_profiles<3, 64>(p, plan, out_kind, st, grid_out);
+        case 4: return launch_profiles<4, 128>(p, plan, out_kind, st, grid_out);
+        case 5: return launch_profiles<5, 256>(p, plan, out_kind, st, grid_out);
+        case 6: return launch_profiles<6, 512>(p, plan, out_kind, st, grid_out);
     }
     return set_error(IDL_EUNSUPPORTED, "idl_profiles: unsupported k%s", "");
+}
+
+// ---- one profile request, as the entry points receive it (what an entry point does not take stays zero) ----
+struct ProfCall {
+    const uint32_t* codes; const uint32_t* nmask; const int64_t* chunk_off; const int32_t* len; int64_t n_seqs_total;
+    const int32_t* sidx; int64_t n_items, seq_id0; int k; const idl_variant* variants; int n_variants; const int32_t* sel; int S;
+    uint64_t seed; const int64_t* edit_off; const uint32_t* edits; int out_kind; void* out; const int64_t* out_off; int64_t out_stride;
+    int pseudocount, accumulate;      // accumulate: bit 0 adds to the counts, bits 8..15 cap the generic kernel's CTAs per SM
+    const float* mean; const float* scale; int32_t* status; unsigned char* ws; size_t ws_bytes; cudaStream_t st;
+    double* stats_partials; double* stats_n; int* n_parts;   // OUT_STATS: the generic kernel's partials, and how many it wrote
+    const void* prep; size_t prep_size;                        // prepared buffer (idl_profiles_prepared)
+    void* chunk; size_t chunk_size; int64_t max_long;          // chunked-path scratch (idl_profiles_chunked)
+};
+
+// a request with the arguments every entry point takes (S = n_variants: no slot selection)
+static ProfCall prof_call(const uint32_t* codes, const uint32_t* nmask, const int64_t* chunk_off, const int32_t* len, int64_t n_seqs_total, const int32_t* sidx,
+                          int64_t n_items, int64_t seq_id0, int k, const idl_variant* variants, int n_variants, uint64_t seed, void* ws, size_t ws_bytes, void* stream) {
+    ProfCall c{};
+    c.codes = codes; c.nmask = nmask; c.chunk_off = chunk_off; c.len = len; c.n_seqs_total = n_seqs_total; c.sidx = sidx;
+    c.n_items = n_items; c.seq_id0 = seq_id0; c.k = k; c.variants = variants; c.n_variants = n_variants; c.S = n_variants; c.seed = seed;
+    c.ws = reinterpret_cast<unsigned char*>(ws); c.ws_bytes = ws_bytes; c.st = (cudaStream_t)stream;
+    return c;
+}
+
+// the checks every request starts with; `who` names the entry point in the messages
+static int check_request(const ProfCall& c, const char* who) {
+    if (!c.codes || !c.nmask || !c.chunk_off || !c.len || !c.variants || (!c.out && c.out_kind != OUT_STATS) || !c.out_off || !c.ws)
+        return set_error(IDL_EINVAL, "%s: null pointer", who);
+    if (c.ws_bytes < WS_TOTAL) return set_error(IDL_EINVAL, "%s: workspace too small (need %lld bytes)", who, (long long)WS_TOTAL);
+    return IDL_OK;
 }
 
 // ---- host-side plan of one call: variant descriptors, gap tables, output offsets ----
@@ -1348,8 +1387,7 @@ struct HostPlan {
     int kind0;
 };
 
-static int make_plan(const char* who, const idl_variant* variants, int n_variants, const int64_t* out_off, int S, const int64_t* d_edit_off,
-                     const uint32_t* d_edits, unsigned char* ws, cudaStream_t st, HostPlan& hp) {
+static int make_plan(const char* who, const ProfCall& c, HostPlan& hp) {
     static thread_local VarDesc h_vars[MAX_VARIANTS];
     static thread_local uint32_t h_gtab[MAX_TABS * RNG_BLOCK];
     double tab_p[MAX_TABS];
@@ -1365,8 +1403,8 @@ static int make_plan(const char* who, const idl_variant* variants, int n_variant
     hp.n_bern = hp.n_ent = 0;
     hp.has_explicit = false;
     hp.randn_small = true;
-    for (int v = 0; v < n_variants; ++v) {
-        const idl_variant& iv = variants[v];
+    for (int v = 0; v < c.n_variants; ++v) {
+        const idl_variant& iv = c.variants[v];
         VarDesc& d = h_vars[v];
         d.kind = iv.kind; d.rng_id = iv.rng_id; d.n_bp = iv.n_bp; d.explicit_idx = iv.explicit_idx; d.tab1 = 0; d.tab2 = 0;
         d.slope1 = 0.f; d.slope2 = 0.f;
@@ -1381,66 +1419,66 @@ static int make_plan(const char* who, const idl_variant* variants, int n_variant
         }
         if (d.tab1 < 0 || d.tab2 < 0) return set_error(IDL_EUNSUPPORTED, "%s: too many distinct mutation rates", who, 0);
         if (iv.kind == IDL_KIND_RANDOM_N && (iv.n_bp < 0 || iv.n_bp > LIST_CAP / 2)) return set_error(IDL_EUNSUPPORTED, "%s: Random_N n_bp must be <= 1024", who, 0);
-        if (iv.kind == IDL_KIND_EXPLICIT && (!d_edit_off || !d_edits)) return set_error(IDL_EINVAL, "%s: explicit variant without edit lists", who, 0);
+        if (iv.kind == IDL_KIND_EXPLICIT && (!c.edit_off || !c.edits)) return set_error(IDL_EINVAL, "%s: explicit variant without edit lists", who, 0);
         if (iv.kind == IDL_KIND_EXPLICIT) hp.has_explicit = true;
         else if (iv.kind == IDL_KIND_RANDOM_N) { if (iv.n_bp * PC_K > 127) hp.randn_small = false; else if (iv.n_bp > 0) hp.n_ent += iv.n_bp; }
         else if (iv.kind != IDL_KIND_CLEAN) ++hp.n_bern;
     }
     hp.kind0 = h_vars[0].kind;
     hp.n_tabs = n_tabs;
-    hp.inl = n_variants <= SVARS && S <= SVARS && n_tabs <= STABS;
+    hp.inl = c.n_variants <= SVARS && c.S <= SVARS && n_tabs <= STABS;
     if (hp.inl) {
         memset(&hp.plan, 0, sizeof(hp.plan));
-        memcpy(hp.plan.vars, h_vars, sizeof(VarDesc) * n_variants);
-        for (int s = 0; s < S; ++s) hp.plan.out_off[s] = out_off[s];
+        memcpy(hp.plan.vars, h_vars, sizeof(VarDesc) * c.n_variants);
+        for (int s = 0; s < c.S; ++s) hp.plan.out_off[s] = c.out_off[s];
         memcpy(hp.plan.gtab, h_gtab, sizeof(uint32_t) * RNG_BLOCK * n_tabs);
     } else {   // big plans travel through the workspace (pageable staging: the host arrays may be reused after the calls return)
-        IDL_CUDA_CHECK(cudaMemcpyAsync(ws + WS_VARS, h_vars, sizeof(VarDesc) * n_variants, cudaMemcpyHostToDevice, st));
-        IDL_CUDA_CHECK(cudaMemcpyAsync(ws + WS_OUTOFF, out_off, sizeof(int64_t) * S, cudaMemcpyHostToDevice, st));
-        if (n_tabs) IDL_CUDA_CHECK(cudaMemcpyAsync(ws + WS_GTAB, h_gtab, sizeof(uint32_t) * RNG_BLOCK * n_tabs, cudaMemcpyHostToDevice, st));
+        IDL_CUDA_CHECK(cudaMemcpyAsync(c.ws + WS_VARS, h_vars, sizeof(VarDesc) * c.n_variants, cudaMemcpyHostToDevice, c.st));
+        IDL_CUDA_CHECK(cudaMemcpyAsync(c.ws + WS_OUTOFF, c.out_off, sizeof(int64_t) * c.S, cudaMemcpyHostToDevice, c.st));
+        if (n_tabs) IDL_CUDA_CHECK(cudaMemcpyAsync(c.ws + WS_GTAB, h_gtab, sizeof(uint32_t) * RNG_BLOCK * n_tabs, cudaMemcpyHostToDevice, c.st));
     }
     return IDL_OK;
 }
 
 // identity of a prepared buffer: FNV-1a over everything the prepared data depends on
-static unsigned long long prep_stamp_of(const uint32_t* d_codes, const int32_t* d_sidx, int64_t n_items, int64_t seq_id0, const idl_variant* variants,
-                                        int n_variants, uint64_t seed, int pseudocount) {
+static unsigned long long prep_stamp_of(const ProfCall& c) {
     unsigned long long h = 1469598103934665603ull;
     auto mix = [&](const void* ptr, size_t nb) {
         const unsigned char* b = reinterpret_cast<const unsigned char*>(ptr);
         for (size_t i = 0; i < nb; ++i) { h ^= b[i]; h *= 1099511628211ull; }
     };
-    mix(&d_codes, sizeof(d_codes)); mix(&d_sidx, sizeof(d_sidx)); mix(&n_items, sizeof(n_items)); mix(&seq_id0, sizeof(seq_id0));
-    mix(&seed, sizeof(seed)); mix(&pseudocount, sizeof(pseudocount));
-    for (int v = 0; v < n_variants; ++v) {   // slot 0 (statistics row) and the Bernoulli slots: what the buffer holds
-        const idl_variant& iv = variants[v];
+    mix(&c.codes, sizeof(c.codes)); mix(&c.sidx, sizeof(c.sidx)); mix(&c.n_items, sizeof(c.n_items)); mix(&c.seq_id0, sizeof(c.seq_id0));
+    mix(&c.seed, sizeof(c.seed)); mix(&c.pseudocount, sizeof(c.pseudocount));
+    for (int v = 0; v < c.n_variants; ++v) {   // slot 0 (statistics row) and the Bernoulli slots: what the buffer holds
+        const idl_variant& iv = c.variants[v];
         const bool bern = iv.kind == IDL_KIND_TRANSITION || iv.kind == IDL_KIND_TRANSVERSION || iv.kind == IDL_KIND_BOTH;
         if (v == 0 || bern) { mix(&iv.kind, sizeof(iv.kind)); mix(&iv.rng_id, sizeof(iv.rng_id)); mix(&iv.p1, sizeof(iv.p1)); mix(&iv.p2, sizeof(iv.p2)); }
     }
     return h ? h : 1ull;
 }
 
-static void fill_params(ProfParams& p, const uint32_t* d_codes, const uint32_t* d_nmask, const int64_t* d_chunk_off, const int32_t* d_len,
-                        int64_t n_seqs_total, const int32_t* d_sidx, int64_t n_items, int64_t seq_id0, int n_variants, const int32_t* d_sel, int S,
-                        uint64_t seed, const int64_t* d_edit_off, const uint32_t* d_edits, void* d_out, int64_t out_stride, int pseudocount,
-                        int accumulate, const float* d_mean, const float* d_scale, int32_t* d_status, unsigned char* ws, const HostPlan& hp) {
+// kernel parameters of a planned request; zeroes the work counters they point at
+static int fill_params(ProfParams& p, const ProfCall& c, const HostPlan& hp) {
+    IDL_CUDA_CHECK(cudaMemsetAsync(c.ws, 0, 24, c.st));   // work counter, deferred-item counter, deferred scan cursor
     memset(&p, 0, sizeof(p));
-    p.codes = d_codes; p.nmask = d_nmask; p.chunk_off = d_chunk_off; p.len = d_len; p.sidx = d_sidx; p.sel = d_sel;
-    p.n_items = n_items; p.seq_id0 = seq_id0; p.n_seqs_total = n_seqs_total; p.S = S; p.n_vars = n_variants; p.n_tabs = hp.n_tabs;
-    p.vars = reinterpret_cast<const VarDesc*>(ws + WS_VARS);
-    p.seed = seed; p.gtab = reinterpret_cast<const uint32_t*>(ws + WS_GTAB);
-    p.edit_off = d_edit_off; p.edits = d_edits; p.out = d_out;
-    p.out_off = reinterpret_cast<const int64_t*>(ws + WS_OUTOFF);
-    p.out_stride = out_stride; p.pseudocount = pseudocount; p.accumulate = accumulate & 1; p.cta_cap = (accumulate >> 8) & 0xFF;
-    p.mean = d_mean; p.scale = d_scale; p.status = d_status;
-    p.rscale = reinterpret_cast<const float*>(ws + WS_RSCALE);
-    p.work_counter = reinterpret_cast<unsigned long long*>(ws);
+    p.codes = c.codes; p.nmask = c.nmask; p.chunk_off = c.chunk_off; p.len = c.len; p.sidx = c.sidx; p.sel = c.sel;
+    p.n_items = c.n_items; p.seq_id0 = c.seq_id0; p.n_seqs_total = c.n_seqs_total; p.S = c.S; p.n_vars = c.n_variants; p.n_tabs = hp.n_tabs;
+    p.vars = reinterpret_cast<const VarDesc*>(c.ws + WS_VARS);
+    p.seed = c.seed; p.gtab = reinterpret_cast<const uint32_t*>(c.ws + WS_GTAB);
+    p.edit_off = c.edit_off; p.edits = c.edits; p.out = c.out;
+    p.out_off = reinterpret_cast<const int64_t*>(c.ws + WS_OUTOFF);
+    p.out_stride = c.out_stride; p.pseudocount = c.pseudocount; p.accumulate = c.accumulate & 1; p.cta_cap = (c.accumulate >> 8) & 0xFF;
+    p.mean = c.mean; p.scale = c.scale; p.status = c.status;
+    p.rscale = reinterpret_cast<const float*>(c.ws + WS_RSCALE);
+    p.work_counter = reinterpret_cast<unsigned long long*>(c.ws);
     p.inline_plan = hp.inl ? 1 : 0;
+    p.stats_partials = c.stats_partials; p.stats_n = c.stats_n;
 #ifdef IDL_DEVTOOLS
     static const bool want_prof = getenv("IDL_PHASE_PROF") != nullptr;
-    p.phase_prof = want_prof ? reinterpret_cast<unsigned long long*>(ws + WS_PROF) : nullptr;
+    p.phase_prof = want_prof ? reinterpret_cast<unsigned long long*>(c.ws + WS_PROF) : nullptr;
     { const char* e = getenv("IDL_PC_DBG"); p.dbg = e ? atoi(e) : 0; }
 #endif
+    return IDL_OK;
 }
 
 // ---- chunked path (chunked.cuh): scratch layout and sizing ----
@@ -1472,98 +1510,78 @@ static ChunkLayout chunk_layout(int64_t n_items, int64_t max_long, int nd_cap) {
     return l;
 }
 
-static int profiles_impl(const uint32_t* d_codes, const uint32_t* d_nmask, const int64_t* d_chunk_off,
-                         const int32_t* d_len, int64_t n_seqs_total, const int32_t* d_sidx, int64_t n_items,
-                         int64_t seq_id0, int k, const idl_variant* variants, int n_variants, const int32_t* d_sel,
-                         int S, uint64_t seed, const int64_t* d_edit_off, const uint32_t* d_edits, int out_kind,
-                         void* d_out, const int64_t* out_off, int64_t out_stride, int pseudocount, int accumulate,
-                         const float* d_mean, const float* d_scale, int32_t* d_status, void* d_workspace,
-                         size_t workspace_bytes, void* stream, double* d_stats_partials, double* d_stats_n, int* n_parts_out,
-                         const void* d_prep, size_t prep_size, void* d_chunk = nullptr, size_t chunk_size = 0, int64_t max_long = 0) {
-    cudaStream_t st = (cudaStream_t)stream;
-    const int64_t zero_off = 0;
-    if (out_kind == OUT_STATS) { out_off = &zero_off; out_stride = 0; }
-    if (!d_codes || !d_nmask || !d_chunk_off || !d_len || !variants || (!d_out && out_kind != OUT_STATS) || !out_off || !d_workspace)
-        return set_error(IDL_EINVAL, "idl_profiles: null pointer%s", "");
-    if (workspace_bytes < WS_TOTAL) return set_error(IDL_EINVAL, "idl_profiles: workspace too small%s (need %lld bytes)", "", (long long)WS_TOTAL);
-    if (k < 1 || k > 6) return set_error(IDL_EUNSUPPORTED, "idl_profiles: k must be in 1..6%s (got %lld)", "", k);
-    if (n_variants < 1 || n_variants > MAX_VARIANTS || S < 1 || S > MAX_VARIANTS)
+static int profiles_impl(const ProfCall& c) {
+    if (const int rc = check_request(c, "idl_profiles"); rc != IDL_OK) return rc;
+    if (c.k < 1 || c.k > 6) return set_error(IDL_EUNSUPPORTED, "idl_profiles: k must be in 1..6%s (got %lld)", "", c.k);
+    if (c.n_variants < 1 || c.n_variants > MAX_VARIANTS || c.S < 1 || c.S > MAX_VARIANTS)
         return set_error(IDL_EINVAL, "idl_profiles: n_variants / S out of range%s", "");
-    if (!d_sel && S != n_variants) return set_error(IDL_EINVAL, "idl_profiles: S must equal n_variants without d_sel%s", "");
-    if (out_kind == IDL_OUT_STD_F32 && (!d_mean || !d_scale)) return set_error(IDL_EINVAL, "idl_profiles: mean/scale required%s", "");
-    if ((accumulate & 1) && out_kind != IDL_OUT_COUNTS_I32) return set_error(IDL_EINVAL, "idl_profiles: accumulate only for counts%s", "");
-    if (n_items <= 0) return IDL_OK;
-    const int F = 1 << (2 * k);
-    if (k >= 1 && F >= 4 && (out_stride % 4 != 0)) return set_error(IDL_EINVAL, "idl_profiles: out_stride must be a multiple of 4%s", "");
+    if (!c.sel && c.S != c.n_variants) return set_error(IDL_EINVAL, "idl_profiles: S must equal n_variants without d_sel%s", "");
+    if (c.out_kind == IDL_OUT_STD_F32 && (!c.mean || !c.scale)) return set_error(IDL_EINVAL, "idl_profiles: mean/scale required%s", "");
+    if ((c.accumulate & 1) && c.out_kind != IDL_OUT_COUNTS_I32) return set_error(IDL_EINVAL, "idl_profiles: accumulate only for counts%s", "");
+    if (c.n_items <= 0) return IDL_OK;
+    if (c.out_stride % 4 != 0) return set_error(IDL_EINVAL, "idl_profiles: out_stride must be a multiple of 4%s", "");
 
-    unsigned char* ws = reinterpret_cast<unsigned char*>(d_workspace);
     HostPlan hp;
-    const int rc_plan = make_plan("idl_profiles", variants, n_variants, out_off, S, d_edit_off, d_edits, ws, st, hp);
-    if (rc_plan != IDL_OK) return rc_plan;
-    IDL_CUDA_CHECK(cudaMemsetAsync(ws, 0, 24, st));   // work counter, deferred-item counter, deferred scan cursor
     ProfParams p;
-    fill_params(p, d_codes, d_nmask, d_chunk_off, d_len, n_seqs_total, d_sidx, n_items, seq_id0, n_variants, d_sel, S, seed, d_edit_off, d_edits,
-                d_out, out_stride, pseudocount, accumulate, d_mean, d_scale, d_status, ws, hp);
-    if (out_kind == IDL_OUT_STD_F32) {
-        rscale_kernel<<<(F + 255) / 256, 256, 0, st>>>(d_scale, reinterpret_cast<float*>(ws + WS_RSCALE), F); note_launch();
+    if (const int rc = make_plan("idl_profiles", c, hp); rc != IDL_OK) return rc;
+    if (const int rc = fill_params(p, c, hp); rc != IDL_OK) return rc;
+    if (c.out_kind == IDL_OUT_STD_F32) {
+        const int F = 1 << (2 * c.k);
+        rscale_kernel<<<(F + 255) / 256, 256, 0, c.st>>>(c.scale, reinterpret_cast<float*>(c.ws + WS_RSCALE), F); note_launch();
         IDL_CUDA_CHECK(cudaGetLastError());
     }
-    p.stats_partials = d_stats_partials; p.stats_n = d_stats_n;
-    if (out_kind == OUT_STATS) return dispatch_k(p, hp.plan, k, out_kind, st, n_parts_out);
+    if (c.out_kind == OUT_STATS) return dispatch_k(p, hp.plan, c.k, c.out_kind, c.st, c.n_parts);
     // ---- chunked path for the long items (k = 6): tiles spread over the whole grid, exact integer reduction ----
-    if (d_chunk && k == 6 && max_long > 0) {
-        const int nd_cap = chunk_dense_cap(variants, n_variants, S);
-        if (nd_cap <= CH_MAX_DENSE && !((uintptr_t)d_chunk & 15)) {
-            const ChunkLayout lay = chunk_layout(n_items, max_long, nd_cap);
-            if (lay.grid > 0 && chunk_size >= lay.bytes) {
-                unsigned char* cb = reinterpret_cast<unsigned char*>(d_chunk);
+    if (c.chunk && c.k == 6 && c.max_long > 0) {
+        const int nd_cap = chunk_dense_cap(c.variants, c.n_variants, c.S);
+        if (nd_cap <= CH_MAX_DENSE && !((uintptr_t)c.chunk & 15)) {
+            const ChunkLayout lay = chunk_layout(c.n_items, c.max_long, nd_cap);
+            if (lay.grid > 0 && c.chunk_size >= lay.bytes) {
+                unsigned char* cb = reinterpret_cast<unsigned char*>(c.chunk);
                 ChParams cp;
                 cp.p = p;
                 cp.hdr = reinterpret_cast<ChHeader*>(cb);
                 cp.tile_off = reinterpret_cast<long long*>(cb + lay.off_tiles);
                 cp.long_rank = reinterpret_cast<int*>(cb + lay.off_rank);
                 cp.partials = reinterpret_cast<int*>(cb + lay.off_partials);
-                cp.max_long = max_long; cp.nd_cap = nd_cap; cp.grid_tiles = lay.grid;
-                ch_plan_kernel<<<1, 1024, 0, st>>>(cp); note_launch();
+                cp.max_long = c.max_long; cp.nd_cap = nd_cap; cp.grid_tiles = lay.grid;
+                ch_plan_kernel<<<1, 1024, 0, c.st>>>(cp); note_launch();
                 IDL_CUDA_CHECK(cudaGetLastError());
                 IDL_CUDA_CHECK(ensure_dyn_smem((const void*)ch_tile_kernel<6>, lay.smem));
-                ch_tile_kernel<6><<<(unsigned)lay.grid, CH_NT, lay.smem, st>>>(cp, hp.plan); note_launch();
+                ch_tile_kernel<6><<<(unsigned)lay.grid, CH_NT, lay.smem, c.st>>>(cp, hp.plan); note_launch();
                 IDL_CUDA_CHECK(cudaGetLastError());
                 long long rgrid = (long long)sm_count() * 2;
-                if (rgrid > n_items) rgrid = n_items;
-                switch (out_kind) {
-                    case IDL_OUT_COUNTS_I32: ch_reduce_kernel<6, IDL_OUT_COUNTS_I32><<<(unsigned)rgrid, CH_NT, 0, st>>>(cp, hp.plan); break;
-                    case IDL_OUT_FREQ_F32: ch_reduce_kernel<6, IDL_OUT_FREQ_F32><<<(unsigned)rgrid, CH_NT, 0, st>>>(cp, hp.plan); break;
-                    case IDL_OUT_STD_F32: ch_reduce_kernel<6, IDL_OUT_STD_F32><<<(unsigned)rgrid, CH_NT, 0, st>>>(cp, hp.plan); break;
-                    default: ch_reduce_kernel<6, IDL_OUT_FREQ_F64><<<(unsigned)rgrid, CH_NT, 0, st>>>(cp, hp.plan); break;
-                }
-                note_launch();
+                if (rgrid > c.n_items) rgrid = c.n_items;
+                using ReduceKernel = void (*)(ChParams, Plan);   // (OUT_STATS requests returned above)
+                const ReduceKernel reduce = kernel_for_out<ReduceKernel>(c.out_kind, nullptr, ch_reduce_kernel<6, IDL_OUT_COUNTS_I32>, ch_reduce_kernel<6, IDL_OUT_FREQ_F32>,
+                                                                         ch_reduce_kernel<6, IDL_OUT_STD_F32>, ch_reduce_kernel<6, IDL_OUT_FREQ_F64>);
+                reduce<<<(unsigned)rgrid, CH_NT, 0, c.st>>>(cp, hp.plan); note_launch();
                 IDL_CUDA_CHECK(cudaGetLastError());
                 p.long_overflow = &cp.hdr->overflow;   // the generic kernel skips the long items (unless the plan found more than max_long)
             }
         }
     }
     // ---- producer/consumer kernel (k = 6, float outputs, whole-schedule featurisation of PREPARED items) ----
-    bool pc_ok = d_prep && k == 6 && (out_kind == IDL_OUT_FREQ_F32 || out_kind == IDL_OUT_STD_F32) && !d_sel && d_status && hp.inl &&
-                 n_variants <= PC_MAXS && n_items >= 2LL * sm_count() && prep_size >= prep_bytes(n_items);
+    bool pc_ok = c.prep && c.k == 6 && (c.out_kind == IDL_OUT_FREQ_F32 || c.out_kind == IDL_OUT_STD_F32) && !c.sel && c.status && hp.inl &&
+                 c.n_variants <= PC_MAXS && c.n_items >= 2LL * sm_count() && c.prep_size >= prep_bytes(c.n_items);
     if (pc_ok) {
         if (hp.has_explicit || !hp.randn_small || hp.n_bern > PC_DENSE || hp.n_ent > PC_LIST || hp.n_ent * PC_K > PC_REM) pc_ok = false;
         // TMA bulk copies: 16-byte aligned rows
-        if (((uintptr_t)d_out & 15) || (out_stride & 3) || ((uintptr_t)d_codes & 15) || ((uintptr_t)d_nmask & 15) || ((uintptr_t)d_prep & 15)) pc_ok = false;
-        for (int v = 0; v < S && pc_ok; ++v) if (out_off[v] & 3) pc_ok = false;
+        if (((uintptr_t)c.out & 15) || (c.out_stride & 3) || ((uintptr_t)c.codes & 15) || ((uintptr_t)c.nmask & 15) || ((uintptr_t)c.prep & 15)) pc_ok = false;
+        for (int v = 0; v < c.S && pc_ok; ++v) if (c.out_off[v] & 3) pc_ok = false;
     }
     if (pc_ok) {
-        p.prep = const_cast<void*>(d_prep);
-        p.prep_stamp = prep_stamp_of(d_codes, d_sidx, n_items, seq_id0, variants, n_variants, seed, pseudocount);
-        auto kern = out_kind == IDL_OUT_STD_F32 ? profiles_pc_kernel<IDL_OUT_STD_F32> : profiles_pc_kernel<IDL_OUT_FREQ_F32>;
+        p.prep = const_cast<void*>(c.prep);
+        p.prep_stamp = prep_stamp_of(c);
+        auto kern = c.out_kind == IDL_OUT_STD_F32 ? profiles_pc_kernel<IDL_OUT_STD_F32> : profiles_pc_kernel<IDL_OUT_FREQ_F32>;
         IDL_CUDA_CHECK(ensure_dyn_smem((const void*)kern, sizeof(PcSmem)));
         long long grid = sm_count();
-        if (grid > n_items) grid = n_items;
-        kern<<<(unsigned)grid, PC_NT, sizeof(PcSmem), st>>>(p, hp.plan); note_launch();
+        if (grid > c.n_items) grid = c.n_items;
+        kern<<<(unsigned)grid, PC_NT, sizeof(PcSmem), c.st>>>(p, hp.plan); note_launch();
         IDL_CUDA_CHECK(cudaGetLastError());
         p.only_deferred = 1;   // whatever the fast kernel could not take is redone by the generic one
     }
-    return dispatch_k(p, hp.plan, k, out_kind, st);
+    return dispatch_k(p, hp.plan, c.k, c.out_kind, c.st);
 }
 
 }  // namespace idl
@@ -1611,9 +1629,10 @@ int idl_profiles(const uint32_t* d_codes, const uint32_t* d_nmask, const int64_t
                  const float* d_mean, const float* d_scale, int32_t* d_status, void* d_workspace,
                  size_t workspace_bytes, void* stream) {
     if (out_kind < IDL_OUT_COUNTS_I32 || out_kind > IDL_OUT_FREQ_F64) return set_error(IDL_EINVAL, "idl_profiles: unknown out_kind%s %lld", "", out_kind);
-    return profiles_impl(d_codes, d_nmask, d_chunk_off, d_len, n_seqs_total, d_sidx, n_items, seq_id0, k, variants, n_variants, d_sel, S,
-                         seed, d_edit_off, d_edits, out_kind, d_out, out_off, out_stride, pseudocount, accumulate, d_mean, d_scale,
-                         d_status, d_workspace, workspace_bytes, stream, nullptr, nullptr, nullptr, nullptr, 0);
+    ProfCall c = prof_call(d_codes, d_nmask, d_chunk_off, d_len, n_seqs_total, d_sidx, n_items, seq_id0, k, variants, n_variants, seed, d_workspace, workspace_bytes, stream);
+    c.sel = d_sel; c.S = S; c.edit_off = d_edit_off; c.edits = d_edits; c.out_kind = out_kind; c.out = d_out; c.out_off = out_off;
+    c.out_stride = out_stride; c.pseudocount = pseudocount; c.accumulate = accumulate; c.mean = d_mean; c.scale = d_scale; c.status = d_status;
+    return profiles_impl(c);
 }
 
 size_t idl_profiles_chunked_bytes(int64_t n_items, int64_t max_long_items, const idl_variant* variants, int n_variants, int S) {
@@ -1633,9 +1652,11 @@ int idl_profiles_chunked(const uint32_t* d_codes, const uint32_t* d_nmask, const
                          void* d_workspace, size_t workspace_bytes, void* stream) {
     if (out_kind < IDL_OUT_COUNTS_I32 || out_kind > IDL_OUT_FREQ_F64) return set_error(IDL_EINVAL, "idl_profiles_chunked: unknown out_kind%s %lld", "", out_kind);
     if (!d_scratch || max_long_items < 0) return set_error(IDL_EINVAL, "idl_profiles_chunked: scratch required%s", "");
-    return profiles_impl(d_codes, d_nmask, d_chunk_off, d_len, n_seqs_total, d_sidx, n_items, seq_id0, k, variants, n_variants, d_sel, S,
-                         seed, d_edit_off, d_edits, out_kind, d_out, out_off, out_stride, pseudocount, accumulate, d_mean, d_scale,
-                         nullptr, d_workspace, workspace_bytes, stream, nullptr, nullptr, nullptr, nullptr, 0, d_scratch, scratch_bytes, max_long_items);
+    ProfCall c = prof_call(d_codes, d_nmask, d_chunk_off, d_len, n_seqs_total, d_sidx, n_items, seq_id0, k, variants, n_variants, seed, d_workspace, workspace_bytes, stream);
+    c.sel = d_sel; c.S = S; c.edit_off = d_edit_off; c.edits = d_edits; c.out_kind = out_kind; c.out = d_out; c.out_off = out_off;
+    c.out_stride = out_stride; c.pseudocount = pseudocount; c.accumulate = accumulate; c.mean = d_mean; c.scale = d_scale;
+    c.chunk = d_scratch; c.chunk_size = scratch_bytes; c.max_long = max_long_items;
+    return profiles_impl(c);
 }
 
 int idl_profiles_prepared(const uint32_t* d_codes, const uint32_t* d_nmask, const int64_t* d_chunk_off,
@@ -1646,9 +1667,10 @@ int idl_profiles_prepared(const uint32_t* d_codes, const uint32_t* d_nmask, cons
                           void* d_workspace, size_t workspace_bytes, void* stream) {
     if (out_kind != IDL_OUT_FREQ_F32 && out_kind != IDL_OUT_STD_F32) return set_error(IDL_EINVAL, "idl_profiles_prepared: float32 outputs only%s", "");
     if (!d_prep || !d_status) return set_error(IDL_EINVAL, "idl_profiles_prepared: d_prep and d_status are required%s", "");
-    return profiles_impl(d_codes, d_nmask, d_chunk_off, d_len, n_seqs_total, d_sidx, n_items, seq_id0, k, variants, n_variants, nullptr, n_variants,
-                         seed, nullptr, nullptr, out_kind, d_out, out_off, out_stride, pseudocount, 0, d_mean, d_scale,
-                         d_status, d_workspace, workspace_bytes, stream, nullptr, nullptr, nullptr, d_prep, prep_size);
+    ProfCall c = prof_call(d_codes, d_nmask, d_chunk_off, d_len, n_seqs_total, d_sidx, n_items, seq_id0, k, variants, n_variants, seed, d_workspace, workspace_bytes, stream);
+    c.out_kind = out_kind; c.out = d_out; c.out_off = out_off; c.out_stride = out_stride; c.pseudocount = pseudocount;
+    c.mean = d_mean; c.scale = d_scale; c.status = d_status; c.prep = d_prep; c.prep_size = prep_size;
+    return profiles_impl(c);
 }
 
 size_t idl_prepare_bytes(int64_t n_items) { return n_items > 0 ? prep_bytes(n_items) : 0; }
@@ -1658,40 +1680,31 @@ int idl_profiles_prepare(const uint32_t* d_codes, const uint32_t* d_nmask, const
                          const idl_variant* variants, int n_variants, uint64_t seed, int pseudocount, void* d_prep, size_t prep_size,
                          double* d_partials, double* d_part_n, int max_parts, int* n_parts, int32_t* d_status, void* d_workspace,
                          size_t workspace_bytes, void* stream) {
-    cudaStream_t st = (cudaStream_t)stream;
-    if (!d_codes || !d_nmask || !d_chunk_off || !d_len || !variants || !d_prep || !d_status || !d_workspace)
-        return set_error(IDL_EINVAL, "idl_profiles_prepare: null pointer%s", "");
+    int64_t offs[PC_MAXS] = {};   // the prepare pass writes no profile rows
+    ProfCall c = prof_call(d_codes, d_nmask, d_chunk_off, d_len, n_seqs_total, d_sidx, n_items, seq_id0, k, variants, n_variants, seed, d_workspace, workspace_bytes, stream);
+    c.out_kind = OUT_STATS; c.out_off = offs; c.pseudocount = pseudocount; c.status = d_status;
+    if (!d_prep || !d_status) return set_error(IDL_EINVAL, "idl_profiles_prepare: null pointer%s", "");
+    if (const int rc = check_request(c, "idl_profiles_prepare"); rc != IDL_OK) return rc;
     if (k != PC_K) return set_error(IDL_EUNSUPPORTED, "idl_profiles_prepare: k must be 6%s (got %lld)", "", k);
-    if (workspace_bytes < WS_TOTAL) return set_error(IDL_EINVAL, "idl_profiles_prepare: workspace too small%s (need %lld bytes)", "", (long long)WS_TOTAL);
     if (n_variants < 1 || n_variants > PC_MAXS) return set_error(IDL_EUNSUPPORTED, "idl_profiles_prepare: 1..64 variants%s", "");
     if (n_items <= 0) { if (n_parts) *n_parts = 0; return IDL_OK; }
     if (prep_size < prep_bytes(n_items)) return set_error(IDL_EINVAL, "idl_profiles_prepare: d_prep too small%s (need %lld bytes)", "", (long long)prep_bytes(n_items));
     if (((uintptr_t)d_prep & 15) || ((uintptr_t)d_codes & 15) || ((uintptr_t)d_nmask & 7)) return set_error(IDL_EINVAL, "idl_profiles_prepare: misaligned buffer%s", "");
     if (d_partials && (!d_part_n || !n_parts || max_parts < sm_count() * 8)) return set_error(IDL_EINVAL, "idl_profiles_prepare: statistics need d_part_n, n_parts and max_parts >= 8 x SMs%s", "");
-    unsigned char* ws = reinterpret_cast<unsigned char*>(d_workspace);
-    int64_t offs[PC_MAXS];
-    for (int s = 0; s < n_variants; ++s) offs[s] = 0;
     HostPlan hp;
-    const int rc_plan = make_plan("idl_profiles_prepare", variants, n_variants, offs, n_variants, nullptr, nullptr, ws, st, hp);
-    if (rc_plan != IDL_OK) return rc_plan;
+    if (const int rc = make_plan("idl_profiles_prepare", c, hp); rc != IDL_OK) return rc;
     if (!hp.inl || hp.has_explicit || hp.n_bern > PC_DENSE) return set_error(IDL_EUNSUPPORTED, "idl_profiles_prepare: at most 3 Bernoulli slots, 4 distinct rates, no explicit lists%s", "");
     if (hp.kind0 == IDL_KIND_RANDOM_N && variants[0].n_bp > 0) return set_error(IDL_EUNSUPPORTED, "idl_profiles_prepare: slot 0 must be clean or a Bernoulli mimic%s", "");
-    IDL_CUDA_CHECK(cudaMemsetAsync(ws, 0, 24, st));
     ProfParams p;
-    fill_params(p, d_codes, d_nmask, d_chunk_off, d_len, n_seqs_total, d_sidx, n_items, seq_id0, n_variants, nullptr, n_variants, seed, nullptr, nullptr,
-                nullptr, 0, pseudocount, 0, nullptr, nullptr, d_status, ws, hp);
+    if (const int rc = fill_params(p, c, hp); rc != IDL_OK) return rc;
     p.prep = d_prep;
-    p.prep_stamp = prep_stamp_of(d_codes, d_sidx, n_items, seq_id0, variants, n_variants, seed, pseudocount);
-    IDL_CUDA_CHECK(ensure_dyn_smem((const void*)prep_kernel<PC_K>, sizeof(PrSmem)));
-    int per_sm = 0;
-    IDL_CUDA_CHECK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, prep_kernel<PC_K>, PR_NT, sizeof(PrSmem)));
-    if (per_sm < 1) return set_error(IDL_ECUDA, "prepare kernel does not fit on an SM%s", "");
-    long long grid = (long long)sm_count() * per_sm;
-    if (grid > n_items) grid = n_items;
-    prep_kernel<PC_K><<<(unsigned)grid, PR_NT, sizeof(PrSmem), st>>>(p, hp.plan); note_launch();
+    p.prep_stamp = prep_stamp_of(c);
+    unsigned grid = 0;
+    if (const int rc = persistent_grid(prep_kernel<PC_K>, PR_NT, sizeof(PrSmem), 0, n_items, "prepare", grid); rc != IDL_OK) return rc;
+    prep_kernel<PC_K><<<grid, PR_NT, sizeof(PrSmem), c.st>>>(p, hp.plan); note_launch();
     IDL_CUDA_CHECK(cudaGetLastError());
     if (!d_partials) {   // no statistics wanted: nobody consumes the "left to the generic kernel" marks of this call (the prepared records keep them)
-        IDL_CUDA_CHECK(cudaMemsetAsync(d_status, 0, sizeof(int32_t) * (size_t)n_items, st));
+        IDL_CUDA_CHECK(cudaMemsetAsync(d_status, 0, sizeof(int32_t) * (size_t)n_items, c.st));
         return IDL_OK;
     }
     // ---- statistics of slot 0: column sums over the prepared rows + the generic kernel for the items the prepare pass left out ----
@@ -1699,20 +1712,15 @@ int idl_profiles_prepare(const uint32_t* d_codes, const uint32_t* d_nmask, const
     if (parts > n_items) parts = (int)n_items;
     const int rows_per_part = (int)((n_items + parts - 1) / parts);
     parts = (int)((n_items + rows_per_part - 1) / rows_per_part);
-    if (pseudocount > 0)   // every frequency is a positive normal float
-        colstats16_kernel<true><<<dim3(PC_F / 4 / CS16_NT, (unsigned)parts), CS16_NT, 0, st>>>(reinterpret_cast<const unsigned char*>(d_prep), n_items, rows_per_part,
-                                                                                             pseudocount, d_partials, d_part_n);
-    else
-        colstats16_kernel<false><<<dim3(PC_F / 4 / CS16_NT, (unsigned)parts), CS16_NT, 0, st>>>(reinterpret_cast<const unsigned char*>(d_prep), n_items, rows_per_part,
-                                                                                              pseudocount, d_partials, d_part_n);
-    note_launch();
+    const auto colstats = pseudocount > 0 ? colstats16_kernel<true> : colstats16_kernel<false>;   // true: every frequency is a positive normal float
+    colstats<<<dim3(PC_F / 4 / CS16_NT, (unsigned)parts), CS16_NT, 0, c.st>>>(reinterpret_cast<const unsigned char*>(d_prep), n_items, rows_per_part, pseudocount,
+                                                                           d_partials, d_part_n); note_launch();
     IDL_CUDA_CHECK(cudaGetLastError());
-    p.only_deferred = 1;
-    p.S = 1; p.n_vars = 1;
+    p.only_deferred = 1; p.S = 1; p.n_vars = 1;
     p.stats_partials = d_partials + (size_t)parts * 2 * PC_F;
     p.stats_n = d_part_n + parts;
     int g2 = 0;
-    const int rc = dispatch_k(p, hp.plan, k, OUT_STATS, st, &g2);
+    const int rc = dispatch_k(p, hp.plan, k, OUT_STATS, c.st, &g2);
     *n_parts = parts + g2;
     return rc;
 }
@@ -1726,22 +1734,22 @@ int idl_profile_stats(const uint32_t* d_codes, const uint32_t* d_nmask, const in
     if (max_parts < sm_count() * 8) return set_error(IDL_EINVAL, "idl_profile_stats: max_parts too small%s (need %lld)", "", (long long)sm_count() * 8);
     *n_parts = 0;
     if (n_items <= 0) return IDL_OK;
-    return profiles_impl(d_codes, d_nmask, d_chunk_off, d_len, n_seqs_total, d_sidx, n_items, seq_id0, k, variant, 1, nullptr, 1, seed,
-                         d_edit_off, d_edits, OUT_STATS, nullptr, nullptr, 0, pseudocount, 0, nullptr, nullptr, d_status, d_workspace,
-                         workspace_bytes, stream, d_partials, d_part_n, n_parts, nullptr, 0);
+    const int64_t zero_off = 0;
+    ProfCall c = prof_call(d_codes, d_nmask, d_chunk_off, d_len, n_seqs_total, d_sidx, n_items, seq_id0, k, variant, 1, seed, d_workspace, workspace_bytes, stream);
+    c.edit_off = d_edit_off; c.edits = d_edits; c.out_kind = OUT_STATS; c.out_off = &zero_off; c.pseudocount = pseudocount; c.status = d_status;
+    c.stats_partials = d_partials; c.stats_n = d_part_n; c.n_parts = n_parts;
+    return profiles_impl(c);
 }
 
 int idl_kmer_counts(const uint32_t* d_codes, const uint32_t* d_nmask, const int64_t* d_chunk_off,
                     const int32_t* d_len, int64_t n, int k, int32_t* d_counts, int accumulate,
                     void* d_workspace, size_t workspace_bytes, void* stream) {
-    idl_variant v;
-    memset(&v, 0, sizeof(v));
-    v.kind = IDL_KIND_CLEAN;
-    const int64_t off0 = 0;
     if (k < 1 || k > 6) return set_error(IDL_EUNSUPPORTED, "idl_kmer_counts: k must be in 1..6%s (got %lld)", "", k);
-    return idl_profiles(d_codes, d_nmask, d_chunk_off, d_len, n, nullptr, n, 0, k, &v, 1, nullptr, 1, 0, nullptr, nullptr,
-                        IDL_OUT_COUNTS_I32, d_counts, &off0, (int64_t)1 << (2 * k), 0, accumulate, nullptr, nullptr, nullptr,
-                        d_workspace, workspace_bytes, stream);
+    const idl_variant clean{IDL_KIND_CLEAN};
+    const int64_t off0 = 0;
+    ProfCall c = prof_call(d_codes, d_nmask, d_chunk_off, d_len, n, nullptr, n, 0, k, &clean, 1, 0, d_workspace, workspace_bytes, stream);
+    c.out_kind = IDL_OUT_COUNTS_I32; c.out = d_counts; c.out_off = &off0; c.out_stride = (int64_t)1 << (2 * k); c.accumulate = accumulate;
+    return profiles_impl(c);
 }
 
 int idl_colstats_parts(int64_t n) { return n > 0 ? (int)((n + cs_rows(n) - 1) / cs_rows(n)) : 0; }
@@ -1770,10 +1778,7 @@ int idl_standardize_f32(const float* d_x, float* d_out, int64_t n, int F, const 
     if (!d_x || !d_out || !d_mean32 || !d_scale32 || n < 0 || F <= 0 || F % 4) return set_error(IDL_EINVAL, "idl_standardize_f32: bad argument%s", "");
     if (n == 0) return IDL_OK;
     const long long n4 = n * (F / 4);
-    long long grid = (n4 + 255) / 256;
-    const long long cap = (long long)sm_count() * 16;
-    if (grid > cap) grid = cap;
-    standardize_f32_kernel<<<(unsigned)grid, 256, 0, (cudaStream_t)stream>>>(d_x, d_out, n4, F / 4, d_mean32, d_scale32); note_launch();
+    standardize_f32_kernel<<<elementwise_grid(n4), 256, 0, (cudaStream_t)stream>>>(d_x, d_out, n4, F / 4, d_mean32, d_scale32); note_launch();
     IDL_CUDA_CHECK(cudaGetLastError());
     return IDL_OK;
 }
@@ -1782,10 +1787,7 @@ int idl_cgr_map(const int32_t* d_counts, int64_t n, int k, int32_t* d_cgr, int a
     if (!d_counts || !d_cgr || n < 0 || k < 1 || k > 12) return set_error(IDL_EINVAL, "idl_cgr_map: bad argument%s", "");
     const long long total = n << (2 * k);
     if (total == 0) return IDL_OK;
-    long long grid = (total + 255) / 256;
-    const long long cap = (long long)sm_count() * 16;
-    if (grid > cap) grid = cap;
-    cgr_map_kernel<<<(unsigned)grid, 256, 0, (cudaStream_t)stream>>>(d_counts, d_cgr, total, k, accumulate); note_launch();
+    cgr_map_kernel<<<elementwise_grid(total), 256, 0, (cudaStream_t)stream>>>(d_counts, d_cgr, total, k, accumulate); note_launch();
     IDL_CUDA_CHECK(cudaGetLastError());
     return IDL_OK;
 }
@@ -1801,10 +1803,7 @@ int idl_revcomp_canonical(int k, int32_t* h_index) {
 int idl_revcomp_fold(const int32_t* d_counts, int64_t n, int k, const int32_t* d_canon, int R, int32_t* d_out, void* stream) {
     if (!d_counts || !d_out || !d_canon || n < 0 || k < 1 || k > 12 || R < 1) return set_error(IDL_EINVAL, "idl_revcomp_fold: bad argument%s", "");
     if (n == 0) return IDL_OK;
-    long long grid = (n * R + 255) / 256;
-    const long long cap = (long long)sm_count() * 16;
-    if (grid > cap) grid = cap;
-    revcomp_fold_kernel<<<(unsigned)grid, 256, 0, (cudaStream_t)stream>>>(d_counts, d_out, n, k, d_canon, R); note_launch();
+    revcomp_fold_kernel<<<elementwise_grid(n * R), 256, 0, (cudaStream_t)stream>>>(d_counts, d_out, n, k, d_canon, R); note_launch();
     IDL_CUDA_CHECK(cudaGetLastError());
     return IDL_OK;
 }
@@ -1823,10 +1822,7 @@ int idl_standardize_f64(const double* d_x, double* d_out64, float* d_out32, int6
     if (!d_x || (!d_out64 && !d_out32) || !d_mean64 || !d_scale64 || n < 0 || F <= 0) return set_error(IDL_EINVAL, "idl_standardize_f64: bad argument%s", "");
     if (n == 0) return IDL_OK;
     const long long total = n * (long long)F;
-    long long grid = (total + 255) / 256;
-    const long long cap = (long long)sm_count() * 16;
-    if (grid > cap) grid = cap;
-    standardize_f64_kernel<<<(unsigned)grid, 256, 0, (cudaStream_t)stream>>>(d_x, d_out64, d_out32, total, F, d_mean64, d_scale64); note_launch();
+    standardize_f64_kernel<<<elementwise_grid(total), 256, 0, (cudaStream_t)stream>>>(d_x, d_out64, d_out32, total, F, d_mean64, d_scale64); note_launch();
     IDL_CUDA_CHECK(cudaGetLastError());
     return IDL_OK;
 }

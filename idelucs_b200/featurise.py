@@ -14,6 +14,7 @@ _OUT_DTYPE = {OUT_COUNTS_I32: torch.int32, OUT_FREQ_F32: torch.float32, OUT_STD_
 
 LONG_MIN = 65536   # items at least this long take the chunked path (csrc/chunked.cuh)
 MAX_EDIT_POS = 1 << 29   # edit entries are pos << 3 | val in 32 bits: mutated variants need sequences shorter than this
+MAX_PARTS = 2048   # scaler partials idl_profiles_prepare / idl_profile_stats may write (>= 8 per SM)
 
 # hard-coded rates of the reference's AugmentFasta (idelucs/utils.py:330-349)
 P_TRANSITION, P_TRANSVERSION, N_RANDOM_N = 1e-2, 0.5e-2, 20
@@ -73,6 +74,33 @@ def _workspace(device, nbytes, tag):
     return ws
 
 
+def _seqset_args(seqset):
+    """(codes, nmask, chunk_off, len, n): the arguments the profile entry points start with"""
+    return _lib.ptr(seqset.codes), _lib.ptr(seqset.nmask), _lib.ptr(seqset.chunk_off), _lib.ptr(seqset.len), seqset.n
+
+
+def _seed(seed):
+    return ctypes.c_uint64(seed & (2 ** 64 - 1))
+
+
+def _workspace_args(lib, device):
+    """(workspace, its size, stream): the arguments the profile entry points end with (inside ``torch.cuda.device(device)``)"""
+    ws = _workspace(device, lib.idl_profiles_workspace_bytes(), "prof")
+    return _lib.ptr(ws), ws.numel(), _lib.stream_ptr()
+
+
+def _stats_buffers(F, device):
+    return (torch.empty((MAX_PARTS, 2, F), dtype=torch.float64, device=device),
+            torch.zeros((MAX_PARTS,), dtype=torch.float64, device=device))
+
+
+def _scaler(parts, part_n, group):
+    """Scaler of this process's partials, or of the whole torch.distributed group's (a collective) when group is given"""
+    if group is not None:
+        parts, part_n = gather_partials(parts, part_n, group)
+    return Scaler.from_partials(parts, part_n)
+
+
 def pack_edit_lists(explicit, n_seqs, device):
     """explicit: list (one per EXPLICIT variant) of per-sequence (pos, val) pairs, val in 0..4
     (A C G T N) -> CSR (int64 offsets, int32-typed uint32 entries pos<<3|val) on the device."""
@@ -107,10 +135,7 @@ class Prepared(object):
         self.buf, self.parts, self.part_n, self.key = buf, parts, part_n, key
 
     def scaler(self, group=None):
-        parts, part_n = self.parts, self.part_n
-        if group is not None:
-            parts, part_n = gather_partials(parts, part_n, group)
-        return Scaler.from_partials(parts, part_n)
+        return _scaler(self.parts, self.part_n, group)
 
 
 def can_prepare(seqset, k, variants, n_items=None):
@@ -134,18 +159,14 @@ def prepare(seqset, k, variants, seed=0, seq_id0=0, pseudocount=1, want_stats=Tr
     nbytes = lib.idl_prepare_bytes(n)
     if buf is None or buf.numel() < nbytes:
         buf = torch.empty(nbytes, dtype=torch.uint8, device=device)
-    max_parts = 2048
-    parts = torch.empty((max_parts, 2, F), dtype=torch.float64, device=device) if want_stats else None
-    part_n = torch.zeros((max_parts,), dtype=torch.float64, device=device) if want_stats else None
+    parts, part_n = _stats_buffers(F, device) if want_stats else (None, None)
     n_parts = ctypes.c_int(0)
     status = torch.zeros((max(n, 1),), dtype=torch.int32, device=device)
     varr = _variant_array(variants)
     with torch.cuda.device(device):
-        ws = _workspace(device, lib.idl_profiles_workspace_bytes(), "prof")
-        _lib.check(lib.idl_profiles_prepare(_lib.ptr(seqset.codes), _lib.ptr(seqset.nmask), _lib.ptr(seqset.chunk_off), _lib.ptr(seqset.len),
-                                            seqset.n, _lib.ptr(sidx), n, int(seq_id0), k, varr, len(variants), ctypes.c_uint64(seed & (2 ** 64 - 1)),
-                                            int(pseudocount), _lib.ptr(buf), buf.numel(), _lib.ptr(parts), _lib.ptr(part_n), max_parts,
-                                            ctypes.byref(n_parts), _lib.ptr(status), _lib.ptr(ws), ws.numel(), _lib.stream_ptr()))
+        _lib.check(lib.idl_profiles_prepare(*_seqset_args(seqset), _lib.ptr(sidx), n, int(seq_id0), k, varr, len(variants), _seed(seed),
+                                            int(pseudocount), _lib.ptr(buf), buf.numel(), _lib.ptr(parts), _lib.ptr(part_n), MAX_PARTS,
+                                            ctypes.byref(n_parts), _lib.ptr(status), *_workspace_args(lib, device)))
     if want_stats:
         parts, part_n = parts[: n_parts.value], part_n[: n_parts.value]
     return Prepared(buf, parts, part_n, (id(seqset), k, seed, seq_id0, pseudocount, len(variants)) if sidx is None else None)
@@ -182,17 +203,15 @@ def profiles(seqset, k, variants, out_kind=OUT_FREQ_F32, seed=0, out=None, out_o
     offs = (ctypes.c_int64 * S)(*[int(o) for o in out_off])
     d_eoff, d_ent = (None, None) if edit_lists is None else edit_lists
     with torch.cuda.device(device):
-        ws = _workspace(device, lib.idl_profiles_workspace_bytes(), "prof")
         if prepared is not None:
             assert sidx is None and sel is None and edit_lists is None and out_kind in (OUT_FREQ_F32, OUT_STD_F32)
             assert prepared.key == (id(seqset), k, seed, seq_id0, pseudocount, nv), "prepared for a different call"
             if status is None:
                 status = torch.zeros(n_items, dtype=torch.int32, device=device)
             _lib.check(lib.idl_profiles_prepared(
-                _lib.ptr(seqset.codes), _lib.ptr(seqset.nmask), _lib.ptr(seqset.chunk_off), _lib.ptr(seqset.len), seqset.n,
-                None, n_items, int(seq_id0), k, varr, nv, ctypes.c_uint64(seed & (2 ** 64 - 1)), out_kind, _lib.ptr(out), offs,
+                *_seqset_args(seqset), None, n_items, int(seq_id0), k, varr, nv, _seed(seed), out_kind, _lib.ptr(out), offs,
                 int(out_stride), int(pseudocount), _lib.ptr(mean), _lib.ptr(scale), _lib.ptr(status), _lib.ptr(prepared.buf),
-                prepared.buf.numel(), _lib.ptr(ws), ws.numel(), _lib.stream_ptr()))
+                prepared.buf.numel(), *_workspace_args(lib, device)))
             return out
         # long sequences (>= 65 536 bases, k = 6): tiles shared by the whole grid instead of one CTA per sequence
         n_long = int((seqset.lengths >= LONG_MIN).sum()) if (k == 6 and sidx is None and chunked is not False) else 0
@@ -203,18 +222,16 @@ def profiles(seqset, k, variants, out_kind=OUT_FREQ_F32, seed=0, out=None, out_o
             if nbytes > 0:
                 scratch = _workspace(device, nbytes, "chunk")
                 _lib.check(lib.idl_profiles_chunked(
-                    _lib.ptr(seqset.codes), _lib.ptr(seqset.nmask), _lib.ptr(seqset.chunk_off), _lib.ptr(seqset.len), seqset.n,
-                    None, n_items, int(seq_id0), k, varr, nv, _lib.ptr(sel), S, ctypes.c_uint64(seed & (2 ** 64 - 1)),
+                    *_seqset_args(seqset), None, n_items, int(seq_id0), k, varr, nv, _lib.ptr(sel), S, _seed(seed),
                     _lib.ptr(d_eoff), _lib.ptr(d_ent), out_kind, _lib.ptr(out), offs, int(out_stride), int(pseudocount),
                     1 if accumulate else 0, _lib.ptr(mean), _lib.ptr(scale), _lib.ptr(scratch), scratch.numel(), n_long,
-                    _lib.ptr(ws), ws.numel(), _lib.stream_ptr()))
+                    *_workspace_args(lib, device)))
                 return out
         _lib.check(lib.idl_profiles(
-            _lib.ptr(seqset.codes), _lib.ptr(seqset.nmask), _lib.ptr(seqset.chunk_off), _lib.ptr(seqset.len), seqset.n,
-            _lib.ptr(sidx), n_items, int(seq_id0), k, varr, nv, _lib.ptr(sel), S, ctypes.c_uint64(seed & (2 ** 64 - 1)),
+            *_seqset_args(seqset), _lib.ptr(sidx), n_items, int(seq_id0), k, varr, nv, _lib.ptr(sel), S, _seed(seed),
             _lib.ptr(d_eoff), _lib.ptr(d_ent), out_kind, _lib.ptr(out), offs, int(out_stride), int(pseudocount),
-            (1 if accumulate else 0) | ((int(cta_cap) & 0xFF) << 8), _lib.ptr(mean), _lib.ptr(scale), _lib.ptr(status), _lib.ptr(ws), ws.numel(),
-            _lib.stream_ptr()))
+            (1 if accumulate else 0) | ((int(cta_cap) & 0xFF) << 8), _lib.ptr(mean), _lib.ptr(scale), _lib.ptr(status),
+            *_workspace_args(lib, device)))
     return out
 
 
@@ -265,31 +282,22 @@ def profile_stats(seqset, k, variant, seed=0, seq_id0=0, edit_lists=None, group=
             pr = prepare(seqset, k, [variant], seed=seed, seq_id0=seq_id0, pseudocount=pseudocount, sidx=idx, buf=buf)
             buf = pr.buf
             parts.append(pr.parts.clone()); part_n.append(pr.part_n.clone())
-        parts, part_n = torch.cat(parts), torch.cat(part_n)
-        if group is not None:
-            parts, part_n = gather_partials(parts, part_n, group)
-        return Scaler.from_partials(parts, part_n)
+        return _scaler(torch.cat(parts), torch.cat(part_n), group)
     lib = _lib.load()
     device = seqset.device
     F = 4 ** k
-    max_parts = 2048
-    parts = torch.empty((max_parts, 2, F), dtype=torch.float64, device=device)
-    part_n = torch.zeros((max_parts,), dtype=torch.float64, device=device)
+    parts, part_n = _stats_buffers(F, device)
     varr = _variant_array([variant])
     n_parts = ctypes.c_int(0)
     d_eoff, d_ent = (None, None) if edit_lists is None else edit_lists
     with torch.cuda.device(device):
-        ws = _workspace(device, lib.idl_profiles_workspace_bytes(), "prof")
-        _lib.check(lib.idl_profile_stats(_lib.ptr(seqset.codes), _lib.ptr(seqset.nmask), _lib.ptr(seqset.chunk_off), _lib.ptr(seqset.len),
-                                         seqset.n, None, seqset.n, int(seq_id0), k, varr, ctypes.c_uint64(seed & (2 ** 64 - 1)),
+        _lib.check(lib.idl_profile_stats(*_seqset_args(seqset), None, seqset.n, int(seq_id0), k, varr, _seed(seed),
                                          _lib.ptr(d_eoff), _lib.ptr(d_ent), int(pseudocount), _lib.ptr(parts), _lib.ptr(part_n),
-                                         max_parts, ctypes.byref(n_parts), None, _lib.ptr(ws), ws.numel(), _lib.stream_ptr()))
+                                         MAX_PARTS, ctypes.byref(n_parts), None, *_workspace_args(lib, device)))
     parts, part_n = parts[: n_parts.value].contiguous(), part_n[: n_parts.value].contiguous()
     if seqset.n == 0:
         parts, part_n = torch.zeros((1, 2, F), dtype=torch.float64, device=device), torch.zeros((1,), dtype=torch.float64, device=device)
-    if group is not None:
-        parts, part_n = gather_partials(parts, part_n, group)
-    return Scaler.from_partials(parts, part_n)
+    return _scaler(parts, part_n, group)
 
 
 def kmer_counts_batch(seqset, k, counts=None):
@@ -299,10 +307,7 @@ def kmer_counts_batch(seqset, k, counts=None):
     if counts is None:
         counts = torch.empty((seqset.n, 4 ** k), dtype=torch.int32, device=seqset.device)
     with torch.cuda.device(seqset.device):
-        ws = _workspace(seqset.device, lib.idl_profiles_workspace_bytes(), "prof")
-        _lib.check(lib.idl_kmer_counts(_lib.ptr(seqset.codes), _lib.ptr(seqset.nmask), _lib.ptr(seqset.chunk_off),
-                                       _lib.ptr(seqset.len), seqset.n, k, _lib.ptr(counts), 1 if accumulate else 0,
-                                       _lib.ptr(ws), ws.numel(), _lib.stream_ptr()))
+        _lib.check(lib.idl_kmer_counts(*_seqset_args(seqset), k, _lib.ptr(counts), 1 if accumulate else 0, *_workspace_args(lib, seqset.device)))
     return counts
 
 
@@ -403,10 +408,7 @@ class Scaler(object):
         """Statistics of x's columns.  group=None: this process only.  With a torch.distributed
         group the per-rank partials are all-gathered (rank order) and merged identically on
         every rank (a collective: every rank of the group must call it)."""
-        parts, part_n = cls.partials(x)
-        if group is not None:
-            parts, part_n = gather_partials(parts, part_n, group)
-        return cls.from_partials(parts, part_n)
+        return _scaler(*cls.partials(x), group)
 
     def transform32(self, x, out=None):
         lib = _lib.load()
