@@ -6,11 +6,11 @@ Reference surface mirrored (idelucs/__init__.py:3-8): ``check_sequence``, ``Summ
 ``cgr``, ``IID_model``, ``IID_loss``, ``info_nce_loss``, ``iDeLUCS_cluster`` (``PlotPolygon`` / ``define_ToolTips`` are GUI / plot
 helpers and out of scope).
 Submodules keep the reference's names: ``kmers``, ``utils``, ``LossFunctions``, ``models``,
-``cluster``.  Nothing here falls back to a CPU implementation.
+``cluster``.  ``hdbscan_device`` is sklearn's HDBSCAN with its all-pairs work on the GPU.  Nothing here falls back to a CPU implementation.
 """
 __version__ = (0, 1, 0)
 
-__all__ = ["kmers", "utils", "LossFunctions", "models", "cluster", "seqset", "featurise"]
+__all__ = ["kmers", "utils", "LossFunctions", "models", "cluster", "seqset", "featurise", "hdbscan"]
 
 
 def __getattr__(name):  # lazy: importing the package must not require torch.cuda to be usable
@@ -33,6 +33,7 @@ def __getattr__(name):  # lazy: importing the package must not require torch.cud
         "info_nce_loss": ("LossFunctions", "info_nce_loss"),
         "IID_model": ("models", "IID_model"),
         "iDeLUCS_cluster": ("cluster", "iDeLUCS_cluster"),
+        "hdbscan_device": ("hdbscan", "hdbscan_device"),
     }
     if name in lazy:
         mod, attr = lazy[name]

@@ -1,7 +1,8 @@
 """``python -m idelucs_b200`` — the reference CLI surface (idelucs/__main__.py:274-318: same
 flags and defaults) driving the B200-native hot path.  Orchestration only: voters x epochs,
 majority vote over voters (k-means on one-hot votes, utils.py:582-602) or HDBSCAN on the latent space when
---n_clusters=0 (the ``hdbscan`` package if importable, else scikit-learn's implementation), metrics and TSV output."""
+--n_clusters=0 (the ``hdbscan`` package if importable, else scikit-learn's algorithm with its all-pairs work on the GPU,
+``hdbscan.hdbscan_device``), metrics and TSV output."""
 import argparse
 import os
 import sys
@@ -36,7 +37,7 @@ def run(args):
         voter_min = np.inf
         for _ in range(args["n_epochs"]):
             voter_min = min(voter_min, model.contrastive_training_epoch())
-        y_pred, probabilities, latent = model.predict()
+        y_pred, probabilities, latent = model.predict(device_latent=use_hdbscan)
         if voter_min < min_loss:
             min_loss, model_latent = voter_min, latent
         if not use_hdbscan:   # relabel in order of first appearance (__main__.py:131-141)
@@ -48,13 +49,14 @@ def run(args):
         msz = len(model.names) // 100 + 1
         try:
             import hdbscan
+        except ImportError:   # scikit-learn's HDBSCAN with its all-pairs work on the GPU (same results as sklearn.cluster.HDBSCAN)
+            from .hdbscan import hdbscan_device
+            labels, probabilities = hdbscan_device(latent, max(msz, 2))
+        else:
             clusterer = hdbscan.HDBSCAN(min_cluster_size=msz, gen_min_span_tree=True, prediction_data=True)
-        except ImportError:   # same algorithm from scikit-learn (>= 1.3) when the hdbscan package is not installed
-            from sklearn.cluster import HDBSCAN
-            clusterer = HDBSCAN(min_cluster_size=max(msz, 2))
-        clusterer.fit(latent)
-        y_pred = clusterer.labels_ + 1
-        probabilities = clusterer.probabilities_
+            clusterer.fit(latent.cpu().numpy().astype(np.float64))
+            labels, probabilities = clusterer.labels_, clusterer.probabilities_
+        y_pred = labels + 1
         args["n_clusters"] = int(np.max(y_pred)) + 1
     else:
         y_pred, probabilities = label_features(np.array(predictions), args["n_clusters"])

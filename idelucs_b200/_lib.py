@@ -81,6 +81,9 @@ PROTOTYPES = {
                                       c_void_p]),
     "idl_iid_loss_scaled": (c_int, [c_void_p, c_void_p, c_int, c_int, c_float, c_float, c_float, c_float, c_void_p, c_float, c_void_p, c_void_p,
                                     c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]),
+    "idl_hdbscan_workspace_bytes": (c_size_t, [c_i64, c_int]),
+    "idl_core_distances": (c_int, [c_void_p, c_i64, c_int, c_i64, c_void_p, c_void_p, c_size_t, c_void_p]),
+    "idl_mreach_mst": (c_int, [c_void_p, c_void_p, c_i64, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]),
 }
 
 _lib = None

@@ -107,8 +107,9 @@ class IID_model(object):
             self._test = SequenceDataset(self.sequence_file, k=self.k, transform=None, GT_file=self.GT_file, reduce=self.reduce)
         return self._test
 
-    def predict(self, data=None):
-        """idelucs/models.py:145-172 -> (y_pred int[N], probabilities float[N], latent float[N,64])"""
+    def predict(self, data=None, device_latent=False):
+        """idelucs/models.py:145-172 -> (y_pred int[N], probabilities float[N], latent float[N,64]); with device_latent the
+        latent stays on the device as the float32 tensor the network produced (what hdbscan_device takes)"""
         x = self._test_set().kmers32
         y_pred, probs, latent = [], [], []
         with torch.no_grad():
@@ -119,8 +120,9 @@ class IID_model(object):
                 y_pred.append(pred)
                 probs.append(p)
                 latent.append(lat)
+        latent = torch.cat(latent)
         return (torch.cat(y_pred).cpu().numpy(), torch.cat(probs).cpu().numpy().astype(np.float64),
-                torch.cat(latent).cpu().numpy().astype(np.float64))
+                latent if device_latent else latent.cpu().numpy().astype(np.float64))
 
     def calculate_probs(self, data=None):
         """idelucs/models.py:175-195 -> float[N, n_clusters]"""

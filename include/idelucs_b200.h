@@ -326,6 +326,26 @@ int idl_fasta_scan(const uint8_t* buf, int64_t nbytes, int64_t* n_records, int64
 int idl_fasta_extract(const uint8_t* buf, int64_t nbytes, int64_t n_records, uint8_t* seq_out, int64_t seq_cap,
                       int64_t* byte_off, int64_t* hdr_off, int64_t* hdr_len);
 
+/* F3 — the all-pairs part of HDBSCAN (sklearn.cluster.HDBSCAN, Euclidean metric, alpha = 1), which the reference runs on
+ * the latent vectors for --n_clusters 0 (idelucs/__main__.py:149-156).  d_x: float32 [n, D] row-major.  Distances are
+ * computed exactly as sklearn does: the inputs widened to double, sum of (x_i[t] - x_j[t])^2 in order t = 0..D-1 with
+ * every operation rounded on its own (no FMA), IEEE sqrt; results compare with sklearn's by ==.  d_ws:
+ * idl_hdbscan_workspace_bytes(n, D) bytes (0 for n outside 1..2^31-1 or D < 1), 16-byte aligned, shared by both calls.
+ * Memory is O(n D): no n x n matrix is stored, every pass recomputes the distances.
+ * idl_core_distances: d_core[i] = the k-th smallest of the n distances d(i, .), counting d(i, i) = 0 and duplicates with
+ *   multiplicity (NearestNeighbors.kneighbors(X, k)[0][:, -1]; sklearn's min_samples is k), 1 <= k <= n.  A radix select
+ *   over the bit patterns of the squared distances: at most 9 launches, no host synchronisation.
+ * idl_mreach_mst: the minimum spanning tree of the complete graph w(i, j) = max(d_core[i], d_core[j], d(i, j)) (sklearn's
+ *   mst_from_data_matrix), with ties broken by (w, min(i, j), max(i, j)), so the tree is unique.  d_src, d_dst int64[n-1] and
+ *   d_w double[n-1] receive its edges in the order Borůvka finds them (not sorted by weight), each oriented away from point 0
+ *   (d_src is the endpoint on the path to point 0) as sklearn's Prim, grown from point 0, emits them.  The call
+ *   SYNCHRONISES `stream` once per Borůvka round (at most ceil(log2 n) rounds: the components are merged on the host) and
+ *   before it returns. */
+size_t idl_hdbscan_workspace_bytes(int64_t n, int D);
+int idl_core_distances(const float* d_x, int64_t n, int D, int64_t k, double* d_core, void* d_ws, size_t ws_bytes, void* stream);
+int idl_mreach_mst(const float* d_x, const double* d_core, int64_t n, int D, int64_t* d_src, int64_t* d_dst, double* d_w, void* d_ws,
+                   size_t ws_bytes, void* stream);
+
 #ifdef __cplusplus
 }
 #endif
