@@ -6,7 +6,7 @@ import ctypes
 import os
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
-# (IDELUCS_B200_LIB: a differently built library, e.g. the -DIDL_DEVTOOLS variant the profiling tools use)
+# (IDELUCS_B200_LIB: load a differently built library instead, e.g. to compare two builds with tools/stats_identity.py)
 LIB_PATH = os.environ.get("IDELUCS_B200_LIB") or os.path.join(_HERE, "lib", "libidelucs_b200.so")
 
 IDL_OK = 0

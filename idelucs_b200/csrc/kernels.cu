@@ -86,26 +86,15 @@ struct ProfParams {
     const float* rscale;  // 1/scale (IEEE), computed into the workspace by rscale_kernel
     int32_t* status;
     unsigned long long* work_counter;
-    unsigned long long* phase_prof;   // optional: cycles per kernel phase summed over CTAs (thread 0), IDL_PHASE_PROF=1
     int only_deferred;                // generic kernel: redo only the items the producer/consumer kernel flagged (status bit 1)
     double* stats_partials;           // OUT_STATS: per-CTA (mean, M2) [gridDim][2][4^k]
     double* stats_n;                  // OUT_STATS: per-CTA row count [gridDim]
-    int dbg;                          // development switches of the producer/consumer kernel (IDL_PC_DBG; builds with -DIDL_DEVTOOLS only)
     int inline_plan;                  // descriptors / offsets / tables come from the Plan kernel parameter (else from vars / out_off / gtab)
     void* prep;                       // prepared buffer (prep.cuh): written by prep_kernel, read by colstats16 / the producer/consumer kernel
     unsigned long long prep_stamp;    // what the prepared buffer must have been prepared for
     const int* long_overflow;         // chunked path active (chunked.cuh): items of >= CH_MIN_LEN bases are skipped here while *long_overflow == 0
 };
 static_assert(sizeof(ProfParams) + sizeof(Plan) <= 4000, "kernel parameters must stay below the 4 KB limit");
-
-// development aids are compiled out of release builds
-#ifdef IDL_DEVTOOLS
-#define IDL_DBG(p) ((p).dbg)
-#define IDL_PROF(p) ((p).phase_prof)
-#else
-#define IDL_DBG(p) 0
-#define IDL_PROF(p) (static_cast<unsigned long long*>(nullptr))
-#endif
 
 constexpr int OUT_STATS = 4;          // internal out kind: column statistics of slot 0's float32 frequencies, nothing is written per row
 
@@ -522,25 +511,11 @@ __device__ __noinline__ void long_path(ProfSmem<K, NT>& sm, const ProfParams& p,
     }
 }
 
-// development aid (IDL_PHASE_PROF=1): thread 0 attributes its elapsed cycles to kernel phases
-struct PhaseClock {
-    unsigned long long* base;
-    long long t_prev;
-    __device__ __forceinline__ void tick(int id) {
-        if (base && threadIdx.x == 0) {
-            const long long t = clock64();
-            atomicAdd(base + id, (unsigned long long)(t - t_prev));
-            t_prev = t;
-        }
-    }
-};
-
 // CTA-wide prep of the Bernoulli / explicit / big-Random_N slots of one group (short path):
 // patches the private copies and accumulates sm.dtot.  Contains barriers (uniform control flow).
 template <int K, int NT>
 __device__ __noinline__ void prep_cta_slots(ProfSmem<K, NT>& sm, const ProfParams& p, const ItemCtx& cx, const VarDesc* vars, int s0,
-                                            long long item, long long seq, unsigned bern_mask, unsigned other_mask, int* dtot,
-                                            int copy0, PhaseClock& pc) {
+                                            long long item, long long seq, unsigned bern_mask, unsigned other_mask, int* dtot, int copy0) {
     using C = ProfCfg<K, NT>;
     constexpr int PRIVW = C::PRIVW;
     const int tid = threadIdx.x, lane = tid & 31;
@@ -561,17 +536,14 @@ __device__ __noinline__ void prep_cta_slots(ProfSmem<K, NT>& sm, const ProfParam
         if (active)
             m = block_masks(vd.kind, cx.seed, cx.seq_id, (uint32_t)vd.rng_id, b, L, cx.nmask, gap_table(sm, p, vd.tab1), vd.slope1,
                             gap_table(sm, p, vd.tab2), vd.slope2);
-        pc.tick(7);
         int total;
         const int off = block_exscan<NT>(block_masks_count(m), sm.scan, &total);
-        pc.tick(8);
         if (total <= LIST_CAP) {  // uniform
             bern_done = true;
             if (active && b == 0) sm.seg_off[j] = off;
             if (tid == 0) sm.seg_off[nb] = total;
             block_masks_write(m, b, cx.codes, sm.list + off);
             __syncthreads();
-            pc.tick(9);
             for (int i = tid; i < total; i += NT) {
                 int jj = 0;
                 while (i >= sm.seg_off[jj + 1]) ++jj;
@@ -580,9 +552,7 @@ __device__ __noinline__ void prep_cta_slots(ProfSmem<K, NT>& sm, const ProfParam
                 const int d = apply_priv<K>(cx, sm.list + so, sm.seg_off[jj + 1] - so, i - so, priv + cc * PRIVW);
                 if (d) atomicAdd(&dtot[cc], d);
             }
-            pc.tick(10);
             __syncthreads();
-            pc.tick(11);
         }
     }
     // ---- remaining CTA-wide slots, one after the other ----
@@ -640,10 +610,6 @@ __global__ void __launch_bounds__(NT, (K == 6 ? 2 : K == 5 ? 4 : 8)) profiles_ke
     const VarDesc* __restrict__ vars = cached ? sm.svars : p.vars;
     const long long* __restrict__ out_offs = cached ? sm.sout_off : reinterpret_cast<const long long*>(p.out_off);
 
-    PhaseClock pclk;
-    pclk.base = IDL_PROF(p);
-    pclk.t_prev = IDL_PROF(p) ? clock64() : 0;
-    auto phase = [&](int id) { pclk.tick(id); };
     // OUT_STATS: shifted-data column sums of this CTA's rows (shift = first row seen), float64
     double acc1[VPT][4], acc2[VPT][4];
     float shiftK[VPT][4];
@@ -740,7 +706,6 @@ __global__ void __launch_bounds__(NT, (K == 6 ? 2 : K == 5 ? 4 : 8)) profiles_ke
         __syncthreads();
         const int base_total = F * p.pseudocount + sm.nvalid;
         if (staged) { cx.codes = sm.sseq; cx.nmask = sm.sseq + SSEQ_CW; }  // every later lookup hits shared memory
-        phase(0);
 
         if (OUT == OUT_STATS) {
             // ---- statistics mode: patch hist[] in place with slot 0's deltas, accumulate, next item ----
@@ -829,7 +794,6 @@ __global__ void __launch_bounds__(NT, (K == 6 ? 2 : K == 5 ? 4 : 8)) profiles_ke
                 }
             }
         }
-        phase(1);
 
         for (int S0 = 0; S0 < p.S;) {
             // ======== supergroup: up to SG slots; their Random_N removals are precomputed together ========
@@ -867,7 +831,6 @@ __global__ void __launch_bounds__(NT, (K == 6 ? 2 : K == 5 ? 4 : 8)) profiles_ke
             }
             __syncthreads();
             const int NSg = sm.sg_n;
-            phase(12);
             // ---- (p1) draws of every small Random_N slot: thread <-> (slot, philox call).  The slot id
             // ---- rides in bits 27..31 of the entry (positions are < 2^16 on this path) ----
             for (int q = tid; q < NSg * 8; q += NT) {
@@ -882,7 +845,6 @@ __global__ void __launch_bounds__(NT, (K == 6 ? 2 : K == 5 ? 4 : 8)) profiles_ke
                 }
             }
             __syncthreads();
-            phase(13);
             // ---- (p2) removed windows of every draw: thread <-> draw (dense over all slots); draw q
             // ---- owns rem[q*K .. +K), unused entries hold 0xFFFF (random_n_removals' rule, core.cuh) ----
             {
@@ -930,7 +892,6 @@ __global__ void __launch_bounds__(NT, (K == 6 ? 2 : K == 5 ? 4 : 8)) profiles_ke
                 }
             }
             __syncthreads();
-            phase(14);
             for (int c = wid; c < NSg; c += NT / 32) {  // totals of the slots whose deltas are known now: warp <-> slot
                 int d = 0;
                 if (sm.pre_kind[c] == 1) {
@@ -946,7 +907,6 @@ __global__ void __launch_bounds__(NT, (K == 6 ? 2 : K == 5 ? 4 : 8)) profiles_ke
                 }
             }
             // (visible to the streamers after the barrier that follows the first patch phase)
-            phase(2);
 
             // ---- half-groups of HG slots, two sets of private copies: the removals of the NEXT
             // ---- half-group are subtracted (fire-and-forget shared atomics) while the current one streams
@@ -967,18 +927,16 @@ __global__ void __launch_bounds__(NT, (K == 6 ? 2 : K == 5 ? 4 : 8)) profiles_ke
             };
             auto prep_half = [&](int h0, int hs, int set) {  // CTA-wide slots of a half-group (contains barriers)
                 const unsigned bm = (sm.mask_bern >> h0) & ((1u << HG) - 1u), om = (sm.mask_other >> h0) & ((1u << HG) - 1u);
-                prep_cta_slots<K, NT>(sm, p, cx, vars, S0 + h0, item, seq, bm, om, sm.dtot + h0, set * HG, pclk);
+                prep_cta_slots<K, NT>(sm, p, cx, vars, S0 + h0, item, seq, bm, om, sm.dtot + h0, set * HG);
                 if (tid < hs && sm.pre_kind[h0 + tid] >= 2) {
                     const float ft2 = (float)(base_total + sm.dtot[h0 + tid]);
                     sm.gy[h0 + tid] = make_float2(ft2, 1.0f / ft2);
                 }
-                phase(3);
             };
             const int nh = (NSg + HG - 1) / HG;
             if ((cta_mask & ((1u << HG) - 1u)) != 0u) { __syncthreads(); prep_half(0, NSg < HG ? NSg : HG, 0); }
             patch_half(0, NSg < HG ? NSg : HG, 0);
             __syncthreads();
-            phase(4);
             for (int h = 0; h < nh; ++h) {
                 const int cur = h & 1, h0 = h * HG;
                 const int hs = NSg - h0 < HG ? NSg - h0 : HG;
@@ -1014,12 +972,10 @@ __global__ void __launch_bounds__(NT, (K == 6 ? 2 : K == 5 ? 4 : 8)) profiles_ke
                     }
                 }
                 __syncthreads();
-                phase(5);
                 if (next_cta) {
                     prep_half(h0 + HG, hs_next, cur ^ 1);
                     patch_half(h0 + HG, hs_next, cur ^ 1);
                     __syncthreads();
-                    phase(4);
                 }
             }
             S0 += NSg;
@@ -1311,8 +1267,7 @@ constexpr int MAX_TABS = 64;
 constexpr size_t WS_OUTOFF = WS_VARS + sizeof(VarDesc) * MAX_VARIANTS;
 constexpr size_t WS_GTAB = WS_OUTOFF + sizeof(int64_t) * MAX_VARIANTS;
 constexpr size_t WS_RSCALE = WS_GTAB + sizeof(uint32_t) * RNG_BLOCK * MAX_TABS;
-constexpr size_t WS_PROF = WS_RSCALE + sizeof(float) * 4096;
-constexpr size_t WS_TOTAL = WS_PROF + 8 * 16;  // 16 phase counters (development builds)
+constexpr size_t WS_TOTAL = WS_RSCALE + sizeof(float) * 4096;
 
 // the instantiation of a kernel template for an output kind (nullptr for an unknown kind)
 template <typename Kernel>
@@ -1473,11 +1428,6 @@ static int fill_params(ProfParams& p, const ProfCall& c, const HostPlan& hp) {
     p.work_counter = reinterpret_cast<unsigned long long*>(c.ws);
     p.inline_plan = hp.inl ? 1 : 0;
     p.stats_partials = c.stats_partials; p.stats_n = c.stats_n;
-#ifdef IDL_DEVTOOLS
-    static const bool want_prof = getenv("IDL_PHASE_PROF") != nullptr;
-    p.phase_prof = want_prof ? reinterpret_cast<unsigned long long*>(c.ws + WS_PROF) : nullptr;
-    { const char* e = getenv("IDL_PC_DBG"); p.dbg = e ? atoi(e) : 0; }
-#endif
     return IDL_OK;
 }
 

@@ -13,7 +13,7 @@
 //     so the slot-0 mutations are generated once for the statistics AND the profile pass.
 //
 // One CTA of 256 threads per sequence at a time, 4 CTAs per SM (51 KB of shared memory each): count the clean
-// histogram into packed uint16 counters (shared atomics), mutation masks of every (slot, 64-base block) by
+// histogram into int32 bins (shared atomics), mutation masks of every (slot, 64-base block) by
 // the register-only mask generator (core.cuh), CTA scan -> position-sorted edit lists -> +-1 deltas
 // (apply_entry), slot 0's deltas applied to the histogram.  Sequences that do not fit (longer than
 // 20 480 bases, list overflows at rates far above the reference's) are flagged (meta.flags, d_status bit 1)
@@ -22,26 +22,13 @@
 
 namespace idl {
 
-#ifndef PR_PACKED
-#define PR_PACKED 0                        // 0: int32 bins, 4 CTAs/SM (0.70 ms per 20 000 sequences); 1: uint16-pair histogram + 1024-entry edit list,
-                                           //    39 KB of shared memory, 5 CTAs/SM — measured slower (0.74 ms: packed updates + the 48-register cap)
-#endif
-#ifndef PR_NT_N
-#define PR_NT_N 256
-#endif
-#ifndef PR_MINB_N
-#define PR_MINB_N (PR_PACKED ? 5 : 4)
-#endif
-constexpr int PR_NT = PR_NT_N;
-constexpr int PR_LIST = PR_PACKED ? 1024 : 2048;   // edits of all dense slots of one sequence
-constexpr int PR_MINB = PR_MINB_N;
+// int32 bins, 4 CTAs/SM: a uint16-pair histogram fits 5 CTAs/SM but measured slower (profiles/README.md)
+constexpr int PR_NT = 256;
+constexpr int PR_MINB = 4;
+constexpr int PR_LIST = 2048;   // edits of all dense slots of one sequence
 
 struct PrSmem {
-#if PR_PACKED
-    alignas(16) uint32_t hist[PC_F / 2];      // clean histogram, then slot 0's: two uint16 counters per word
-#else
     alignas(16) int hist[PC_F];               // clean histogram, then slot 0's (packed to uint16 on the way out)
-#endif
     alignas(16) uint32_t sseq[2][PC_SSEQ_W];  // staged sequences (codes | mask): the next item's words arrive (cp.async) while this one is processed
     alignas(16) uint32_t list[PR_LIST + 8];
     alignas(16) uint16_t delta[PC_DELTA];
@@ -65,17 +52,9 @@ template <int N> __device__ __forceinline__ void cp_async_wait() { asm volatile(
 
 // counts the windows ending in the 16-base code word u of a staged sequence (idelucs/kmers.pyx:36-47) with shared atomics
 // (ATOMS.POPC.INC); returns how many were counted.  Thread <-> word: a 10 kb sequence is 628 work items (2.5 rounds of 256 threads).
-#if PR_PACKED
-__device__ __forceinline__ void pr_bump(uint32_t* hist, uint32_t kmer, int d) {   // +-1 on a packed counter (the sum of all updates never leaves [0, 65535])
-    if (d > 0) atomicAdd(&hist[kmer >> 1], 1u << ((kmer & 1u) * 16u)); else atomicSub(&hist[kmer >> 1], 1u << ((kmer & 1u) * 16u));
-}
-using PrHist = uint32_t;
-#else
 __device__ __forceinline__ void pr_bump(int* hist, uint32_t kmer, int d) { atomicAdd(&hist[kmer], d); }
-using PrHist = int;
-#endif
 template <int K>
-__device__ __forceinline__ int pr_count_word(const uint32_t* codes, const uint32_t* nmask, int u, PrHist* hist) {
+__device__ __forceinline__ int pr_count_word(const uint32_t* codes, const uint32_t* nmask, int u, int* hist) {
     constexpr uint32_t KMASK = (1u << (2 * K)) - 1u;
     const uint32_t w = codes[u], prev = u > 0 ? codes[u - 1] : 0u;
     const uint32_t m = nmask[u >> 1], mprev = u > 1 ? nmask[(u >> 1) - 1] : 0xFFFFFFFFu;   // sequence start = preceded by resets (kmers.pyx:14)
@@ -192,7 +171,7 @@ __global__ void __launch_bounds__(PR_NT, PR_MINB) prep_kernel(const ProfParams p
         }
         __syncthreads();                               // ... and everybody else's; histogram cleared
         if (!defer) {
-            // ---- clean histogram (idelucs/kmers.pyx:38-50), two uint16 counters per word ----
+            // ---- clean histogram (idelucs/kmers.pyx:38-50) ----
             {
                 int nv = 0;
                 for (int u = tid; u < nchunks * 4; u += PR_NT) nv += pr_count_word<K>(codes, nmask, u, sm.hist);
@@ -309,15 +288,11 @@ __global__ void __launch_bounds__(PR_NT, PR_MINB) prep_kernel(const ProfParams p
         } else {
             // ---- hand over: slot 0's histogram, the delta list, the totals ----
             const int n_delta = sm.n_delta;
-#if PR_PACKED
-            for (int i = tid; i < PC_F / 8; i += PR_NT) hist_out[(size_t)item * (PC_F / 8) + i] = reinterpret_cast<const uint4*>(sm.hist)[i];
-#else
             for (int i = tid; i < PC_F / 8; i += PR_NT) {   // 8 bins -> one 16-byte store of uint16 counts (every count <= 20 480)
                 const int4 lo = reinterpret_cast<const int4*>(sm.hist)[2 * i], hi = reinterpret_cast<const int4*>(sm.hist)[2 * i + 1];
                 hist_out[(size_t)item * (PC_F / 8) + i] = make_uint4((uint32_t)lo.x | ((uint32_t)lo.y << 16), (uint32_t)lo.z | ((uint32_t)lo.w << 16),
                                                                      (uint32_t)hi.x | ((uint32_t)hi.y << 16), (uint32_t)hi.z | ((uint32_t)hi.w << 16));
             }
-#endif
             const int nq = (n_delta * 2 + 15) >> 4;
             for (int i = tid; i < nq; i += PR_NT) delta_out[(size_t)item * (PC_DELTA / 8) + i] = reinterpret_cast<const uint4*>(sm.delta)[i];
             if (tid == 0) {

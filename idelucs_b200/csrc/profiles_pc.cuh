@@ -38,13 +38,7 @@ constexpr int PC_NBLD = 256;       // builder threads (warps 0..7)
 constexpr int PC_NFIX = 224;       // fix threads (warps 8..14); warp 15 lane 0 is the store thread
 constexpr int PC_NBUF = 4;         // 16 KB row buffers
 constexpr int PC_NOTH = 1;         // row buffers that take the "other" jobs (dense rows, minority window totals) while the rest stream the main total
-#ifndef PC_TIGHT
-#define PC_TIGHT 0
-#endif
-#ifndef PC_INFL_N
-#define PC_INFL_N (PC_NBUF - 2)
-#endif
-constexpr int PC_INFL = PC_INFL_N;   // bulk copies kept in flight besides the one just issued
+constexpr int PC_INFL = PC_NBUF - 2;   // bulk copies kept in flight besides the one just issued
 constexpr int PC_FIXW = PC_NFIX / 32;   // fix warps: each owns a 4 KB scratch (biased uint8 deltas) and handles whole jobs
 constexpr int PC_SCRW = 1024;      // words of one fix-warp scratch (four bins per word)
 constexpr uint32_t PC_BIAS4 = 0x80808080u;
@@ -171,15 +165,6 @@ __device__ __forceinline__ void fence_proxy_async_smem() { asm volatile("fence.p
 __device__ __forceinline__ void bulk_store(void* gdst, const void* ssrc, uint32_t bytes) {
     asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" ::"l"(gdst), "r"(smem_u32(ssrc)), "r"(bytes) : "memory");
 }
-__device__ __forceinline__ void bulk_store_hint(void* gdst, const void* ssrc, uint32_t bytes, unsigned long long policy) {
-    asm volatile("cp.async.bulk.global.shared::cta.bulk_group.L2::cache_hint [%0], [%1], %2, %3;" ::"l"(gdst), "r"(smem_u32(ssrc)), "r"(bytes), "l"(policy)
-                 : "memory");
-}
-__device__ __forceinline__ unsigned long long policy_evict_first() {
-    unsigned long long pol;
-    asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(pol));
-    return pol;
-}
 __device__ __forceinline__ void mbar_expect_tx(unsigned long long* bar, uint32_t bytes) {
     asm volatile("{\n.reg .b64 st;\nmbarrier.arrive.expect_tx.shared::cta.b64 st, [%0], %1;\n}" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
 }
@@ -208,10 +193,6 @@ __device__ __noinline__ void pc_producer(PcSmem& sm) {
     const ProfParams& p = sm.params;
     constexpr int K = PC_K;
     const int ptid = threadIdx.x - PC_HALF, lane = ptid & 31;
-    long long t_prev = IDL_PROF(p) ? clock64() : 0;
-    auto tick = [&](int id) {
-        if (IDL_PROF(p) && ptid == 0) { const long long t = clock64(); atomicAdd(IDL_PROF(p) + id, (unsigned long long)(t - t_prev)); t_prev = t; }
-    };
     // Items are dispatched by the store thread into a small ring (index, first chunk, length) and the
     // packed words of item A_{i+1} are TMA-loaded into the other half of sseq while A_i is prepared:
     // no global-load latency (~3k cycles under the saturated write stream) and no long-lived
@@ -252,7 +233,6 @@ __device__ __noinline__ void pc_producer(PcSmem& sm) {
         const int nx_phase = b ? n_loads0 : n_loads1;
         if (loads_seq(nx_item, nx_L)) { if (b) ++n_loads0; else ++n_loads1; }
         mbar_wait(&sm.ctx_empty[b], ((it >> 1) & 1) ^ 1);   // every consumer role is done with the previous occupant
-        tick(5);
         const long long item = cur_item;
         if (item >= p.n_items) {
             if (ptid == 0) { cx.item = -1; mbar_arrive(&sm.ctx_full[b]); }
@@ -298,7 +278,6 @@ __device__ __noinline__ void pc_producer(PcSmem& sm) {
             nv = warp_sum(nv);
             if (lane == 0 && nv) atomicAdd(&sm.nvalid, nv);
             bar_named(1, PC_HALF);
-            tick(2);
             if (ptid == 0) cx.base_total = PC_F * p.pseudocount + sm.nvalid;
             // ---- Random_N slots: draws (thread <-> slot, philox call) ----
             const int n_ent = sm.n_ent;   // <= PC_LIST (host-checked)
@@ -362,7 +341,6 @@ __device__ __noinline__ void pc_producer(PcSmem& sm) {
                 }
                 bar_named(1, PC_HALF);
             }
-            tick(3);
             // ---- Bernoulli slots: their window totals come from the prepare pass ----
             if (ptid < sm.n_bern) cx.dtot[sm.bern_slot[ptid]] = ptid == 0 ? cur_m1.x : (ptid == 1 ? cur_m1.y : cur_m1.z);
             bar_named(1, PC_HALF);
@@ -412,11 +390,10 @@ __device__ __noinline__ void pc_producer(PcSmem& sm) {
         }
         const int O = S - M, a = gj0 % PC_NBUF;
         // (the first round of buffers is all main: the main row is the cheapest to have ready at the start of a sequence)
-        const int noth = (IDL_DBG(p) & 64) ? 0 : PC_NOTH;
-        auto lane_type = [&](int q) { return (a + q) % PC_NBUF >= PC_NBUF - noth; };
+        auto lane_type = [&](int q) { return (a + q) % PC_NBUF >= PC_NBUF - PC_NOTH; };
         auto other_type = [&](int q) { return q >= PC_NBUF && lane_type(q); };
         auto lanes_before = [&](int q) {
-            int f = (q / PC_NBUF) * noth;
+            int f = (q / PC_NBUF) * PC_NOTH;
             for (int r = q - q % PC_NBUF; r < q; ++r) f += lane_type(r) ? 1 : 0;
             return f;
         };
@@ -454,7 +431,6 @@ __device__ __noinline__ void pc_producer(PcSmem& sm) {
         }
         if (!cx.defer) gj0 += S;
         cur_item = nx_item; cur_seq = nx_seq; cur_c0 = nx_c0; cur_L = nx_L; cur_phase = nx_phase; cur_m0 = nx_m0; cur_m1 = nx_m1;
-        tick(4);
         bar_named(1, PC_HALF);
         if (ptid == 0) mbar_arrive(&sm.ctx_full[b]);   // release: hand the context over to the consumers
     }
@@ -481,16 +457,6 @@ __device__ __forceinline__ void cvt_granule(uint2 pk, float magic, float2& c01, 
     c23 = make_float2(__uint_as_float(__byte_perm(pk.y, 0x4B000000u, 0x7410)), __uint_as_float(__byte_perm(pk.y, 0x4B000000u, 0x7432)));
     c01 = __fadd2_rn(c01, nmag); c23 = __fadd2_rn(c23, nmag);                    // exact count + pseudocount
 }
-
-// development aid (IDL_PHASE_PROF=1): one thread of a role attributes its elapsed cycles to phases
-struct PcClock {
-    unsigned long long* base;
-    long long t_prev;
-    __device__ __forceinline__ void start(unsigned long long* b) { base = b; t_prev = b ? clock64() : 0; }
-    __device__ __forceinline__ void tick(int id) {
-        if (base) { const long long t = clock64(); atomicAdd(base + id, (unsigned long long)(t - t_prev)); t_prev = t; }
-    }
-};
 
 // RN(1/x) from the hardware approximation and the per-bin ulp correction computed in the kernel prologue
 __device__ __forceinline__ float rcp_approx(float x) {
@@ -527,13 +493,9 @@ __device__ __forceinline__ void pc_builder(PcSmem& sm, const ProfParams& p) {
     const int tid = threadIdx.x;
     const float magic = 8388608.0f - (float)p.pseudocount;
     int gj0 = 0;                                     // jobs of the previous sequences (CTA lifetime)
-    PcClock clk;
-    clk.start(tid == 0 && (IDL_DBG(p) & 16) ? IDL_PROF(p) : nullptr);
     for (int it = 0;; ++it) {
         const int b = it & 1;
-        clk.tick(13);
         mbar_wait(&sm.ctx_full[b], (it >> 1) & 1);
-        clk.tick(12);
         PcCtx& cx = sm.ctx[b];
         const long long item = cx.item;
         if (item < 0) return;
@@ -588,10 +550,8 @@ __device__ __forceinline__ void pc_builder(PcSmem& sm, const ProfParams& p) {
                         val[g] = finish_granule2<STD>(d01, d23, fy, smem_stats2<STD>(sm, vec));
                     }
                 }
-                clk.tick(13);
                 // the bulk copy of the buffer's previous job has been read (counter = truth, the mbarrier is only the way to sleep)
                 while (ld_acquire_smem(&sm.free_count[buf]) < use) mbar_try_once(&sm.row_free[buf], (use & 1) ^ 1);
-                clk.tick(14);
                 float4* row = reinterpret_cast<float4*>(sm.rowbuf[buf]);
 #pragma unroll
                 for (int g = 0; g < GPT; ++g) row[tid + g * NB] = val[g];
@@ -607,7 +567,6 @@ __device__ __forceinline__ void pc_builder(PcSmem& sm, const ProfParams& p) {
 // STORE thread (warp 15, lane 0): dispatches the items and writes each job's row with one TMA bulk copy
 __device__ __forceinline__ void pc_store(PcSmem& sm, const ProfParams& p) {
     int gj = 0;
-    const unsigned long long pol_ef = policy_evict_first();
     // ---- dispatcher.  The atomic and the dependent loads of (sequence, length, first chunk) are two global
     // round trips; they are issued one iteration before their results are needed, and a stall here is absorbed
     // by the rows the other roles have already finished.
@@ -639,17 +598,13 @@ __device__ __forceinline__ void pc_store(PcSmem& sm, const ProfParams& p) {
     long long b_item = 0, b_seq = 0, b_c0 = 0;
     int b_L = 0;
     int4 b_m0 = make_int4(0, 0, 0, 1), b_m1 = make_int4(0, 0, 0, 0);
-    PcClock clk;
-    clk.start((IDL_DBG(p) & 48) ? IDL_PROF(p) : nullptr);
     for (int it = 0;; ++it) {
         const int b = it & 1;
         if (it >= 1) publish(it + 3, b_item, b_seq, b_c0, b_L, b_m0, b_m1);      // loaded during the previous iteration
         b_item = a_item;
         load_info(b_item, b_seq, b_c0, b_L, b_m0, b_m1);              // index it + 4
         a_item = (long long)atomicAdd(p.work_counter, 1ull);          // index it + 5
-        clk.tick(6);
         mbar_wait(&sm.ctx_full[b], (it >> 1) & 1);
-        clk.tick(0);
         PcCtx& cx = sm.ctx[b];
         const long long item = cx.item;
         if (item < 0) break;
@@ -660,32 +615,15 @@ __device__ __forceinline__ void pc_store(PcSmem& sm, const ProfParams& p) {
                 const unsigned long long jd = jd_next;
                 if (j + 1 < S) jd_next = cx.job_dst[j + 1];
                 const int buf = gj % PC_NBUF;
-                clk.tick(6);
                 mbar_wait(&sm.row_full[buf], (gj / PC_NBUF) & 1);
-                clk.tick(1);
                 unsigned char* dst = reinterpret_cast<unsigned char*>(p.out) + (jd & ~15ull);
-#if PC_TIGHT
-                // ONE copy in flight per SM, re-issued the moment the previous one has been read (the regime in which a pure
-                // store stream reaches 7.0 instead of 6.3 TB/s, tools/ubench/tma_store.cu): the row is known to be ready before the
-                // wait, and the previous buffer's bookkeeping comes after the issue
-                if (gj >= 1) bulk_wait_read<0>();
                 bulk_store(dst, sm.rowbuf[buf], PC_F * 4);
-                bulk_commit();
-                if (gj >= 1) {
-                    st_release_smem(&sm.free_count[(gj - 1) % PC_NBUF], (gj - 1) / PC_NBUF + 1);
-                    mbar_arrive(&sm.row_free[(gj - 1) % PC_NBUF]);
-                }
-#else
-                if (IDL_DBG(p) & 4) bulk_store_hint(dst, sm.rowbuf[buf], PC_F * 4, pol_ef);
-                else bulk_store(dst, sm.rowbuf[buf], PC_F * 4);
                 bulk_commit();
                 if (gj >= PC_INFL) {
                     bulk_wait_read<PC_INFL>();         // all but the PC_INFL most recent copies have left shared memory
-                    clk.tick(7);
                     st_release_smem(&sm.free_count[(gj - PC_INFL) % PC_NBUF], (gj - PC_INFL) / PC_NBUF + 1);
                     mbar_arrive(&sm.row_free[(gj - PC_INFL) % PC_NBUF]);
                 }
-#endif
             }
         }
         mbar_arrive(&sm.ctx_empty[b]);
@@ -720,13 +658,9 @@ __device__ __forceinline__ void pc_fix(PcSmem& sm, const ProfParams& p) {
     float vt_prev[RPL];                                // ... and the template values it found there
 #pragma unroll
     for (int u = 0; u < RPL; ++u) { km_prev[u] = 0xFFFFu; vt_prev[u] = 0.f; }
-    PcClock clk;
-    clk.start(ftid == 0 && (IDL_DBG(p) & 16) ? IDL_PROF(p) : nullptr);
     for (int it = 0;; ++it) {
         const int b = it & 1;
-        clk.tick(11);
         mbar_wait(&sm.ctx_full[b], (it >> 1) & 1);
-        clk.tick(8);
         PcCtx& cx = sm.ctx[b];
         const long long item = cx.item;
         if (item < 0) return;
@@ -775,7 +709,6 @@ __device__ __forceinline__ void pc_fix(PcSmem& sm, const ProfParams& p) {
                     for (int u = 0; u < RPL; ++u)
                         if (km[u] != 0xFFFFu) vnew[u] = value(km[u], d[u], fy);
                 }
-                clk.tick(9);
                 if (rebuilt) {
                     mbar_wait(&sm.row_built[fw], n_built & 1);     // the builders wrote a fresh row (they waited for row_free)
                     ++n_built;
@@ -787,7 +720,6 @@ __device__ __forceinline__ void pc_fix(PcSmem& sm, const ProfParams& p) {
                         if (km_prev[u] != 0xFFFFu) row[km_prev[u]] = vt_prev[u];
                     __syncwarp();
                 }
-                clk.tick(10);
                 // the row now holds the template: remember its values at this job's bins (the next job's undo list), then overwrite
 #pragma unroll
                 for (int u = 0; u < RPL; ++u) {
@@ -801,7 +733,6 @@ __device__ __forceinline__ void pc_fix(PcSmem& sm, const ProfParams& p) {
                 fence_proxy_async_smem();              // generic-proxy writes -> visible to the TMA engine
                 __syncwarp();
                 if (lane == 0) mbar_arrive(&sm.row_full[fw]);
-                clk.tick(11);
             }
             gj0 += S;
         }

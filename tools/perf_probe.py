@@ -64,14 +64,6 @@ def main():
                                                mean=mean, scale=scale, prepared=prep))
         b = nv * n * F * 4 + n * L / 4
         print("%-28s best %8.3f ms avg %8.3f ms  %8.1f Mprofiles/s  %7.1f GB/s" % (name, best, avg, nv * n / best / 1e3, b / best / 1e6))
-        if os.environ.get("IDL_PHASE_PROF"):
-            ws = list(ft._workspaces.values())[0]
-            prof = ws[-128:].view(torch.int64)
-            torch.cuda.synchronize()
-            cyc = prof.cpu().numpy().astype(float) / (4 * n)   # 4 launches (1 warm + 3 timed), per sequence
-            names = ["C.wait", "C.stream", "P.count", "P.randN", "P.bern", "P.wait", "restore", "b.gen", "b.scan", "b.write", "b.apply", "b.bar", "sg.plan", "sg.p1", "sg.p2"]
-            print("     cycles/sequence (thread 0): " + "  ".join("%s %.0f" % (nm, c) for nm, c in zip(names, cyc)) + "  total %.0f" % cyc[:7].sum())
-            prof.zero_()
     best, avg = timeit(lambda: ft.Scaler.fit(out[0]))
     print("scaler fit on [%d,%d]: %.3f ms" % (n, F, best))
     big = out[:8]

@@ -37,8 +37,8 @@ def main():
             a.record(); fn(); b.record(); torch.cuda.synchronize()
             ts.append(a.elapsed_time(b))
         by = nv * n * F * 4 + n * L / 4
-        print("%-20s dbg=%s best %.3f ms  %.1f GB/s" % (name, os.environ.get("IDL_PC_DBG", "0"), min(ts), by / min(ts) / 1e6))
-        if name.startswith("all") and not os.environ.get("IDL_PHASE_PROF"):
+        print("%-20s best %.3f ms  %.1f GB/s" % (name, min(ts), by / min(ts) / 1e6))
+        if name.startswith("all"):
             fs = lambda: ft.prepare(ss, k, variants, seed=1)
             fs(); torch.cuda.synchronize()
             ts = []
@@ -47,12 +47,4 @@ def main():
                 a.record(); fs(); b.record(); torch.cuda.synchronize()
                 ts.append(a.elapsed_time(b))
             print("%-20s best %.3f ms" % ("prepare pass", min(ts)))
-        if os.environ.get("IDL_PHASE_PROF"):
-            ws = list(ft._workspaces.values())[0]
-            prof = ws[-128:].view(torch.int64)
-            cyc = prof.cpu().numpy().astype(float) / (4 * n)
-            names = ["S.ctxwait", "S.rowwait", "P.count", "P.randN", "P.bern", "P.ctxwait", "S.issue", "S.dlagwait", "F.ctxwait", "F.patch", "F.donewait", "F.fixups",
-                     "B.ctxwait", "B.build", "B.emptywait"]
-            print("   cycles/seq: " + "  ".join("%s %.0f" % (nm, c) for nm, c in zip(names, cyc)))
-            prof.zero_()
 main()
