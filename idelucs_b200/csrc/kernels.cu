@@ -1137,6 +1137,17 @@ __global__ void standardize_f32_kernel(const float* __restrict__ x, float* __res
     }
 }
 
+// any F and alignment (the canonical k-mer widths R = 2 and 10 of k = 1, 2 are not multiples of 4): one element per step,
+// the same (x - mean32) / scale32 as standardize_f32_kernel.  x may be out (in place).
+__global__ void standardize_f32_elem_kernel(const float* x, float* out, long long total, int F, const float* __restrict__ mean,
+                                            const float* __restrict__ scale) {
+    const long long stride = (long long)gridDim.x * blockDim.x;
+    const int cstep = (int)(stride % F);
+    long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    int c = (int)(i % F);
+    for (; i < total; i += stride, c = c + cstep >= F ? c + cstep - F : c + cstep) out[i] = (x[i] - mean[c]) / scale[c];
+}
+
 __global__ void standardize_f64_kernel(const double* __restrict__ x, double* __restrict__ out64, float* __restrict__ out32,
                                        long long total, int F, const double* __restrict__ mean, const double* __restrict__ scale) {
     const long long stride = (long long)gridDim.x * blockDim.x;
@@ -1725,10 +1736,18 @@ int idl_scaler_finalize(const double* d_partials, const double* d_part_n, int n_
 
 int idl_standardize_f32(const float* d_x, float* d_out, int64_t n, int F, const float* d_mean32, const float* d_scale32,
                         void* stream) {
-    if (!d_x || !d_out || !d_mean32 || !d_scale32 || n < 0 || F <= 0 || F % 4) return set_error(IDL_EINVAL, "idl_standardize_f32: bad argument%s", "");
+    if (!d_x || !d_out || !d_mean32 || !d_scale32 || n < 0 || F <= 0) return set_error(IDL_EINVAL, "idl_standardize_f32: bad argument%s", "");
     if (n == 0) return IDL_OK;
-    const long long n4 = n * (F / 4);
-    standardize_f32_kernel<<<elementwise_grid(n4), 256, 0, (cudaStream_t)stream>>>(d_x, d_out, n4, F / 4, d_mean32, d_scale32); note_launch();
+    const bool aligned16 = ((reinterpret_cast<uintptr_t>(d_x) | reinterpret_cast<uintptr_t>(d_out) | reinterpret_cast<uintptr_t>(d_mean32) |
+                             reinterpret_cast<uintptr_t>(d_scale32)) & 15) == 0;
+    if (F % 4 == 0 && aligned16) {
+        const long long n4 = n * (F / 4);
+        standardize_f32_kernel<<<elementwise_grid(n4), 256, 0, (cudaStream_t)stream>>>(d_x, d_out, n4, F / 4, d_mean32, d_scale32);
+    } else {
+        const long long total = n * (long long)F;
+        standardize_f32_elem_kernel<<<elementwise_grid(total), 256, 0, (cudaStream_t)stream>>>(d_x, d_out, total, F, d_mean32, d_scale32);
+    }
+    note_launch();
     IDL_CUDA_CHECK(cudaGetLastError());
     return IDL_OK;
 }

@@ -201,7 +201,8 @@ int idl_scaler_finalize(const double* d_partials, const double* d_part_n, int n_
                         double* d_var64, double* d_scale64, float* d_mean32, float* d_scale32, void* stream);
 
 /* replaces StandardScaler.transform at idelucs/utils.py:361-363 (float32, in place or out of
- * place: (x - mean32) / scale32 with IEEE float32 rounding) and :405 (float64:
+ * place: (x - mean32) / scale32 with IEEE float32 rounding; any F >= 1, 128-bit accesses when
+ * F % 4 == 0 and all four pointers are 16-byte aligned) and :405 (float64:
  * (x - mean64) / scale64, optionally also written as float32 like models.py:163 casts it). */
 int idl_standardize_f32(const float* d_x, float* d_out, int64_t n, int F, const float* d_mean32,
                         const float* d_scale32, void* stream);
