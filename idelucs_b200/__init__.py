@@ -6,11 +6,12 @@ Reference surface mirrored (idelucs/__init__.py:3-8): ``check_sequence``, ``Summ
 ``cgr``, ``IID_model``, ``IID_loss``, ``info_nce_loss``, ``iDeLUCS_cluster`` (``PlotPolygon`` / ``define_ToolTips`` are GUI / plot
 helpers and out of scope).
 Submodules keep the reference's names: ``kmers``, ``utils``, ``LossFunctions``, ``models``,
-``cluster``.  ``hdbscan_device`` is sklearn's HDBSCAN with its all-pairs work on the GPU.  Nothing here falls back to a CPU implementation.
+``cluster``.  ``hdbscan_device`` is sklearn's HDBSCAN and ``silhouette_samples_device`` /
+``silhouette_score_device`` are sklearn's silhouette metrics, each with its all-pairs work on the GPU.  Nothing here falls back to a CPU implementation.
 """
 __version__ = (0, 1, 0)
 
-__all__ = ["kmers", "utils", "LossFunctions", "models", "cluster", "seqset", "featurise", "hdbscan"]
+__all__ = ["kmers", "utils", "LossFunctions", "models", "cluster", "seqset", "featurise", "hdbscan", "metrics"]
 
 
 def __getattr__(name):  # lazy: importing the package must not require torch.cuda to be usable
@@ -34,6 +35,8 @@ def __getattr__(name):  # lazy: importing the package must not require torch.cud
         "IID_model": ("models", "IID_model"),
         "iDeLUCS_cluster": ("cluster", "iDeLUCS_cluster"),
         "hdbscan_device": ("hdbscan", "hdbscan_device"),
+        "silhouette_samples_device": ("metrics", "silhouette_samples_device"),
+        "silhouette_score_device": ("metrics", "silhouette_score_device"),
     }
     if name in lazy:
         mod, attr = lazy[name]

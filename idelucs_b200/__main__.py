@@ -2,7 +2,8 @@
 flags and defaults) driving the B200-native hot path.  Orchestration only: voters x epochs,
 majority vote over voters (k-means on one-hot votes, utils.py:582-602) or HDBSCAN on the latent space when
 --n_clusters=0 (the ``hdbscan`` package if importable, else scikit-learn's algorithm with its all-pairs work on the GPU,
-``hdbscan.hdbscan_device``), metrics and TSV output."""
+``hdbscan.hdbscan_device``), metrics (silhouette on the GPU, ``metrics.silhouette_score_device``) and TSV output:
+assignments.tsv and metrics.tsv under Results/<fasta stem>/<time>/."""
 import argparse
 import os
 import sys
@@ -14,7 +15,7 @@ import numpy as np
 def run(args):
     import torch  # noqa: F401
     from . import models
-    from .utils import SummaryFasta, cluster_acc, label_features
+    from .utils import SummaryFasta, compute_results, external_results, label_features
     start = time.time()
     use_hdbscan = False
     if args["n_clusters"] == 0:   # idelucs/__main__.py:75-83: 200 output units, clusters from HDBSCAN on the latent space
@@ -37,7 +38,7 @@ def run(args):
         voter_min = np.inf
         for _ in range(args["n_epochs"]):
             voter_min = min(voter_min, model.contrastive_training_epoch())
-        y_pred, probabilities, latent = model.predict(device_latent=use_hdbscan)
+        y_pred, probabilities, latent = model.predict(device_latent=True)
         if voter_min < min_loss:
             min_loss, model_latent = voter_min, latent
         if not use_hdbscan:   # relabel in order of first appearance (__main__.py:131-141)
@@ -68,14 +69,31 @@ def run(args):
         for name, c, pr in zip(model.names, y_pred, probabilities):
             fh.write(f"{name}\t{int(c)}\t{float(pr):.6f}\n")
     print("\n")
+    y_true = None
     if model.GT is not None:
-        from sklearn import metrics
         labels = {c: i for i, c in enumerate(sorted(set(model.GT)))}
         y_true = np.array([labels[c] for c in model.GT])
-        _, acc = cluster_acc(y_true, np.asarray(y_pred))
-        print(f"ACC \t {acc:.5f}")
-        print(f"ARI \t {metrics.adjusted_rand_score(y_true, y_pred):.5f}")
-        print(f"NMI \t {metrics.adjusted_mutual_info_score(y_true, y_pred):.5f}")
+    # __main__.py:163-232: the metrics of the last voter's latent space
+    n_found = len(np.unique(y_pred))
+    if 1 < n_found < len(y_pred):
+        results, _ = compute_results(y_pred, latent, y_true)
+        note = None
+    else:   # silhouette and Davies-Bouldin are undefined; the run still reports what it can
+        results = {"Davies-Boulding": float("nan"), "Silhouette-Score": float("nan")}
+        if y_true is not None:
+            results.update(external_results(y_pred, y_true)[0])
+        note = f"Silhouette and Davies-Bouldin need 2 to {len(y_pred) - 1} clusters, got {n_found}: written as nan"
+    with open(os.path.join(out_dir, "metrics.tsv"), "w") as fh:
+        fh.write("\t".join(results) + "\n")
+        fh.write("\t".join(repr(float(v)) for v in results.values()) + "\n")
+    if y_true is not None:
+        print(f"ACC \t {results['ACC']:.5f}")
+        print(f"ARI \t {results['ARI']:.5f}")
+        print(f"NMI \t {results['NMI']:.5f}")
+    if note:
+        print(note)
+    print(f"Silhouette \t {results['Silhouette-Score']:.5f}")
+    print(f"Davies-Bouldin \t {results['Davies-Boulding']:.5f}")
     print(f"Elapsed \t {time.time() - start:.1f} s   results in {out_dir}")
     return y_pred
 

@@ -84,6 +84,8 @@ PROTOTYPES = {
     "idl_hdbscan_workspace_bytes": (c_size_t, [c_i64, c_int]),
     "idl_core_distances": (c_int, [c_void_p, c_i64, c_int, c_i64, c_void_p, c_void_p, c_size_t, c_void_p]),
     "idl_mreach_mst": (c_int, [c_void_p, c_void_p, c_i64, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]),
+    "idl_silhouette_workspace_bytes": (c_size_t, [c_i64, c_i64]),
+    "idl_silhouette_samples": (c_int, [c_void_p, c_void_p, c_i64, c_int, c_i64, c_void_p, c_void_p, c_size_t, c_void_p]),
 }
 
 _lib = None

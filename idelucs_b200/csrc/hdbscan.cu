@@ -8,8 +8,8 @@
 // an FMA), then an IEEE sqrt.  That is the arithmetic of sklearn's EuclideanDistance, so core distances and MST
 // weights compare with sklearn's by ==.
 //
-// Both passes share one tile loop: a CTA owns BI = 64 rows and walks all n columns in BJ = 64-column tiles; the two
-// 64 x DT fp64 panels sit in shared memory and every thread accumulates a 4 x 4 micro-tile of squared distances.
+// Both passes share one tile loop (sq_tile, pairwise.cuh): a CTA owns BI = 64 rows and walks all n columns in BJ = 64-column
+// tiles; the two 64 x DT fp64 panels sit in shared memory and every thread accumulates a 4 x 4 micro-tile of squared distances.
 // Nothing of size n x n is ever stored: the core distances are a radix select over the fp64 bit patterns of the
 // squared distances (non-negative doubles order like their bits, and sqrt is monotone), recomputing the distances on
 // every pass; the MST is Borůvka, one all-pairs pass per round.
@@ -23,11 +23,11 @@
 
 #include "../../include/idelucs_b200.h"
 #include "common.h"
+#include "pairwise.cuh"
 
 namespace idl {
 namespace {
 
-constexpr int BI = 64, BJ = 64, DT = 32, NT = 256;
 constexpr int BINS = 256;       // 8-bit radix digits: at most 8 passes over the 64-bit keys
 constexpr int LIST_MAX = 128;   // a row whose candidate bucket holds <= this many keys collects them and finishes in one pass
 constexpr int MODE_HIST = 0, MODE_LIST = 1, MODE_DONE = 2;
@@ -40,47 +40,6 @@ struct RowSel {
     long long rank, count;
     int nbits, mode;
 };
-
-struct Panels {
-    double a[DT][BI + 1];   // +1: the transposed stores of the loader hit distinct banks
-    double b[DT][BJ + 1];
-};
-
-// acc[r][c] = squared distance of rows row0 + ty + 16 r and columns col0 + tx + 16 c (0 outside [0, n))
-__device__ __forceinline__ void sq_tile(const float* __restrict__ x, long long n, int D, long long row0, long long col0, Panels& s,
-                                        double acc[4][4]) {
-    const int tx = threadIdx.x & 15, ty = threadIdx.x >> 4;
-#pragma unroll
-    for (int r = 0; r < 4; ++r)
-#pragma unroll
-        for (int c = 0; c < 4; ++c) acc[r][c] = 0.0;
-    for (int t0 = 0; t0 < D; t0 += DT) {
-        __syncthreads();
-        for (int e = threadIdx.x; e < DT * BI; e += NT) {
-            const int rr = e / DT, t = e % DT;
-            const long long gi = row0 + rr, gj = col0 + rr;
-            const bool tin = t0 + t < D;
-            s.a[t][rr] = (tin && gi < n) ? (double)x[gi * D + t0 + t] : 0.0;
-            s.b[t][rr] = (tin && gj < n) ? (double)x[gj * D + t0 + t] : 0.0;
-        }
-        __syncthreads();
-        const int tn = min(DT, D - t0);
-        for (int t = 0; t < tn; ++t) {
-            double av[4], bv[4];
-#pragma unroll
-            for (int r = 0; r < 4; ++r) av[r] = s.a[t][ty + 16 * r];
-#pragma unroll
-            for (int c = 0; c < 4; ++c) bv[c] = s.b[t][tx + 16 * c];
-#pragma unroll
-            for (int r = 0; r < 4; ++r)
-#pragma unroll
-                for (int c = 0; c < 4; ++c) {
-                    const double df = __dsub_rn(av[r], bv[c]);
-                    acc[r][c] = __dadd_rn(acc[r][c], __dmul_rn(df, df));
-                }
-        }
-    }
-}
 
 __global__ void core_init_kernel(RowSel* __restrict__ sel, long long n, long long k) {
     const long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x;

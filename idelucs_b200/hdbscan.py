@@ -23,6 +23,14 @@ def _as_device_matrix(latent):
     return x.to(device=dev, dtype=torch.float32).contiguous()
 
 
+def _check_finite(x):
+    import torch
+    if not bool(torch.isfinite(x).all()):
+        if bool(torch.isnan(x).any()):
+            raise ValueError("Input X contains NaN.")
+        raise ValueError("Input X contains infinity or a value too large for dtype('float32').")
+
+
 def _workspace(x):
     import torch
     n, D = x.shape
@@ -82,14 +90,9 @@ def hdbscan_device(latent, min_cluster_size, min_samples=None):
     (labels int64[N], -1 = noise; probabilities float64[N]) for a float32 [N, D] CUDA tensor or a numpy array (rounded to
     float32).  min_samples counts the point itself and defaults to min_cluster_size, as in sklearn.  Unlike sklearn,
     non-finite values are rejected with ValueError instead of being given special labels."""
-    import torch
     _check_params(min_cluster_size, min_samples)
     x = _as_device_matrix(latent)
-    finite = torch.isfinite(x)
-    if not bool(finite.all()):
-        if bool(torch.isnan(x).any()):
-            raise ValueError("Input X contains NaN.")
-        raise ValueError("Input X contains infinity or a value too large for dtype('float32').")
+    _check_finite(x)
     n = x.shape[0]
     if n == 1:
         raise ValueError("n_samples=1 while HDBSCAN requires more than one sample")

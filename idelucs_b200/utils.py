@@ -389,18 +389,30 @@ def label_features(predictions, n_clusters):
 
 
 def compute_results(y_pred, data, y_true=None):
-    """idelucs/utils.py:606-625: internal (and, with ground truth, external) clustering metrics -> (dict, assignment)."""
+    """idelucs/utils.py:606-625: internal (and, with ground truth, external) clustering metrics -> (dict, assignment).
+    A CUDA tensor `data` gets its silhouette score on the GPU (metrics.silhouette_score_device) and its Davies-Bouldin
+    score from sklearn on a float64 host copy; numpy `data` goes to sklearn for both."""
     from sklearn import metrics
-    d = {"Davies-Boulding": metrics.davies_bouldin_score(data, y_pred), "Silhouette-Score": metrics.silhouette_score(data, y_pred)}
+    if torch.is_tensor(data) and data.is_cuda:
+        from .metrics import silhouette_score_device
+        host = data.cpu().numpy().astype(np.float64)
+        d = {"Davies-Boulding": metrics.davies_bouldin_score(host, y_pred), "Silhouette-Score": silhouette_score_device(data, y_pred)}
+    else:
+        d = {"Davies-Boulding": metrics.davies_bouldin_score(data, y_pred), "Silhouette-Score": metrics.silhouette_score(data, y_pred)}
     if y_true is not None:
-        d["NMI"] = metrics.adjusted_mutual_info_score(y_true, y_pred)
-        d["ARI"] = metrics.adjusted_rand_score(y_true, y_pred)
-        d["Homogeneity"] = metrics.homogeneity_score(y_true, y_pred)
-        d["Completeness"] = metrics.completeness_score(y_true, y_pred)
-        ind, acc = cluster_acc(y_true, y_pred)
-        d["ACC"] = acc
+        ext, ind = external_results(y_pred, y_true)
+        d.update(ext)
         return d, ind
     return d, None
+
+
+def external_results(y_pred, y_true):
+    """the ground-truth part of compute_results -> ({NMI, ARI, Homogeneity, Completeness, ACC}, assignment)"""
+    from sklearn import metrics
+    d = {"NMI": metrics.adjusted_mutual_info_score(y_true, y_pred), "ARI": metrics.adjusted_rand_score(y_true, y_pred),
+         "Homogeneity": metrics.homogeneity_score(y_true, y_pred), "Completeness": metrics.completeness_score(y_true, y_pred)}
+    ind, d["ACC"] = cluster_acc(y_true, y_pred)
+    return d, ind
 
 
 def cluster_acc(y_true, y_pred):

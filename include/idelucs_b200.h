@@ -347,6 +347,25 @@ int idl_core_distances(const float* d_x, int64_t n, int D, int64_t k, double* d_
 int idl_mreach_mst(const float* d_x, const double* d_core, int64_t n, int D, int64_t* d_src, int64_t* d_dst, double* d_w, void* d_ws,
                    size_t ws_bytes, void* stream);
 
+/* F4 — per-sample silhouette coefficients (sklearn.metrics.silhouette_samples, Euclidean metric), the internal
+ * clustering metric the reference writes to metrics.tsv (idelucs/utils.py compute_results).  d_x: float32 [n, D]
+ * row-major; d_labels: int32 [n], every label in 0..n_labels-1 (empty labels are allowed); d_out: double [n].
+ * Arithmetic (results compare with a sequential fp64 reference by ==):
+ *   d(i, j)  = exactly the distance of idl_core_distances: inputs widened to double, sum of (x_i[t] - x_j[t])^2 in order
+ *              t = 0..D-1 with every operation rounded on its own (no FMA), IEEE sqrt;
+ *   S_c(i)   = ((0 + d(i, j1)) + d(i, j2)) + ... over the points j1 < j2 < ... of cluster c, self included (d(i, i) = 0);
+ *   intra    = S_own / (n_own - 1);  inter = min over non-empty c != own of S_c / n_c;
+ *   s(i)     = (inter - intra) / max(intra, inter), and 0 when n_own = 1 or the quotient is NaN (intra = inter = 0, or no
+ *              other non-empty cluster): sklearn's nan_to_num.
+ * d_ws: idl_silhouette_workspace_bytes(n, n_labels) bytes (0 for n outside 1..2^31-1 or n_labels outside 1..n),
+ * 16-byte aligned; memory is O(n D + n): no n x n matrix is stored.  The call copies the labels to the host and
+ * SYNCHRONISES `stream` once, before any kernel runs: a label outside 0..n_labels-1 returns IDL_EINVAL naming its
+ * position.  The host groups the points by label (stable counting sort) and one all-pairs kernel follows, enqueued
+ * on `stream` (d_out is ready when `stream` is). */
+size_t idl_silhouette_workspace_bytes(int64_t n, int64_t n_labels);
+int idl_silhouette_samples(const float* d_x, const int32_t* d_labels, int64_t n, int D, int64_t n_labels, double* d_out, void* d_ws,
+                           size_t ws_bytes, void* stream);
+
 #ifdef __cplusplus
 }
 #endif
