@@ -13,10 +13,12 @@ import numpy as np
 
 
 def run(args):
-    import torch  # noqa: F401
+    import torch
     from . import models
     from .utils import SummaryFasta, compute_results, external_results, label_features
     start = time.time()
+    # the all-pairs passes after training (HDBSCAN, silhouette) are split over every visible GPU; training uses one
+    devices = list(range(torch.cuda.device_count()))
     use_hdbscan = False
     if args["n_clusters"] == 0:   # idelucs/__main__.py:75-83: 200 output units, clusters from HDBSCAN on the latent space
         args["n_clusters"], use_hdbscan = 200, True
@@ -51,8 +53,9 @@ def run(args):
         try:
             import hdbscan
         except ImportError:   # scikit-learn's HDBSCAN with its all-pairs work on the GPU (same results as sklearn.cluster.HDBSCAN)
-            from .hdbscan import hdbscan_device
-            labels, probabilities = hdbscan_device(latent, max(msz, 2))
+            from .hdbscan import default_devices, hdbscan_device
+            with default_devices(devices):
+                labels, probabilities = hdbscan_device(latent, max(msz, 2))
         else:
             clusterer = hdbscan.HDBSCAN(min_cluster_size=msz, gen_min_span_tree=True, prediction_data=True)
             clusterer.fit(latent.cpu().numpy().astype(np.float64))
@@ -76,7 +79,7 @@ def run(args):
     # __main__.py:163-232: the metrics of the last voter's latent space
     n_found = len(np.unique(y_pred))
     if 1 < n_found < len(y_pred):
-        results, _ = compute_results(y_pred, latent, y_true)
+        results, _ = compute_results(y_pred, latent, y_true, devices=devices)
         note = None
     else:   # silhouette and Davies-Bouldin are undefined; the run still reports what it can
         results = {"Davies-Boulding": float("nan"), "Silhouette-Score": float("nan")}

@@ -84,8 +84,13 @@ PROTOTYPES = {
     "idl_hdbscan_workspace_bytes": (c_size_t, [c_i64, c_int]),
     "idl_core_distances": (c_int, [c_void_p, c_i64, c_int, c_i64, c_void_p, c_void_p, c_size_t, c_void_p]),
     "idl_mreach_mst": (c_int, [c_void_p, c_void_p, c_i64, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]),
+    "idl_core_distances_rows": (c_int, [c_void_p, c_i64, c_int, c_i64, c_i64, c_i64, c_void_p, c_void_p, c_size_t, c_void_p]),
+    "idl_mreach_mst_parts": (c_int, [c_int, ctypes.POINTER(c_int), ctypes.POINTER(c_void_p), ctypes.POINTER(c_void_p), ctypes.POINTER(c_i64),
+                                     ctypes.POINTER(c_i64), c_i64, c_int, c_void_p, c_void_p, c_void_p, ctypes.POINTER(c_void_p),
+                                     ctypes.POINTER(c_size_t), ctypes.POINTER(c_void_p)]),
     "idl_silhouette_workspace_bytes": (c_size_t, [c_i64, c_i64]),
     "idl_silhouette_samples": (c_int, [c_void_p, c_void_p, c_i64, c_int, c_i64, c_void_p, c_void_p, c_size_t, c_void_p]),
+    "idl_silhouette_samples_rows": (c_int, [c_void_p, c_void_p, c_i64, c_int, c_i64, c_i64, c_i64, c_void_p, c_void_p, c_size_t, c_void_p]),
 }
 
 _lib = None

@@ -15,10 +15,12 @@
 // every pass; the MST is Borůvka, one all-pairs pass per round.
 #include <cuda_runtime.h>
 #include <stdint.h>
+#include <stdio.h>
 #include <string.h>
 
 #include <algorithm>
 #include <numeric>
+#include <string>
 #include <vector>
 
 #include "../../include/idelucs_b200.h"
@@ -41,15 +43,16 @@ struct RowSel {
     int nbits, mode;
 };
 
-__global__ void core_init_kernel(RowSel* __restrict__ sel, long long n, long long k) {
-    const long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x;
-    if (i < n) sel[i] = RowSel{0ull, k, n, 0, n <= LIST_MAX ? MODE_LIST : MODE_HIST};
+__global__ void core_init_kernel(RowSel* __restrict__ sel, long long n, long long k, long long row_begin, long long row_end) {
+    const long long i = row_begin + blockIdx.x * (long long)blockDim.x + threadIdx.x;
+    if (i < row_end) sel[i] = RowSel{0ull, k, n, 0, n <= LIST_MAX ? MODE_LIST : MODE_HIST};
 }
 
 // one radix-select pass: every unfinished row either histograms the next 8-bit digit of the keys that match its prefix
 // (MODE_HIST) or collects those keys and picks the rank-th (MODE_LIST).  CTAs whose rows are all done return at once.
-__global__ void __launch_bounds__(NT) core_pass_kernel(const float* __restrict__ x, long long n, int D, RowSel* __restrict__ sel,
-                                                       double* __restrict__ core) {
+// CTA b owns the rows row_begin + 64 b ..; rows at or past row_end are treated as done (their keys are not collected).
+__global__ void __launch_bounds__(NT) core_pass_kernel(const float* __restrict__ x, long long n, int D, long long row_begin, long long row_end,
+                                                       RowSel* __restrict__ sel, double* __restrict__ core) {
     extern __shared__ __align__(16) unsigned char smem[];
     Panels& s = *reinterpret_cast<Panels*>(smem);
     unsigned int(*hist)[BINS] = reinterpret_cast<unsigned int(*)[BINS]>(smem + sizeof(Panels));   // LIST rows: 128 u64 keys
@@ -57,13 +60,13 @@ __global__ void __launch_bounds__(NT) core_pass_kernel(const float* __restrict__
     __shared__ int s_mode[BI], s_shift[BI];
     __shared__ unsigned int s_cnt[BI];
     __shared__ int s_busy;
-    const long long row0 = (long long)blockIdx.x * BI;
+    const long long row0 = row_begin + (long long)blockIdx.x * BI;
     if (threadIdx.x == 0) s_busy = 0;
     __syncthreads();
     if (threadIdx.x < BI) {
         const long long i = row0 + threadIdx.x;
         int mode = MODE_DONE;
-        if (i < n) {
+        if (i < row_end) {
             const RowSel rs = sel[i];
             mode = rs.mode;
             s_prefix[threadIdx.x] = rs.prefix;
@@ -143,21 +146,23 @@ __global__ void __launch_bounds__(NT) core_pass_kernel(const float* __restrict__
 }
 
 // one Borůvka round: for every point the lightest edge (w, min(i, j), max(i, j)) to a point of another component;
-// pt_w / pt_pair receive it and comp_w[comp[i]] its weight bits (atomicMin; non-negative doubles order like their bits)
-__global__ void __launch_bounds__(NT) mst_nearest_kernel(const float* __restrict__ x, long long n, int D, const double* __restrict__ core,
-                                                         const int* __restrict__ comp, unsigned long long* __restrict__ pt_w,
-                                                         unsigned long long* __restrict__ pt_pair, unsigned long long* __restrict__ comp_w) {
+// pt_w / pt_pair receive it and comp_w[comp[i]] its weight bits (atomicMin; non-negative doubles order like their bits).
+// Only the points i of [row_begin, row_end) are searched from (CTA b owns row_begin + 64 b ..); their partners j are all n.
+__global__ void __launch_bounds__(NT) mst_nearest_kernel(const float* __restrict__ x, long long n, int D, long long row_begin, long long row_end,
+                                                         const double* __restrict__ core, const int* __restrict__ comp,
+                                                         unsigned long long* __restrict__ pt_w, unsigned long long* __restrict__ pt_pair,
+                                                         unsigned long long* __restrict__ comp_w) {
     __shared__ Panels s;
     const int tx = threadIdx.x & 15, ty = threadIdx.x >> 4;
-    const long long row0 = (long long)blockIdx.x * BI;
+    const long long row0 = row_begin + (long long)blockIdx.x * BI;
     double ci[4];
     int gi[4];
     unsigned long long bw[4], bp[4];
 #pragma unroll
     for (int r = 0; r < 4; ++r) {
         const long long i = row0 + ty + 16 * r;
-        ci[r] = i < n ? core[i] : 0.0;
-        gi[r] = i < n ? comp[i] : -1;
+        ci[r] = i < row_end ? core[i] : 0.0;
+        gi[r] = i < row_end ? comp[i] : -1;
         bw[r] = bp[r] = NONE;
     }
     double acc[4][4];
@@ -196,7 +201,7 @@ __global__ void __launch_bounds__(NT) mst_nearest_kernel(const float* __restrict
             }
         }
         const long long i = row0 + ty + 16 * r;
-        if (tx == 0 && i < n) {
+        if (tx == 0 && i < row_end) {
             pt_w[i] = bw[r];
             pt_pair[i] = bp[r];
             if (bw[r] != NONE) atomicMin(&comp_w[gi[r]], bw[r]);
@@ -204,12 +209,13 @@ __global__ void __launch_bounds__(NT) mst_nearest_kernel(const float* __restrict
     }
 }
 
-// the component's lightest edge: among its points whose edge has the component's lightest weight, the smallest pair
-__global__ void mst_pair_kernel(long long n, const int* __restrict__ comp, const unsigned long long* __restrict__ pt_w,
+// the component's lightest edge: among its points (of [row_begin, row_end)) whose edge has the component's lightest weight,
+// the smallest pair
+__global__ void mst_pair_kernel(long long row_begin, long long row_end, const int* __restrict__ comp, const unsigned long long* __restrict__ pt_w,
                                 const unsigned long long* __restrict__ pt_pair, const unsigned long long* __restrict__ comp_w,
                                 unsigned long long* __restrict__ comp_pair) {
-    const long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x;
-    if (i >= n || pt_w[i] == NONE) return;
+    const long long i = row_begin + blockIdx.x * (long long)blockDim.x + threadIdx.x;
+    if (i >= row_end || pt_w[i] == NONE) return;
     const int c = comp[i];
     if (pt_w[i] == comp_w[c]) atomicMin(&comp_pair[c], pt_pair[i]);
 }
@@ -251,108 +257,69 @@ int check_ws(const char* who, int64_t n, int D, size_t ws_bytes) {
     return IDL_OK;
 }
 
-}  // namespace
-}  // namespace idl
-
-using namespace idl;
-
-extern "C" size_t idl_hdbscan_workspace_bytes(int64_t n, int D) {
-    if (n < 1 || n > MAX_N || D < 1) return 0;
-    return std::max(core_ws(n), mst_ws(n, nullptr, nullptr));
-}
-
-extern "C" int idl_core_distances(const float* d_x, int64_t n, int D, int64_t k, double* d_core, void* d_ws, size_t ws_bytes, void* stream) {
-    static const char* who = "idl_core_distances";
-    if (!d_x || !d_core || !d_ws) return set_error(IDL_EINVAL, "%s: null pointer", who);
-    if (int rc = check_shape(who, n, D)) return rc;
-    if (k < 1 || k > n) return set_error(IDL_EINVAL, "%s: k must be in 1..n (got %lld)", who, (long long)k);
-    if (int rc = check_ws(who, n, D, ws_bytes)) return rc;
-    cudaStream_t st = (cudaStream_t)stream;
+// the k-th smallest distance of every row of [row_begin, row_end) (arguments already checked; an empty range enqueues nothing)
+int core_rows(const float* d_x, int64_t n, int D, int64_t k, int64_t row_begin, int64_t row_end, double* d_core, void* d_ws, cudaStream_t st) {
+    const int64_t rows = row_end - row_begin;
+    if (rows == 0) return IDL_OK;
     RowSel* sel = reinterpret_cast<RowSel*>(d_ws);
     IDL_CUDA_CHECK(cudaFuncSetAttribute(core_pass_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CORE_SMEM));
-    core_init_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(sel, n, k);
+    core_init_kernel<<<(unsigned)((rows + 255) / 256), 256, 0, st>>>(sel, n, k, row_begin, row_end);
     note_launch();
     IDL_CUDA_CHECK(cudaGetLastError());
-    const unsigned grid = (unsigned)((n + BI - 1) / BI);
+    const unsigned grid = (unsigned)((rows + BI - 1) / BI);
     for (int pass = 0; pass < 8; ++pass) {   // every row is done after at most 8 digits; finished CTAs exit at once
-        core_pass_kernel<<<grid, NT, CORE_SMEM, st>>>(d_x, n, D, sel, d_core);
+        core_pass_kernel<<<grid, NT, CORE_SMEM, st>>>(d_x, n, D, row_begin, row_end, sel, d_core);
         note_launch();
         IDL_CUDA_CHECK(cudaGetLastError());
     }
     return IDL_OK;
 }
 
-extern "C" int idl_mreach_mst(const float* d_x, const double* d_core, int64_t n, int D, int64_t* d_src, int64_t* d_dst, double* d_w, void* d_ws,
-                              size_t ws_bytes, void* stream) {
-    static const char* who = "idl_mreach_mst";
-    if (!d_x || !d_core || !d_src || !d_dst || !d_w || !d_ws) return set_error(IDL_EINVAL, "%s: null pointer", who);
-    if (int rc = check_shape(who, n, D)) return rc;
-    if (int rc = check_ws(who, n, D, ws_bytes)) return rc;
-    if (n == 1) return IDL_OK;   // no edges
-    cudaStream_t st = (cudaStream_t)stream;
-    MstWs w;
-    mst_ws(n, &w, reinterpret_cast<char*>(d_ws));
+// restores the caller's current device on every return path
+struct DeviceGuard {
+    int dev = -1;
+    ~DeviceGuard() {
+        if (dev >= 0) cudaSetDevice(dev);
+    }
+};
 
-    // components are dense ids 0..m-1; the host keeps the point -> component map and merges between rounds
-    std::vector<int> comp(n);
-    std::iota(comp.begin(), comp.end(), 0);
-    std::vector<unsigned long long> cw, cp;
-    std::vector<int> parent, newid;
-    std::vector<int64_t> src, dst;
-    std::vector<double> wt;
-    src.reserve(n - 1); dst.reserve(n - 1); wt.reserve(n - 1);
+// One Borůvka merge on the host: cw / cp hold every component's lightest outgoing edge (weight bits, pair key).  With the
+// strict edge order (w, min, max) the only cycles are two components choosing the same edge, which the union-find skips the
+// second time.  The new edges are appended to src / dst / wt, comp is renumbered densely and m becomes the new count.
+int merge_round(const char* who, std::vector<int>& comp, const std::vector<unsigned long long>& cw, const std::vector<unsigned long long>& cp,
+                long long& m, std::vector<int64_t>& src, std::vector<int64_t>& dst, std::vector<double>& wt) {
+    std::vector<int> parent(m), newid(m, -1);
+    std::iota(parent.begin(), parent.end(), 0);
     auto find = [&](int a) {
         while (parent[a] != a) a = parent[a] = parent[parent[a]];
         return a;
     };
-    long long m = n;
-    const unsigned grid = (unsigned)((n + BI - 1) / BI);
-    while (m > 1) {
-        IDL_CUDA_CHECK(cudaMemcpyAsync(w.comp, comp.data(), n * sizeof(int), cudaMemcpyHostToDevice, st));
-        IDL_CUDA_CHECK(cudaMemsetAsync(w.comp_w, 0xff, m * 8, st));
-        IDL_CUDA_CHECK(cudaMemsetAsync(w.comp_pair, 0xff, m * 8, st));
-        mst_nearest_kernel<<<grid, NT, 0, st>>>(d_x, n, D, d_core, w.comp, w.pt_w, w.pt_pair, w.comp_w);
-        note_launch();
-        IDL_CUDA_CHECK(cudaGetLastError());
-        mst_pair_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(n, w.comp, w.pt_w, w.pt_pair, w.comp_w, w.comp_pair);
-        note_launch();
-        IDL_CUDA_CHECK(cudaGetLastError());
-        cw.resize(m);
-        cp.resize(m);
-        IDL_CUDA_CHECK(cudaMemcpyAsync(cw.data(), w.comp_w, m * 8, cudaMemcpyDeviceToHost, st));
-        IDL_CUDA_CHECK(cudaMemcpyAsync(cp.data(), w.comp_pair, m * 8, cudaMemcpyDeviceToHost, st));
-        IDL_CUDA_CHECK(cudaStreamSynchronize(st));
-
-        // every component's lightest edge joins it to another; with the strict edge order (w, min, max) the only
-        // cycles are two components choosing the same edge, which the union-find skips the second time
-        parent.resize(m);
-        std::iota(parent.begin(), parent.end(), 0);
-        for (long long c = 0; c < m; ++c) {
-            if (cw[c] == NONE || cp[c] == NONE) return set_error(IDL_ECUDA, "%s: component without an outgoing edge", who);
-            const int64_t a = (int64_t)(cp[c] >> 32), b = (int64_t)(cp[c] & 0xffffffffu);
-            const int ra = find(comp[a]), rb = find(comp[b]);
-            if (ra == rb) continue;
-            parent[std::max(ra, rb)] = std::min(ra, rb);
-            src.push_back(a);
-            dst.push_back(b);
-            double wd;
-            memcpy(&wd, &cw[c], sizeof(wd));
-            wt.push_back(wd);
-        }
-        newid.assign(m, -1);
-        long long m2 = 0;
-        for (long long c = 0; c < m; ++c) {
-            const int r = find((int)c);
-            if (newid[r] < 0) newid[r] = (int)m2++;
-        }
-        for (int64_t i = 0; i < n; ++i) comp[i] = newid[find(comp[i])];
-        m = m2;
+    for (long long c = 0; c < m; ++c) {
+        if (cw[c] == NONE || cp[c] == NONE) return set_error(IDL_ECUDA, "%s: component without an outgoing edge", who);
+        const int64_t a = (int64_t)(cp[c] >> 32), b = (int64_t)(cp[c] & 0xffffffffu);
+        const int ra = find(comp[a]), rb = find(comp[b]);
+        if (ra == rb) continue;
+        parent[std::max(ra, rb)] = std::min(ra, rb);
+        src.push_back(a);
+        dst.push_back(b);
+        double wd;
+        memcpy(&wd, &cw[c], sizeof(wd));
+        wt.push_back(wd);
     }
-    if ((int64_t)src.size() != n - 1) return set_error(IDL_ECUDA, "%s: spanning tree has %lld edges", who, (long long)src.size());
+    long long m2 = 0;
+    for (long long c = 0; c < m; ++c) {
+        const int r = find((int)c);
+        if (newid[r] < 0) newid[r] = (int)m2++;
+    }
+    for (size_t i = 0; i < comp.size(); ++i) comp[i] = newid[find(comp[i])];
+    m = m2;
+    return IDL_OK;
+}
 
-    // orient every edge away from point 0, parent first, as sklearn's Prim (which grows the tree from point 0) emits it:
-    // make_single_linkage takes the (left, right) children of each merge from the edge direction, and the cluster
-    // numbering of tree_to_labels follows them
+// orient every edge of the spanning tree away from point 0, parent first, as sklearn's Prim (which grows the tree from point
+// 0) emits it: make_single_linkage takes the (left, right) children of each merge from the edge direction, and the cluster
+// numbering of tree_to_labels follows them
+void orient_from_point0(int64_t n, std::vector<int64_t>& src, std::vector<int64_t>& dst) {
     std::vector<int64_t> off(n + 1, 0), adj(2 * (n - 1)), stack;
     for (int64_t e = 0; e < n - 1; ++e) ++off[src[e] + 1], ++off[dst[e] + 1];
     for (int64_t i = 0; i < n; ++i) off[i + 1] += off[i];
@@ -374,9 +341,154 @@ extern "C" int idl_mreach_mst(const float* d_x, const double* d_core, int64_t n,
             stack.push_back(v);
         }
     }
+}
+
+// The mutual-reachability MST with its all-pairs work split into row ranges that partition [0, n) (arguments already checked,
+// n >= 2).  Part p searches the lightest outgoing edge of the points of its rows on devices[p], with its own replica of x and
+// core, its own workspace and streams[p].  Components are dense ids 0..m-1; the host keeps the point -> component map,
+// reduces the parts' per-component minima and merges the components between rounds.
+int mst_parts(const char* who, int n_parts, const int* devices, const float* const* d_x, const double* const* d_core, const int64_t* row_begin,
+              const int64_t* row_end, int64_t n, int D, int64_t* d_src, int64_t* d_dst, double* d_w, void* const* d_ws, void* const* streams) {
+    DeviceGuard guard;
+    IDL_CUDA_CHECK(cudaGetDevice(&guard.dev));
+    std::vector<MstWs> w(n_parts);
+    for (int p = 0; p < n_parts; ++p) mst_ws(n, &w[p], reinterpret_cast<char*>(d_ws[p]));
+    std::vector<int> comp(n);
+    std::iota(comp.begin(), comp.end(), 0);
+    std::vector<std::vector<unsigned long long>> pw(n_parts), pp(n_parts);
+    std::vector<unsigned long long> cw, cp;
+    std::vector<int64_t> src, dst;
+    std::vector<double> wt;
+    src.reserve(n - 1); dst.reserve(n - 1); wt.reserve(n - 1);
+    long long m = n;
+    while (m > 1) {
+        // every part is launched before any is read back: a copy to pageable memory blocks the host until its stream is done
+        for (int p = 0; p < n_parts; ++p) {
+            const int64_t rows = row_end[p] - row_begin[p];
+            if (rows == 0) continue;
+            cudaStream_t st = (cudaStream_t)streams[p];
+            IDL_CUDA_CHECK(cudaSetDevice(devices[p]));
+            IDL_CUDA_CHECK(cudaMemcpyAsync(w[p].comp, comp.data(), n * sizeof(int), cudaMemcpyHostToDevice, st));
+            IDL_CUDA_CHECK(cudaMemsetAsync(w[p].comp_w, 0xff, m * 8, st));
+            IDL_CUDA_CHECK(cudaMemsetAsync(w[p].comp_pair, 0xff, m * 8, st));
+            mst_nearest_kernel<<<(unsigned)((rows + BI - 1) / BI), NT, 0, st>>>(d_x[p], n, D, row_begin[p], row_end[p], d_core[p], w[p].comp,
+                                                                               w[p].pt_w, w[p].pt_pair, w[p].comp_w);
+            note_launch();
+            IDL_CUDA_CHECK(cudaGetLastError());
+            mst_pair_kernel<<<(unsigned)((rows + 255) / 256), 256, 0, st>>>(row_begin[p], row_end[p], w[p].comp, w[p].pt_w, w[p].pt_pair,
+                                                                           w[p].comp_w, w[p].comp_pair);
+            note_launch();
+            IDL_CUDA_CHECK(cudaGetLastError());
+        }
+        for (int p = 0; p < n_parts; ++p) {
+            if (row_end[p] == row_begin[p]) continue;
+            cudaStream_t st = (cudaStream_t)streams[p];
+            pw[p].resize(m);
+            pp[p].resize(m);
+            IDL_CUDA_CHECK(cudaSetDevice(devices[p]));
+            IDL_CUDA_CHECK(cudaMemcpyAsync(pw[p].data(), w[p].comp_w, m * 8, cudaMemcpyDeviceToHost, st));
+            IDL_CUDA_CHECK(cudaMemcpyAsync(pp[p].data(), w[p].comp_pair, m * 8, cudaMemcpyDeviceToHost, st));
+            IDL_CUDA_CHECK(cudaStreamSynchronize(st));
+        }
+        // per component the lexicographic minimum of (w, pair) over the parts: what the two atomicMin steps give on one device
+        cw.assign(m, NONE);
+        cp.assign(m, NONE);
+        for (int p = 0; p < n_parts; ++p) {
+            if (row_end[p] == row_begin[p]) continue;
+            for (long long c = 0; c < m; ++c)
+                if (pw[p][c] < cw[c] || (pw[p][c] == cw[c] && pp[p][c] < cp[c])) cw[c] = pw[p][c], cp[c] = pp[p][c];
+        }
+        if (int rc = merge_round(who, comp, cw, cp, m, src, dst, wt)) return rc;
+    }
+    if ((int64_t)src.size() != n - 1) return set_error(IDL_ECUDA, "%s: spanning tree has %lld edges", who, (long long)src.size());
+    orient_from_point0(n, src, dst);
+    cudaStream_t st = (cudaStream_t)streams[0];
+    IDL_CUDA_CHECK(cudaSetDevice(devices[0]));
     IDL_CUDA_CHECK(cudaMemcpyAsync(d_src, src.data(), (n - 1) * sizeof(int64_t), cudaMemcpyHostToDevice, st));
     IDL_CUDA_CHECK(cudaMemcpyAsync(d_dst, dst.data(), (n - 1) * sizeof(int64_t), cudaMemcpyHostToDevice, st));
     IDL_CUDA_CHECK(cudaMemcpyAsync(d_w, wt.data(), (n - 1) * sizeof(double), cudaMemcpyHostToDevice, st));
     IDL_CUDA_CHECK(cudaStreamSynchronize(st));   // the host vectors die on return
     return IDL_OK;
+}
+
+}  // namespace
+
+int check_rows(const char* who, int64_t n, int64_t row_begin, int64_t row_end) {
+    if (row_begin < 0 || row_begin > row_end || row_end > n) {
+        char what[160];
+        snprintf(what, sizeof(what), "%s: row range [%lld, %lld) is not inside [0, %lld)", who, (long long)row_begin, (long long)row_end,
+                 (long long)n);
+        return set_error(IDL_EINVAL, "%s", what);
+    }
+    return IDL_OK;
+}
+
+}  // namespace idl
+
+using namespace idl;
+
+extern "C" size_t idl_hdbscan_workspace_bytes(int64_t n, int D) {
+    if (n < 1 || n > MAX_N || D < 1) return 0;
+    return std::max(core_ws(n), mst_ws(n, nullptr, nullptr));
+}
+
+extern "C" int idl_core_distances(const float* d_x, int64_t n, int D, int64_t k, double* d_core, void* d_ws, size_t ws_bytes, void* stream) {
+    static const char* who = "idl_core_distances";
+    if (!d_x || !d_core || !d_ws) return set_error(IDL_EINVAL, "%s: null pointer", who);
+    if (int rc = check_shape(who, n, D)) return rc;
+    if (k < 1 || k > n) return set_error(IDL_EINVAL, "%s: k must be in 1..n (got %lld)", who, (long long)k);
+    if (int rc = check_ws(who, n, D, ws_bytes)) return rc;
+    return core_rows(d_x, n, D, k, 0, n, d_core, d_ws, (cudaStream_t)stream);
+}
+
+extern "C" int idl_core_distances_rows(const float* d_x, int64_t n, int D, int64_t k, int64_t row_begin, int64_t row_end, double* d_core,
+                                       void* d_ws, size_t ws_bytes, void* stream) {
+    static const char* who = "idl_core_distances_rows";
+    if (!d_x || !d_core || !d_ws) return set_error(IDL_EINVAL, "%s: null pointer", who);
+    if (int rc = check_shape(who, n, D)) return rc;
+    if (k < 1 || k > n) return set_error(IDL_EINVAL, "%s: k must be in 1..n (got %lld)", who, (long long)k);
+    if (int rc = check_rows(who, n, row_begin, row_end)) return rc;
+    if (int rc = check_ws(who, n, D, ws_bytes)) return rc;
+    return core_rows(d_x, n, D, k, row_begin, row_end, d_core, d_ws, (cudaStream_t)stream);
+}
+
+extern "C" int idl_mreach_mst(const float* d_x, const double* d_core, int64_t n, int D, int64_t* d_src, int64_t* d_dst, double* d_w, void* d_ws,
+                              size_t ws_bytes, void* stream) {
+    static const char* who = "idl_mreach_mst";
+    if (!d_x || !d_core || !d_src || !d_dst || !d_w || !d_ws) return set_error(IDL_EINVAL, "%s: null pointer", who);
+    if (int rc = check_shape(who, n, D)) return rc;
+    if (int rc = check_ws(who, n, D, ws_bytes)) return rc;
+    if (n == 1) return IDL_OK;   // no edges
+    int dev;
+    IDL_CUDA_CHECK(cudaGetDevice(&dev));
+    const int64_t begin = 0;
+    return mst_parts(who, 1, &dev, &d_x, &d_core, &begin, &n, n, D, d_src, d_dst, d_w, &d_ws, &stream);
+}
+
+extern "C" int idl_mreach_mst_parts(int n_parts, const int* devices, const float* const* d_x, const double* const* d_core, const int64_t* row_begin,
+                                    const int64_t* row_end, int64_t n, int D, int64_t* d_src, int64_t* d_dst, double* d_w, void* const* d_ws,
+                                    const size_t* ws_bytes, void* const* streams) {
+    static const char* who = "idl_mreach_mst_parts";
+    if (!devices || !d_x || !d_core || !row_begin || !row_end || !d_src || !d_dst || !d_w || !d_ws || !ws_bytes || !streams)
+        return set_error(IDL_EINVAL, "%s: null pointer", who);
+    if (n_parts < 1) return set_error(IDL_EINVAL, "%s: n_parts must be >= 1 (got %lld)", who, (long long)n_parts);
+    std::vector<std::string> part(n_parts);   // "idl_mreach_mst_parts: part p", the prefix of a part's error texts
+    for (int p = 0; p < n_parts; ++p) part[p] = std::string(who) + ": part " + std::to_string(p);
+    for (int p = 0; p < n_parts; ++p)
+        if (!d_x[p] || !d_core[p] || !d_ws[p]) return set_error(IDL_EINVAL, "%s: null pointer", part[p].c_str());
+    if (int rc = check_shape(who, n, D)) return rc;
+    for (int p = 0; p < n_parts; ++p)
+        if (int rc = check_rows(part[p].c_str(), n, row_begin[p], row_end[p])) return rc;
+    for (int p = 0; p <= n_parts; ++p) {   // part p begins where part p - 1 ends; part 0 at 0, and the last part ends at n
+        const int64_t at = p < n_parts ? row_begin[p] : n, want = p ? row_end[p - 1] : 0;
+        if (at == want) continue;
+        char what[200];
+        snprintf(what, sizeof(what), "%s: the row ranges do not partition [0, %lld) in order: part %d %s at %lld, not %lld", who, (long long)n,
+                 p < n_parts ? p : p - 1, p < n_parts ? "begins" : "ends", (long long)(p < n_parts ? at : want), (long long)(p < n_parts ? want : at));
+        return set_error(IDL_EINVAL, "%s", what);
+    }
+    for (int p = 0; p < n_parts; ++p)
+        if (int rc = check_ws(part[p].c_str(), n, D, ws_bytes[p])) return rc;
+    if (n == 1) return IDL_OK;   // no edges
+    return mst_parts(who, n_parts, devices, d_x, d_core, row_begin, row_end, n, D, d_src, d_dst, d_w, d_ws, streams);
 }

@@ -31,17 +31,18 @@ struct SilSmem {
     double d[BI][BJ + 1];   // distances of the current tile, row-major
 };
 
-// out[i] = silhouette of row i; order: int32[n], the points in label-sorted order (stable); off: int32[n_labels + 1],
-// cluster c holds the positions off[c] .. off[c + 1] - 1 of `order`
+// out[i] = silhouette of row i for the rows of [row_begin, row_end) (CTA b owns row_begin + 64 b ..); order: int32[n], the
+// points in label-sorted order (stable); off: int32[n_labels + 1], cluster c holds the positions off[c] .. off[c + 1] - 1 of `order`
 __global__ void __launch_bounds__(NT) silhouette_kernel(const float* __restrict__ x, const int* __restrict__ labels, long long n, int D,
-                                                        const int* __restrict__ order, const int* __restrict__ off, double* __restrict__ out) {
+                                                        long long row_begin, long long row_end, const int* __restrict__ order,
+                                                        const int* __restrict__ off, double* __restrict__ out) {
     extern __shared__ __align__(16) unsigned char smem[];
     SilSmem& s = *reinterpret_cast<SilSmem*>(smem);
     const int tx = threadIdx.x & 15, ty = threadIdx.x >> 4;
-    const long long row0 = (long long)blockIdx.x * BI;
+    const long long row0 = row_begin + (long long)blockIdx.x * BI;
     // the fold state of row row0 + threadIdx.x (threads < BI)
     const long long i = row0 + threadIdx.x;
-    const bool folds = threadIdx.x < BI && i < n;
+    const bool folds = threadIdx.x < BI && i < row_end;
     const int own = folds ? labels[i] : -1;
     int c = 0;                     // the cluster of the next column position
     long long end = folds ? off[1] : 0;   // its end position
@@ -97,27 +98,9 @@ __global__ void __launch_bounds__(NT) silhouette_kernel(const float* __restrict_
 constexpr size_t align256(size_t b) { return (b + 255) & ~(size_t)255; }
 constexpr size_t SIL_SMEM = sizeof(SilSmem);
 
-}  // namespace
-}  // namespace idl
-
-using namespace idl;
-
-extern "C" size_t idl_silhouette_workspace_bytes(int64_t n, int64_t n_labels) {
-    if (n < 1 || n > SIL_MAX_N || n_labels < 1 || n_labels > n) return 0;
-    return align256((size_t)n * sizeof(int)) + align256((size_t)(n_labels + 1) * sizeof(int));
-}
-
-extern "C" int idl_silhouette_samples(const float* d_x, const int32_t* d_labels, int64_t n, int D, int64_t n_labels, double* d_out, void* d_ws,
-                                      size_t ws_bytes, void* stream) {
-    static const char* who = "idl_silhouette_samples";
-    if (!d_x || !d_labels || !d_out || !d_ws) return set_error(IDL_EINVAL, "%s: null pointer", who);
-    if (n < 1 || n > SIL_MAX_N) return set_error(IDL_EINVAL, "%s: n must be in 1..2147483647 (got %lld)", who, (long long)n);
-    if (D < 1) return set_error(IDL_EINVAL, "%s: D must be >= 1 (got %lld)", who, (long long)D);
-    if (n_labels < 1 || n_labels > n) return set_error(IDL_EINVAL, "%s: n_labels must be in 1..n (got %lld)", who, (long long)n_labels);
-    const size_t need = idl_silhouette_workspace_bytes(n, n_labels);
-    if (ws_bytes < need) return set_error(IDL_EINVAL, "%s: workspace too small (need %lld bytes)", who, (long long)need);
-    cudaStream_t st = (cudaStream_t)stream;
-
+// silhouette of the rows of [row_begin, row_end) (arguments already checked except the label values)
+int silhouette_rows(const char* who, const float* d_x, const int32_t* d_labels, int64_t n, int D, int64_t n_labels, int64_t row_begin,
+                    int64_t row_end, double* d_out, void* d_ws, cudaStream_t st) {
     // group the points by label on the host: a stable counting sort
     std::vector<int32_t> lab(n);
     IDL_CUDA_CHECK(cudaMemcpyAsync(lab.data(), d_labels, n * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
@@ -131,6 +114,7 @@ extern "C" int idl_silhouette_samples(const float* d_x, const int32_t* d_labels,
         }
         ++off[lab[i] + 1];
     }
+    if (row_end == row_begin) return IDL_OK;
     for (int64_t c = 0; c < n_labels; ++c) off[c + 1] += off[c];
     {
         std::vector<int32_t> fill(off.begin(), off.end() - 1);
@@ -144,8 +128,51 @@ extern "C" int idl_silhouette_samples(const float* d_x, const int32_t* d_labels,
     IDL_CUDA_CHECK(cudaMemcpyAsync(d_off, off.data(), (n_labels + 1) * sizeof(int32_t), cudaMemcpyHostToDevice, st));
 
     IDL_CUDA_CHECK(cudaFuncSetAttribute(silhouette_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SIL_SMEM));
-    silhouette_kernel<<<(unsigned)((n + BI - 1) / BI), NT, SIL_SMEM, st>>>(d_x, d_labels, n, D, d_order, d_off, d_out);
+    silhouette_kernel<<<(unsigned)((row_end - row_begin + BI - 1) / BI), NT, SIL_SMEM, st>>>(d_x, d_labels, n, D, row_begin, row_end, d_order,
+                                                                                           d_off, d_out);
     note_launch();
     IDL_CUDA_CHECK(cudaGetLastError());
     return IDL_OK;
+}
+
+int check_args(const char* who, const float* d_x, const int32_t* d_labels, int64_t n, int D, int64_t n_labels, const double* d_out,
+               const void* d_ws) {
+    if (!d_x || !d_labels || !d_out || !d_ws) return set_error(IDL_EINVAL, "%s: null pointer", who);
+    if (n < 1 || n > SIL_MAX_N) return set_error(IDL_EINVAL, "%s: n must be in 1..2147483647 (got %lld)", who, (long long)n);
+    if (D < 1) return set_error(IDL_EINVAL, "%s: D must be >= 1 (got %lld)", who, (long long)D);
+    if (n_labels < 1 || n_labels > n) return set_error(IDL_EINVAL, "%s: n_labels must be in 1..n (got %lld)", who, (long long)n_labels);
+    return IDL_OK;
+}
+
+int check_ws(const char* who, int64_t n, int64_t n_labels, size_t ws_bytes) {
+    const size_t need = idl_silhouette_workspace_bytes(n, n_labels);
+    if (ws_bytes < need) return set_error(IDL_EINVAL, "%s: workspace too small (need %lld bytes)", who, (long long)need);
+    return IDL_OK;
+}
+
+}  // namespace
+}  // namespace idl
+
+using namespace idl;
+
+extern "C" size_t idl_silhouette_workspace_bytes(int64_t n, int64_t n_labels) {
+    if (n < 1 || n > SIL_MAX_N || n_labels < 1 || n_labels > n) return 0;
+    return align256((size_t)n * sizeof(int)) + align256((size_t)(n_labels + 1) * sizeof(int));
+}
+
+extern "C" int idl_silhouette_samples(const float* d_x, const int32_t* d_labels, int64_t n, int D, int64_t n_labels, double* d_out, void* d_ws,
+                                      size_t ws_bytes, void* stream) {
+    static const char* who = "idl_silhouette_samples";
+    if (int rc = check_args(who, d_x, d_labels, n, D, n_labels, d_out, d_ws)) return rc;
+    if (int rc = check_ws(who, n, n_labels, ws_bytes)) return rc;
+    return silhouette_rows(who, d_x, d_labels, n, D, n_labels, 0, n, d_out, d_ws, (cudaStream_t)stream);
+}
+
+extern "C" int idl_silhouette_samples_rows(const float* d_x, const int32_t* d_labels, int64_t n, int D, int64_t n_labels, int64_t row_begin,
+                                           int64_t row_end, double* d_out, void* d_ws, size_t ws_bytes, void* stream) {
+    static const char* who = "idl_silhouette_samples_rows";
+    if (int rc = check_args(who, d_x, d_labels, n, D, n_labels, d_out, d_ws)) return rc;
+    if (int rc = check_rows(who, n, row_begin, row_end)) return rc;
+    if (int rc = check_ws(who, n, n_labels, ws_bytes)) return rc;
+    return silhouette_rows(who, d_x, d_labels, n, D, n_labels, row_begin, row_end, d_out, d_ws, (cudaStream_t)stream);
 }

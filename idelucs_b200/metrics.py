@@ -8,13 +8,15 @@ apart instead of 0, are the exception."""
 import numpy as np
 
 from . import _lib
-from .hdbscan import _as_device_matrix, _check_finite
+from .hdbscan import _as_device_matrix, _check_finite, _parts, _replicas
 
 
-def silhouette_samples_device(X, labels):
+def silhouette_samples_device(X, labels, devices=None):
     """sklearn.metrics.silhouette_samples(X, labels) -> float64 [N] numpy array, for a float32 [N, D] CUDA tensor or a
     numpy array (rounded to float32).  labels: any integer array of length N, encoded densely as sklearn's LabelEncoder
-    does; 2 to N - 1 distinct labels.  Non-finite values of X are rejected with ValueError."""
+    does; 2 to N - 1 distinct labels.  Non-finite values of X are rejected with ValueError.  devices: None (the tensor's
+    device, or the current one for a numpy array) or a list of CUDA devices (repeats allowed) over which the rows are split
+    as in hdbscan.row_parts; the values do not depend on it."""
     import torch
     x = _as_device_matrix(X)
     _check_finite(x)
@@ -26,17 +28,23 @@ def silhouette_samples_device(X, labels):
     n_labels = len(uniq)
     if not 1 < n_labels < n:
         raise ValueError("Number of labels is %d. Valid values are 2 to n_samples - 1 (inclusive)" % n_labels)
-    lab = torch.from_numpy(enc.astype(np.int32)).to(x.device)
     lib = _lib.load()
-    ws = torch.empty(lib.idl_silhouette_workspace_bytes(n, n_labels), dtype=torch.uint8, device=x.device)
-    out = torch.empty(n, dtype=torch.float64, device=x.device)
-    with torch.cuda.device(x.device):
-        _lib.check(lib.idl_silhouette_samples(_lib.ptr(x), _lib.ptr(lab), n, D, n_labels, _lib.ptr(out), _lib.ptr(ws), ws.numel(),
-                                              _lib.stream_ptr()))
-    return out.cpu().numpy()
+    parts = _parts(x, devices)
+    xs = _replicas(x, parts)
+    labs = _replicas(torch.from_numpy(enc.astype(np.int32)), parts)
+    outs = {d: torch.empty(n, dtype=torch.float64, device=d) for d in xs}
+    for d, b, e in parts:   # every call synchronises its stream once (the label check), then leaves its kernel running
+        ws = torch.empty(lib.idl_silhouette_workspace_bytes(n, n_labels), dtype=torch.uint8, device=d)
+        with torch.cuda.device(d):
+            _lib.check(lib.idl_silhouette_samples_rows(_lib.ptr(xs[d]), _lib.ptr(labs[d]), n, D, n_labels, b, e, _lib.ptr(outs[d]),
+                                                       _lib.ptr(ws), ws.numel(), _lib.stream_ptr()))
+    out = np.empty(n, dtype=np.float64)
+    for d, b, e in parts:
+        out[b:e] = outs[d][b:e].cpu().numpy()
+    return out
 
 
-def silhouette_score_device(X, labels):
+def silhouette_score_device(X, labels, devices=None):
     """sklearn.metrics.silhouette_score(X, labels) (all samples, Euclidean metric): the mean of silhouette_samples_device,
     taken on the host as sklearn takes it."""
-    return float(np.mean(silhouette_samples_device(X, labels)))
+    return float(np.mean(silhouette_samples_device(X, labels, devices)))

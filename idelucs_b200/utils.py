@@ -388,15 +388,16 @@ def label_features(predictions, n_clusters):
     return np.array(y), D.max(axis=1)
 
 
-def compute_results(y_pred, data, y_true=None):
+def compute_results(y_pred, data, y_true=None, devices=None):
     """idelucs/utils.py:606-625: internal (and, with ground truth, external) clustering metrics -> (dict, assignment).
-    A CUDA tensor `data` gets its silhouette score on the GPU (metrics.silhouette_score_device) and its Davies-Bouldin
-    score from sklearn on a float64 host copy; numpy `data` goes to sklearn for both."""
+    A CUDA tensor `data` gets its silhouette score on the GPU (metrics.silhouette_score_device, split over `devices` when
+    that is a list of CUDA devices) and its Davies-Bouldin score from sklearn on a float64 host copy; numpy `data` goes to
+    sklearn for both."""
     from sklearn import metrics
     if torch.is_tensor(data) and data.is_cuda:
         from .metrics import silhouette_score_device
         host = data.cpu().numpy().astype(np.float64)
-        d = {"Davies-Boulding": metrics.davies_bouldin_score(host, y_pred), "Silhouette-Score": silhouette_score_device(data, y_pred)}
+        d = {"Davies-Boulding": metrics.davies_bouldin_score(host, y_pred), "Silhouette-Score": silhouette_score_device(data, y_pred, devices)}
     else:
         d = {"Davies-Boulding": metrics.davies_bouldin_score(data, y_pred), "Silhouette-Score": metrics.silhouette_score(data, y_pred)}
     if y_true is not None:

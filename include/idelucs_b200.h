@@ -346,6 +346,22 @@ size_t idl_hdbscan_workspace_bytes(int64_t n, int D);
 int idl_core_distances(const float* d_x, int64_t n, int D, int64_t k, double* d_core, void* d_ws, size_t ws_bytes, void* stream);
 int idl_mreach_mst(const float* d_x, const double* d_core, int64_t n, int D, int64_t* d_src, int64_t* d_dst, double* d_w, void* d_ws,
                    size_t ws_bytes, void* stream);
+/* The same work split by rows, for one process driving several devices; results are bit-identical to the calls above.
+ * idl_core_distances_rows: d_core[i] for the rows i of [row_begin, row_end) only (0 <= row_begin <= row_end <= n) of the
+ *   full-length d_core; every row still takes its k-th smallest distance over all n columns.  Same workspace as above.
+ * idl_mreach_mst_parts: idl_mreach_mst with every Borůvka round's all-pairs pass split into n_parts >= 1 row ranges
+ *   [row_begin[p], row_end[p]) that partition [0, n) in order (empty parts allowed).  Part p runs on device devices[p] (a
+ *   device may appear in several parts) with its own replicas d_x[p] and d_core[p] of the full x and core, its own workspace
+ *   d_ws[p] (ws_bytes[p] >= idl_hdbscan_workspace_bytes(n, D)) and streams[p], a stream of that device.  Per round the host
+ *   takes every component's lightest edge over the parts.  d_src / d_dst / d_w are written on devices[0] through
+ *   streams[0].  All arrays are HOST arrays of n_parts entries.  The call SYNCHRONISES every part's stream once per round
+ *   and streams[0] before it returns; the caller's current device is restored.  idl_mreach_mst is the one-part call on the
+ *   current device. */
+int idl_core_distances_rows(const float* d_x, int64_t n, int D, int64_t k, int64_t row_begin, int64_t row_end, double* d_core, void* d_ws,
+                            size_t ws_bytes, void* stream);
+int idl_mreach_mst_parts(int n_parts, const int* devices, const float* const* d_x, const double* const* d_core, const int64_t* row_begin,
+                         const int64_t* row_end, int64_t n, int D, int64_t* d_src, int64_t* d_dst, double* d_w, void* const* d_ws,
+                         const size_t* ws_bytes, void* const* streams);
 
 /* F4 — per-sample silhouette coefficients (sklearn.metrics.silhouette_samples, Euclidean metric), the internal
  * clustering metric the reference writes to metrics.tsv (idelucs/utils.py compute_results).  d_x: float32 [n, D]
@@ -365,6 +381,11 @@ int idl_mreach_mst(const float* d_x, const double* d_core, int64_t n, int D, int
 size_t idl_silhouette_workspace_bytes(int64_t n, int64_t n_labels);
 int idl_silhouette_samples(const float* d_x, const int32_t* d_labels, int64_t n, int D, int64_t n_labels, double* d_out, void* d_ws,
                            size_t ws_bytes, void* stream);
+/* the same for the rows of [row_begin, row_end) only (0 <= row_begin <= row_end <= n): d_out[i] for those rows of the
+ * full-length d_out, each row still against all n columns; the grouping, the label check and the synchronisation are those of
+ * idl_silhouette_samples.  Split over devices, every call computes bits identical to the one-call result. */
+int idl_silhouette_samples_rows(const float* d_x, const int32_t* d_labels, int64_t n, int D, int64_t n_labels, int64_t row_begin,
+                                int64_t row_end, double* d_out, void* d_ws, size_t ws_bytes, void* stream);
 
 #ifdef __cplusplus
 }
