@@ -12,6 +12,7 @@ LIB_PATH = os.environ.get("IDELUCS_B200_LIB") or os.path.join(_HERE, "lib", "lib
 IDL_OK = 0
 KIND_CLEAN, KIND_TRANSITION, KIND_TRANSVERSION, KIND_BOTH, KIND_RANDOM_N, KIND_EXPLICIT = range(6)
 OUT_COUNTS_I32, OUT_FREQ_F32, OUT_STD_F32, OUT_FREQ_F64 = range(4)
+OUT_CANON_F32, OUT_CANON_STD_F32, OUT_CANON_F64 = 9, 10, 11   # canonical k-mer rows (= 8 + the frequency kind)
 
 c_void_p, c_int, c_i64, c_u64, c_size_t, c_double, c_float = (
     ctypes.c_void_p, ctypes.c_int, ctypes.c_int64, ctypes.c_uint64, ctypes.c_size_t, ctypes.c_double, ctypes.c_float)

@@ -275,7 +275,7 @@ struct ChRedSmem {
 template <int K, int OUT>
 __global__ void __launch_bounds__(CH_NT, 2) ch_reduce_kernel(const ChParams cp, const __grid_constant__ Plan plan) {
     constexpr int F = CH_F, VEC = F / 4, VPT = VEC / CH_NT;
-    constexpr int ESZ = OUT == IDL_OUT_FREQ_F64 ? 8 : 4;
+    constexpr int ESZ = (OUT == IDL_OUT_FREQ_F64 || OUT == IDL_OUT_CANON_F64) ? 8 : 4;
     __shared__ ChRedSmem sm;
     const ProfParams& p = cp.p;
     const int tid = threadIdx.x, lane = tid & 31;
@@ -388,6 +388,21 @@ __global__ void __launch_bounds__(CH_NT, 2) ch_reduce_kernel(const ChParams cp, 
             const float y = 1.0f / ftot;
             const bool big = total >= (1 << 24);
             void* out_row = reinterpret_cast<unsigned char*>(p.out) + (size_t)ESZ * (size_t)(out_offs[s] + item * p.out_stride);
+            if constexpr (is_canon(OUT)) {
+                // canonical rows pair bins of different threads: the row goes through sm.hist (whose counts wait in registers)
+                int4 keep[VPT];
+#pragma unroll
+                for (int vv = 0; vv < VPT; ++vv) {
+                    const int vec = tid + vv * CH_NT;
+                    keep[vv] = reinterpret_cast<const int4*>(sm.hist)[vec];
+                    reinterpret_cast<int4*>(sm.hist)[vec] = row[vv];
+                }
+                __syncthreads();
+                emit_canon_row<K, CH_NT, OUT>(out_row, [&](uint32_t m) { return sm.hist[m] + p.pseudocount; }, p.mean, p.scale, sm.scan);
+                __syncthreads();
+#pragma unroll
+                for (int vv = 0; vv < VPT; ++vv) reinterpret_cast<int4*>(sm.hist)[tid + vv * CH_NT] = keep[vv];
+            } else {
 #pragma unroll
             for (int vv = 0; vv < VPT; ++vv) {
                 const int vec = tid + vv * CH_NT;
@@ -404,6 +419,7 @@ __global__ void __launch_bounds__(CH_NT, 2) ch_reduce_kernel(const ChParams cp, 
                     rscale[0] = rs.x; rscale[1] = rs.y; rscale[2] = rs.z; rscale[3] = rs.w;
                 }
                 emit_granule<OUT>(out_row, vec, ci, cf, total, ftot, y, big, p.accumulate, mean, scale, rscale);
+            }
             }
             __syncthreads();
             if (kind == KIND_RANDOM_N) {   // undo the removals

@@ -220,6 +220,78 @@ __device__ __forceinline__ int block_exscan(int v, int* scratch, int* total) {
 }
 
 // ---------------------------------------------------------------------------------------
+// canonical (reverse-complement folded) rows: IDL_OUT_CANON_* = 8 + the matching frequency kind
+// ---------------------------------------------------------------------------------------
+constexpr int OUT_CANON_BIT = 8;
+constexpr bool is_canon(int out) { return (out & OUT_CANON_BIT) != 0; }
+
+// utils.py:191-206: index of the reverse complement of k-mer m
+constexpr uint32_t revcomp_index(uint32_t m, int k) {
+    uint32_t x = ~m & ((k < 16 ? (1u << (2 * k)) : 0u) - 1u), r = 0;
+    for (int t = 0; t < k; ++t) { r = (r << 2) | (x & 3u); x >>= 2; }
+    return r;
+}
+constexpr int canonical_count(int k) {
+    int R = 0;
+    for (uint32_t m = 0; m < (1u << (2 * k)); ++m) R += m <= revcomp_index(m, k) ? 1 : 0;
+    return R;
+}
+// the canonical k-mers of idl_revcomp_canonical (kmer <= revcomp, increasing), entry = kmer | revcomp << 16; built by the
+// compiler into the module's global data (8.3 KB at k = 6)
+template <int K>
+struct CanonTab {
+    static constexpr int R = canonical_count(K);
+    uint32_t e[R];
+    constexpr CanonTab() : e{} {
+        int r = 0;
+        for (uint32_t m = 0; m < (1u << (2 * K)); ++m) {
+            const uint32_t c = revcomp_index(m, K);
+            if (m <= c) e[r++] = m | (c << 16);
+        }
+    }
+};
+template <int K>
+__device__ const CanonTab<K> g_canon = CanonTab<K>();
+
+// One canonical row, CTA-wide (contains barriers: every thread of the CTA calls it).  cnt(m) = count of k-mer m plus the
+// pseudocount, read from shared memory.  f_r = int((a + b) * 0.5) over the pair (m_r, revcomp(m_r)) (revcomp_fold_kernel's
+// rule), T = the exact integer sum of the f_r (a reduction before the first store), then normalize_counts_kernel's float64
+// division; the float32 kinds round that quotient and the standardised kind applies idl_standardize_f32's IEEE
+// (x - mean32) / scale32.  A thread stores columns r = tid + j NT: scalar, coalesced, any offset and stride.
+template <int K, int NT, int OUT, class Cnt>
+__device__ __forceinline__ void emit_canon_row(void* out_row, Cnt cnt, const float* mean, const float* scale, int* scan) {
+    constexpr int R = CanonTab<K>::R, RPT = (R + NT - 1) / NT;
+    int f[RPT];
+    int part = 0;
+#pragma unroll
+    for (int j = 0; j < RPT; ++j) {
+        const int r = threadIdx.x + j * NT;
+        f[j] = 0;
+        if (R % NT == 0 || r < R) {
+            const uint32_t e = __ldg(&g_canon<K>.e[r]);
+            f[j] = (int)((double)(cnt(e & 0xFFFFu) + cnt(e >> 16)) * 0.5);
+            part += f[j];
+        }
+    }
+    int total;
+    block_exscan<NT>(part, scan, &total);
+    const double dt = (double)total;
+#pragma unroll
+    for (int j = 0; j < RPT; ++j) {
+        const int r = threadIdx.x + j * NT;
+        if (R % NT != 0 && r >= R) break;
+        const double q = (double)f[j] / dt;
+        if (OUT == IDL_OUT_CANON_F64) {
+            __stcs(reinterpret_cast<double*>(out_row) + r, q);
+        } else {
+            float x = (float)q;
+            if (OUT == IDL_OUT_CANON_STD_F32) x = (x - __ldg(mean + r)) / __ldg(scale + r);
+            __stcs(reinterpret_cast<float*>(out_row) + r, x);
+        }
+    }
+}
+
+// ---------------------------------------------------------------------------------------
 // K2/K3 profiles kernel
 //
 // Per work item (one sequence) a CTA
@@ -445,7 +517,7 @@ __device__ __noinline__ void long_path(ProfSmem<K, NT>& sm, const ProfParams& p,
                                        const long long* out_offs, long long item, long long seq, int base_total) {
     using C = ProfCfg<K, NT>;
     constexpr int VEC = C::VEC, VPT = C::VPT;
-    constexpr int ESZ = OUT == IDL_OUT_FREQ_F64 ? 8 : 4;
+    constexpr int ESZ = (OUT == IDL_OUT_FREQ_F64 || OUT == IDL_OUT_CANON_F64) ? 8 : 4;
     const int tid = threadIdx.x, lane = tid & 31;
     const int L = cx.L;
     const int nblocks = (L + RNG_BLOCK - 1) / RNG_BLOCK;
@@ -487,6 +559,9 @@ __device__ __noinline__ void long_path(ProfSmem<K, NT>& sm, const ProfParams& p,
                 const float y = 1.0f / ftot;
                 const bool big = total >= (1 << 24);
                 void* row = reinterpret_cast<unsigned char*>(p.out) + (size_t)ESZ * (size_t)(out_offs[s] + item * p.out_stride);
+                if constexpr (is_canon(OUT)) {
+                    emit_canon_row<K, NT, OUT>(row, [&](uint32_t m) { return sm.hist[m] + p.pseudocount; }, p.mean, p.scale, sm.scan);
+                } else {
 #pragma unroll
                 for (int vv = 0; vv < VPT; ++vv) {
                     const int vec = tid + vv * NT;
@@ -504,6 +579,7 @@ __device__ __noinline__ void long_path(ProfSmem<K, NT>& sm, const ProfParams& p,
                         rscale[0] = rs.x; rscale[1] = rs.y; rscale[2] = rs.z; rscale[3] = rs.w;
                     }
                     emit_granule<OUT>(row, vec, ci, cf, total, ftot, y, big, p.accumulate, mean, scale, rscale);
+                }
                 }
                 __syncthreads();
             }
@@ -589,7 +665,7 @@ template <int K, int NT, int OUT>
 __global__ void __launch_bounds__(NT, (K == 6 ? 2 : K == 5 ? 4 : 8)) profiles_kernel(const ProfParams p, const __grid_constant__ Plan plan) {
     using C = ProfCfg<K, NT>;
     constexpr int F = C::F, VEC = C::VEC, VPT = C::VPT, G = C::G, PRIVW = C::PRIVW;
-    constexpr int ESZ = OUT == IDL_OUT_FREQ_F64 ? 8 : 4;
+    constexpr int ESZ = (OUT == IDL_OUT_FREQ_F64 || OUT == IDL_OUT_CANON_F64) ? 8 : 4;
     constexpr bool NEED_F = (OUT == IDL_OUT_FREQ_F32 || OUT == IDL_OUT_STD_F32);
     extern __shared__ __align__(16) unsigned char smem_raw[];
     ProfSmem<K, NT>& sm = *reinterpret_cast<ProfSmem<K, NT>*>(smem_raw);
@@ -944,6 +1020,24 @@ __global__ void __launch_bounds__(NT, (K == 6 ? 2 : K == 5 ? 4 : 8)) profiles_ke
                 const int hs_next = has_next ? (NSg - h0 - HG < HG ? NSg - h0 - HG : HG) : 0;
                 const bool next_cta = has_next && ((cta_mask >> (h0 + HG)) & ((1u << HG) - 1u)) != 0u;
                 if (has_next && !next_cta) patch_half(h0 + HG, hs_next, cur ^ 1);
+                if constexpr (is_canon(OUT)) {
+                    // ---- canonical rows read both bins of a reverse-complement pair, which other threads' granules hold:
+                    // ---- slot by slot from the copies, then (after every read) the copies are restored ----
+                    for (int c = 0; c < hs; ++c) {
+                        const uint32_t* cp = priv + (cur * HG + c) * PRIVW;
+                        emit_canon_row<K, NT, OUT>(
+                            reinterpret_cast<unsigned char*>(p.out) + sm.grow[h0 + c],
+                            [&](uint32_t m) { return (int)((cp[m >> 1] >> ((m & 1u) * 16u)) & 0xFFFFu) + p.pseudocount; }, p.mean, p.scale, sm.scan);
+                    }
+                    __syncthreads();
+#pragma unroll
+                    for (int vv = 0; vv < VPT; ++vv) {
+                        const int vec = tid + vv * NT;
+                        if (VEC % NT != 0 && vec >= VEC) break;
+                        const uint2 clean = clean16[vec];
+                        for (int c = 0; c < hs; ++c) reinterpret_cast<uint2*>(priv + (cur * HG + c) * PRIVW)[vec] = clean;
+                    }
+                } else {
                 // ---- stream the hs profiles of this half-group (and restore its copies) ----
                 // granule-major: the scaler statistics of ONE granule (12 registers) are live at a time
 #pragma unroll
@@ -970,6 +1064,7 @@ __global__ void __launch_bounds__(NT, (K == 6 ? 2 : K == 5 ? 4 : 8)) profiles_ke
                             emit_granule<OUT>(row, vec, ci, cf, base_total + sm.dtot[h0 + c], fy.x, fy.y, false, p.accumulate, mean, scale, rscale);
                         }
                     }
+                }
                 }
                 __syncthreads();
                 if (next_cta) {
@@ -1221,13 +1316,6 @@ IDL_HD uint32_t cgr_index(uint32_t m, int k) {
     }
     return (ci << k) | cj;
 }
-// utils.py:191-206: index of the reverse complement of k-mer m
-IDL_HD uint32_t revcomp_index(uint32_t m, int k) {
-    uint32_t x = ~m & ((k < 16 ? (1u << (2 * k)) : 0u) - 1u), r = 0;
-    for (int t = 0; t < k; ++t) { r = (r << 2) | (x & 3u); x >>= 2; }
-    return r;
-}
-
 __global__ void cgr_map_kernel(const int32_t* __restrict__ counts, int32_t* __restrict__ cgr, long long total, int k, int accumulate) {
     const long long F = 1ll << (2 * k);
     for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
@@ -1282,16 +1370,26 @@ constexpr size_t WS_TOTAL = WS_RSCALE + sizeof(float) * 4096;
 
 // the instantiation of a kernel template for an output kind (nullptr for an unknown kind)
 template <typename Kernel>
-static Kernel kernel_for_out(int out_kind, Kernel stats, Kernel counts_i32, Kernel freq_f32, Kernel std_f32, Kernel freq_f64) {
+static Kernel kernel_for_out(int out_kind, Kernel stats, Kernel counts_i32, Kernel freq_f32, Kernel std_f32, Kernel freq_f64, Kernel canon_f32,
+                             Kernel canon_std_f32, Kernel canon_f64) {
     static_assert(IDL_OUT_COUNTS_I32 == 0 && IDL_OUT_FREQ_F32 == 1 && IDL_OUT_STD_F32 == 2 && IDL_OUT_FREQ_F64 == 3 && OUT_STATS == 4, "by_kind order");
+    static_assert(IDL_OUT_CANON_F32 == OUT_CANON_BIT + IDL_OUT_FREQ_F32 && IDL_OUT_CANON_STD_F32 == OUT_CANON_BIT + IDL_OUT_STD_F32 &&
+                  IDL_OUT_CANON_F64 == OUT_CANON_BIT + IDL_OUT_FREQ_F64, "canonical kinds = 8 + frequency kind");
     const Kernel by_kind[] = {counts_i32, freq_f32, std_f32, freq_f64, stats};
+    const Kernel canon_by_kind[] = {nullptr, canon_f32, canon_std_f32, canon_f64};
+    if (out_kind >= IDL_OUT_CANON_F32 && out_kind <= IDL_OUT_CANON_F64) return canon_by_kind[out_kind - OUT_CANON_BIT];
     return out_kind >= 0 && out_kind <= OUT_STATS ? by_kind[out_kind] : nullptr;
+}
+// the output kinds the public entry points accept
+static bool public_out_kind(int out_kind) {
+    return (out_kind >= IDL_OUT_COUNTS_I32 && out_kind <= IDL_OUT_FREQ_F64) || (out_kind >= IDL_OUT_CANON_F32 && out_kind <= IDL_OUT_CANON_F64);
 }
 
 template <int K, int NT>
 static int launch_profiles(const ProfParams& p, const Plan& plan, int out_kind, cudaStream_t st, int* grid_out) {
     const auto kern = kernel_for_out(out_kind, profiles_kernel<K, NT, OUT_STATS>, profiles_kernel<K, NT, IDL_OUT_COUNTS_I32>, profiles_kernel<K, NT, IDL_OUT_FREQ_F32>,
-                                     profiles_kernel<K, NT, IDL_OUT_STD_F32>, profiles_kernel<K, NT, IDL_OUT_FREQ_F64>);
+                                     profiles_kernel<K, NT, IDL_OUT_STD_F32>, profiles_kernel<K, NT, IDL_OUT_FREQ_F64>, profiles_kernel<K, NT, IDL_OUT_CANON_F32>,
+                                     profiles_kernel<K, NT, IDL_OUT_CANON_STD_F32>, profiles_kernel<K, NT, IDL_OUT_CANON_F64>);
     if (!kern) return set_error(IDL_EINVAL, "unknown out_kind%s %lld", "", out_kind);
     const size_t smem = sizeof(ProfSmem<K, NT>);
     unsigned grid = 0;
@@ -1477,10 +1575,12 @@ static int profiles_impl(const ProfCall& c) {
     if (c.n_variants < 1 || c.n_variants > MAX_VARIANTS || c.S < 1 || c.S > MAX_VARIANTS)
         return set_error(IDL_EINVAL, "idl_profiles: n_variants / S out of range%s", "");
     if (!c.sel && c.S != c.n_variants) return set_error(IDL_EINVAL, "idl_profiles: S must equal n_variants without d_sel%s", "");
-    if (c.out_kind == IDL_OUT_STD_F32 && (!c.mean || !c.scale)) return set_error(IDL_EINVAL, "idl_profiles: mean/scale required%s", "");
+    if ((c.out_kind == IDL_OUT_STD_F32 || c.out_kind == IDL_OUT_CANON_STD_F32) && (!c.mean || !c.scale))
+        return set_error(IDL_EINVAL, "idl_profiles: mean/scale required%s", "");
     if ((c.accumulate & 1) && c.out_kind != IDL_OUT_COUNTS_I32) return set_error(IDL_EINVAL, "idl_profiles: accumulate only for counts%s", "");
     if (c.n_items <= 0) return IDL_OK;
-    if (c.out_stride % 4 != 0) return set_error(IDL_EINVAL, "idl_profiles: out_stride must be a multiple of 4%s", "");
+    // (canonical rows are written one element at a time: any stride)
+    if (c.out_stride % 4 != 0 && !is_canon(c.out_kind)) return set_error(IDL_EINVAL, "idl_profiles: out_stride must be a multiple of 4%s", "");
 
     HostPlan hp;
     ProfParams p;
@@ -1515,7 +1615,9 @@ static int profiles_impl(const ProfCall& c) {
                 if (rgrid > c.n_items) rgrid = c.n_items;
                 using ReduceKernel = void (*)(ChParams, Plan);   // (OUT_STATS requests returned above)
                 const ReduceKernel reduce = kernel_for_out<ReduceKernel>(c.out_kind, nullptr, ch_reduce_kernel<6, IDL_OUT_COUNTS_I32>, ch_reduce_kernel<6, IDL_OUT_FREQ_F32>,
-                                                                         ch_reduce_kernel<6, IDL_OUT_STD_F32>, ch_reduce_kernel<6, IDL_OUT_FREQ_F64>);
+                                                                         ch_reduce_kernel<6, IDL_OUT_STD_F32>, ch_reduce_kernel<6, IDL_OUT_FREQ_F64>,
+                                                                         ch_reduce_kernel<6, IDL_OUT_CANON_F32>, ch_reduce_kernel<6, IDL_OUT_CANON_STD_F32>,
+                                                                         ch_reduce_kernel<6, IDL_OUT_CANON_F64>);
                 reduce<<<(unsigned)rgrid, CH_NT, 0, c.st>>>(cp, hp.plan); note_launch();
                 IDL_CUDA_CHECK(cudaGetLastError());
                 p.long_overflow = &cp.hdr->overflow;   // the generic kernel skips the long items (unless the plan found more than max_long)
@@ -1589,7 +1691,7 @@ int idl_profiles(const uint32_t* d_codes, const uint32_t* d_nmask, const int64_t
                  void* d_out, const int64_t* out_off, int64_t out_stride, int pseudocount, int accumulate,
                  const float* d_mean, const float* d_scale, int32_t* d_status, void* d_workspace,
                  size_t workspace_bytes, void* stream) {
-    if (out_kind < IDL_OUT_COUNTS_I32 || out_kind > IDL_OUT_FREQ_F64) return set_error(IDL_EINVAL, "idl_profiles: unknown out_kind%s %lld", "", out_kind);
+    if (!public_out_kind(out_kind)) return set_error(IDL_EINVAL, "idl_profiles: unknown out_kind%s %lld", "", out_kind);
     ProfCall c = prof_call(d_codes, d_nmask, d_chunk_off, d_len, n_seqs_total, d_sidx, n_items, seq_id0, k, variants, n_variants, seed, d_workspace, workspace_bytes, stream);
     c.sel = d_sel; c.S = S; c.edit_off = d_edit_off; c.edits = d_edits; c.out_kind = out_kind; c.out = d_out; c.out_off = out_off;
     c.out_stride = out_stride; c.pseudocount = pseudocount; c.accumulate = accumulate; c.mean = d_mean; c.scale = d_scale; c.status = d_status;
@@ -1611,7 +1713,7 @@ int idl_profiles_chunked(const uint32_t* d_codes, const uint32_t* d_nmask, const
                          void* d_out, const int64_t* out_off, int64_t out_stride, int pseudocount, int accumulate,
                          const float* d_mean, const float* d_scale, void* d_scratch, size_t scratch_bytes, int64_t max_long_items,
                          void* d_workspace, size_t workspace_bytes, void* stream) {
-    if (out_kind < IDL_OUT_COUNTS_I32 || out_kind > IDL_OUT_FREQ_F64) return set_error(IDL_EINVAL, "idl_profiles_chunked: unknown out_kind%s %lld", "", out_kind);
+    if (!public_out_kind(out_kind)) return set_error(IDL_EINVAL, "idl_profiles_chunked: unknown out_kind%s %lld", "", out_kind);
     if (!d_scratch || max_long_items < 0) return set_error(IDL_EINVAL, "idl_profiles_chunked: scratch required%s", "");
     ProfCall c = prof_call(d_codes, d_nmask, d_chunk_off, d_len, n_seqs_total, d_sidx, n_items, seq_id0, k, variants, n_variants, seed, d_workspace, workspace_bytes, stream);
     c.sel = d_sel; c.S = S; c.edit_off = d_edit_off; c.edits = d_edits; c.out_kind = out_kind; c.out = d_out; c.out_off = out_off;
@@ -1626,6 +1728,8 @@ int idl_profiles_prepared(const uint32_t* d_codes, const uint32_t* d_nmask, cons
                           void* d_out, const int64_t* out_off, int64_t out_stride, int pseudocount,
                           const float* d_mean, const float* d_scale, int32_t* d_status, const void* d_prep, size_t prep_size,
                           void* d_workspace, size_t workspace_bytes, void* stream) {
+    if (public_out_kind(out_kind) && is_canon(out_kind))
+        return set_error(IDL_EINVAL, "idl_profiles_prepared: canonical output kinds are not supported (use idl_profiles or idl_profiles_chunked)%s", "");
     if (out_kind != IDL_OUT_FREQ_F32 && out_kind != IDL_OUT_STD_F32) return set_error(IDL_EINVAL, "idl_profiles_prepared: float32 outputs only%s", "");
     if (!d_prep || !d_status) return set_error(IDL_EINVAL, "idl_profiles_prepared: d_prep and d_status are required%s", "");
     ProfCall c = prof_call(d_codes, d_nmask, d_chunk_off, d_len, n_seqs_total, d_sidx, n_items, seq_id0, k, variants, n_variants, seed, d_workspace, workspace_bytes, stream);

@@ -7,10 +7,12 @@ import torch
 
 from . import _lib
 from ._lib import (KIND_BOTH, KIND_CLEAN, KIND_EXPLICIT, KIND_RANDOM_N, KIND_TRANSITION, KIND_TRANSVERSION,  # noqa: F401
-                   OUT_COUNTS_I32, OUT_FREQ_F32, OUT_FREQ_F64, OUT_STD_F32)
+                   OUT_CANON_F32, OUT_CANON_F64, OUT_CANON_STD_F32, OUT_COUNTS_I32, OUT_FREQ_F32, OUT_FREQ_F64, OUT_STD_F32)
 
 _OUT_DTYPE = {OUT_COUNTS_I32: torch.int32, OUT_FREQ_F32: torch.float32, OUT_STD_F32: torch.float32,
-              OUT_FREQ_F64: torch.float64}
+              OUT_FREQ_F64: torch.float64, OUT_CANON_F32: torch.float32, OUT_CANON_STD_F32: torch.float32,
+              OUT_CANON_F64: torch.float64}
+CANON_KINDS = (OUT_CANON_F32, OUT_CANON_STD_F32, OUT_CANON_F64)
 
 LONG_MIN = 65536   # items at least this long take the chunked path (csrc/chunked.cuh)
 MAX_EDIT_POS = 1 << 29   # edit entries are pos << 3 | val in 32 bits: mutated variants need sequences shorter than this
@@ -179,13 +181,14 @@ def profiles(seqset, k, variants, out_kind=OUT_FREQ_F32, seed=0, out=None, out_o
              mean=None, scale=None, sidx=None, sel=None, S=None, edit_lists=None, seq_id0=0, pseudocount=None,
              accumulate=False, status=None, prepared=None, chunked=None, max_long=None, cta_cap=0):
     """Run K2+K3.  Default output: tensor [S, n_items, 4^k] (variant-major) of the out_kind's
-    dtype.  See include/idelucs_b200.h::idl_profiles for the argument meaning.  ``prepared`` (from ``prepare`` with the
+    dtype; [S, n_items, R] (R = canonical_width(k)) for the canonical kinds OUT_CANON_*.  See
+    include/idelucs_b200.h::idl_profiles for the argument meaning.  ``prepared`` (from ``prepare`` with the
     same SeqSet / variants / seed / seq_id0) routes float32 outputs through idl_profiles_prepared (k = 6 fast path).  Sets with
     sequences of >= 65 536 bases go through idl_profiles_chunked (k = 6; chunked=False forces the generic kernel).  ``cta_cap`` > 0
     caps the generic kernel at that many CTAs per SM (room for a concurrent stream)."""
     lib = _lib.load()
     device = seqset.device
-    F = 4 ** k
+    F = canonical_width(k) if out_kind in CANON_KINDS else 4 ** k
     n_items = int(sidx.numel()) if sidx is not None else seqset.n
     nv = len(variants)
     if S is None:
@@ -339,6 +342,11 @@ def canonical_index(k, device):
     return _canon_cache[key]
 
 
+def canonical_width(k):
+    """R: the number of canonical k-mers, the width of a row of the canonical output kinds (idl_revcomp_canonical)"""
+    return _lib.load().idl_revcomp_canonical(k, None)
+
+
 def revcomp_fold(counts, k):
     """kmer_rev_comp on int32 counts [..., 4^k] (pseudocount included) -> int32 [..., R] (idl_revcomp_fold)"""
     lib = _lib.load()
@@ -366,9 +374,12 @@ def normalize_counts(counts, want64=True, want32=False):
 
 def reduced_profiles(seqset, k, variants, seed=0, edit_lists=None, seq_id0=0, want64=True, want32=False):
     """reduce=True path of kmersFasta (idelucs/utils.py:246-250): +1-pseudocount counts of every variant ->
-    canonical folding -> counts / sum.  Returns [V, N, R] float64 and / or float32."""
-    c = profiles(seqset, k, variants, out_kind=OUT_COUNTS_I32, seed=seed, edit_lists=edit_lists, seq_id0=seq_id0, pseudocount=1)
-    return normalize_counts(revcomp_fold(c, k), want64=want64, want32=want32)
+    canonical folding -> counts / sum, folded in the profile kernel's row emission (OUT_CANON_F64 / OUT_CANON_F32: the
+    values of ``normalize_counts(revcomp_fold(counts + 1))`` without the [V, N, 4^k] counts).  Returns [V, N, R] float64
+    and / or float32."""
+    kinds = ([OUT_CANON_F64] if want64 else []) + ([OUT_CANON_F32] if want32 else [])
+    res = tuple(profiles(seqset, k, variants, out_kind=o, seed=seed, edit_lists=edit_lists, seq_id0=seq_id0, pseudocount=1) for o in kinds)
+    return res[0] if len(res) == 1 else res
 
 
 class Scaler(object):

@@ -214,6 +214,13 @@ def cgrFasta(fname, k=6, transform=None):
     return list(ss.names), _to_host(ft.normalize_counts(cells))
 
 
+def canonical_scaler(ss, k, variants, seed, seq_id0=0, group=None):
+    """Scaler of the t_norm slot's float32 canonical rows: the [N, R] matrix is written (OUT_CANON_F32) and fitted by
+    idl_colstats like every other matrix, then freed"""
+    x0 = ft.profiles(ss, k, variants[:1], out_kind=ft.OUT_CANON_F32, seed=seed, seq_id0=seq_id0)[0]
+    return ft.Scaler.fit(x0, group=group)
+
+
 def augment_device(ss, n_mimics, k=6, seed=None, group=None, seq_id0=0, reduce=False):
     """Device-resident AugmentFasta: returns (profiles float32 [n_mimics+1, N, 4^k] — slot 0 =
     t_norm, slot j = mimic j — standardised with the t_norm statistics, and the Scaler).
@@ -221,10 +228,9 @@ def augment_device(ss, n_mimics, k=6, seed=None, group=None, seq_id0=0, reduce=F
     seed = _draw_seed() if seed is None else seed
     variants = ft.mimic_schedule(n_mimics)
     if reduce:
-        x32 = ft.reduced_profiles(ss, k, variants, seed=seed, seq_id0=seq_id0, want64=False, want32=True)
-        sc = ft.Scaler.fit(x32[0], group=group)
-        V, n, R = x32.shape
-        return sc.transform32(x32.reshape(V * n, R)).reshape(V, n, R), sc, seed
+        sc = canonical_scaler(ss, k, variants, seed, seq_id0, group)
+        out = ft.profiles(ss, k, variants, out_kind=ft.OUT_CANON_STD_F32, seed=seed, seq_id0=seq_id0, mean=sc.mean32, scale=sc.scale32)
+        return out, sc, seed
     # t_norm statistics (never materialised) and all standardised slots; k = 6: the prepare pass generates the Bernoulli
     # mimics once for both
     out, sc = ft.schedule_profiles(ss, k, variants, out_kind=ft.OUT_STD_F32, seed=seed, seq_id0=seq_id0, group=group)
@@ -264,7 +270,8 @@ class PairBatchLoader(object):
     (sequence i, mimic j); the pair set is fixed for the whole run like the reference's
     (same seed => same mimic).  When the standardised profiles fit ``materialize_bytes`` they
     are produced once and batches are gathers; otherwise every batch is regenerated from the
-    packed sequences by the mimic kernel (selection mode), which gives identical values."""
+    packed sequences by the mimic kernel (selection mode), which gives identical values.
+    reduce=True (model_size 'small') follows the same rule with the canonical-k-mer rows (R columns)."""
 
     def __init__(self, ss, n_mimics, k=6, batch_size=512, seed=None, materialize_bytes=8 << 30, group=None,
                  seq_id0=0, drop_last=False, reduce=False):
@@ -273,13 +280,15 @@ class PairBatchLoader(object):
         self.n_pairs = (len(self.variants) - 1) * ss.n
         self.seed = _draw_seed() if seed is None else seed
         self.seq_id0 = seq_id0
-        F = 4 ** k
-        if reduce:   # canonical-k-mer profiles (model_size 'small'): always materialised
-            self.profiles, self.scaler, _ = augment_device(ss, n_mimics, k, seed=self.seed, group=group, seq_id0=seq_id0, reduce=True)
-        elif len(self.variants) * ss.n * F * 4 <= materialize_bytes:
-            self.profiles, self.scaler, _ = augment_device(ss, n_mimics, k, seed=self.seed, group=group, seq_id0=seq_id0)
+        self.out_kind = ft.OUT_CANON_STD_F32 if reduce else ft.OUT_STD_F32
+        F = ft.canonical_width(k) if reduce else 4 ** k
+        if len(self.variants) * ss.n * F * 4 <= materialize_bytes:
+            self.profiles, self.scaler, _ = augment_device(ss, n_mimics, k, seed=self.seed, group=group, seq_id0=seq_id0, reduce=reduce)
         else:
-            self.scaler = ft.profile_stats(ss, k, self.variants[0], seed=self.seed, seq_id0=seq_id0, group=group)
+            if reduce:
+                self.scaler = canonical_scaler(ss, k, self.variants, self.seed, seq_id0, group)
+            else:
+                self.scaler = ft.profile_stats(ss, k, self.variants[0], seed=self.seed, seq_id0=seq_id0, group=group)
             self.profiles = None
 
     def __len__(self):
@@ -300,7 +309,7 @@ class PairBatchLoader(object):
         lib = _lib.load()
         with torch.cuda.device(pair_ids.device):
             _lib.check(lib.idl_pair_selection(_lib.ptr(ids), B, n, _lib.ptr(sidx), _lib.ptr(sel), _lib.stream_ptr()))
-        out = ft.profiles(self.ss, self.k, self.variants, out_kind=ft.OUT_STD_F32, seed=self.seed, sidx=sidx,
+        out = ft.profiles(self.ss, self.k, self.variants, out_kind=self.out_kind, seed=self.seed, sidx=sidx,
                           sel=sel, mean=self.scaler.mean32, scale=self.scaler.scale32, seq_id0=self.seq_id0, cta_cap=cta_cap)
         return {"true": out[0], "modified": out[1], "both": out.view(-1, out.shape[-1])}   # 'both' = the two sides stacked, no copy
 

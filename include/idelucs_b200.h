@@ -55,7 +55,12 @@ enum {
     IDL_OUT_COUNTS_I32 = 0, /* raw window counts, no pseudocount (kmers.pyx:2-50) */
     IDL_OUT_FREQ_F32 = 1,   /* float32((count+pc)/sum)  (utils.py:242-250 then :353 astype) */
     IDL_OUT_STD_F32 = 2,    /* (freq32 - mean32) / scale32  (utils.py:358-366 via sklearn) */
-    IDL_OUT_FREQ_F64 = 3    /* float64 (count+pc)/sum  (utils.py:250) */
+    IDL_OUT_FREQ_F64 = 3,   /* float64 (count+pc)/sum  (utils.py:250) */
+    /* canonical k-mer rows of kmersFasta(reduce=True) (utils.py:246-250): R = idl_revcomp_canonical(k) columns in its order;
+     * each value is 8 + the matching frequency kind */
+    IDL_OUT_CANON_F32 = 9,      /* float32 of IDL_OUT_CANON_F64's float64 quotient */
+    IDL_OUT_CANON_STD_F32 = 10, /* (canon32 - mean32[r]) / scale32[r], IEEE float32 */
+    IDL_OUT_CANON_F64 = 11      /* float64 f_r / T */
 };
 
 /* One mimic variant.  rng_id is the variant's identity in the counter-based RNG, so the
@@ -107,7 +112,13 @@ size_t idl_profiles_workspace_bytes(void);
  * val 0..3 = set A/C/G/T, 4 = set N; position-sorted and unique per list; positions < 2^29, which also bounds the length of
  * sequences that take a non-clean variant — clean counting accepts any length < 2^31), n_seqs_total =
  * number of sequences the CSR is indexed over.  d_mean/d_scale: float32[4^k] for
- * IDL_OUT_STD_F32.  accumulate: bit 0 set (COUNTS only) adds into d_out like kmers.pyx does; bits 8..15 = n > 0 caps the generic
+ * IDL_OUT_STD_F32.
+ * Canonical kinds (IDL_OUT_CANON_*): row width R = idl_revcomp_canonical(k), column r = canonical k-mer m_r of that list.
+ * With a = count[m_r] + pseudocount and b = count[revcomp(m_r)] + pseudocount, f_r = int((a + b) * 0.5) (a palindrome gives
+ * a) and T = sum of the R values f_r (an exact integer, not the window total); CANON_F64 = f_r / T in float64, CANON_F32 =
+ * float32 of that quotient, CANON_STD_F32 = (CANON_F32 - d_mean[r]) / d_scale[r] with d_mean / d_scale float32[R].  This is
+ * idl_normalize_counts(idl_revcomp_fold(counts + pseudocount)) bit for bit, without the [n, 4^k] count rows.  Any out_off /
+ * out_stride; idl_profiles_chunked takes them too, idl_profiles_prepared does not.  accumulate: bit 0 set (COUNTS only) adds into d_out like kmers.pyx does; bits 8..15 = n > 0 caps the generic
  * kernel at n CTAs per SM (a caller that overlaps the call with other work on another stream leaves room for it; 0 = fill the GPU).
  * d_status int32[n_items] (optional, zero on entry): scratch flags of the fast kernels (bit 1 marks items handed to the generic
  * kernel inside a call; clear again when the work is done).  No rate or length makes a mutation get dropped: edit lists that
