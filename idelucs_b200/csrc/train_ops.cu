@@ -757,6 +757,9 @@ int iid_loss_small_launch(const float* d_z1, const float* d_z2, int B, int C, fl
 
 using namespace idl;
 
+// the float4 kernels below need 16-byte aligned buffers (a torch view at an odd storage offset is not): rejected, not faulted on
+static bool misaligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) != 0; }
+
 extern "C" {
 
 int idl_nce_normalize(const float* d_h, int n2, int D, float* d_fn, float* d_inv_norm, void* stream) {
@@ -817,6 +820,8 @@ int idl_relu_dropout_forward(const float* d_parts, int n_parts, const float* d_b
                              uint32_t tag, float* d_out, void* stream) {
     if (!d_parts || !d_out || n_parts < 1 || M < 1 || N < 4 || (N & 3) || !(p >= 0.f) || !(p < 1.f))
         return set_error(IDL_EINVAL, "idl_relu_dropout_forward: bad argument%s (N must be a multiple of 4, 0 <= p < 1)", "");
+    if (misaligned16(d_parts) || misaligned16(d_bias) || misaligned16(d_out))
+        return set_error(IDL_EINVAL, "idl_relu_dropout_forward: misaligned buffer%s (parts, bias and out are read and written as float4)", "");
     const long long n4 = (long long)M * N / 4;
     const double th = (double)p * 4294967296.0;
     const uint32_t thresh = th >= 4294967295.0 ? 0xFFFFFFFFu : (uint32_t)th;
@@ -831,6 +836,8 @@ int idl_relu_dropout_forward(const float* d_parts, int n_parts, const float* d_b
 
 int idl_sum_parts_bias(const float* d_parts, int n_parts, const float* d_bias, int64_t M, int N, float* d_out, void* stream) {
     if (!d_parts || !d_out || n_parts < 1 || M < 1 || N < 4 || (N & 3)) return set_error(IDL_EINVAL, "idl_sum_parts_bias: bad argument%s (N must be a multiple of 4)", "");
+    if (misaligned16(d_parts) || misaligned16(d_bias) || misaligned16(d_out))
+        return set_error(IDL_EINVAL, "idl_sum_parts_bias: misaligned buffer%s (parts, bias and out are read and written as float4)", "");
     const long long n4 = (long long)M * N / 4;
     long long grid = (n4 + 255) / 256;
     if (grid > 148 * 8) grid = 148 * 8;
@@ -842,6 +849,8 @@ int idl_sum_parts_bias(const float* d_parts, int n_parts, const float* d_bias, i
 
 int idl_relu_dropout_backward(const float* d_out, const float* d_dy, int64_t n, float p, float* d_dx, void* stream) {
     if (!d_out || !d_dy || !d_dx || n < 4 || (n & 3) || !(p >= 0.f) || !(p < 1.f)) return set_error(IDL_EINVAL, "idl_relu_dropout_backward: bad argument%s", "");
+    if (misaligned16(d_out) || misaligned16(d_dy) || misaligned16(d_dx))
+        return set_error(IDL_EINVAL, "idl_relu_dropout_backward: misaligned buffer%s (out, dy and dx are read and written as float4)", "");
     long long grid = (n / 4 + 255) / 256;
     if (grid > 148 * 8) grid = 148 * 8;
     relu_dropout_bwd_kernel<<<(unsigned)grid, 256, 0, (cudaStream_t)stream>>>(d_out, d_dy, n / 4, 1.0f / (1.0f - p), d_dx);
@@ -877,6 +886,8 @@ int idl_rmsprop_allreduce_step(const uint64_t* h_grad_peers, const uint64_t* h_p
     if (!h_grad_peers || !h_param_peers || !d_square_avg || world < 1 || world > MAX_PEERS || rank < 0 || rank >= world || n_total <= 0 ||
         n_total % (4LL * world) != 0)
         return set_error(IDL_EINVAL, "idl_rmsprop_allreduce_step: bad argument%s (n_total must be a multiple of 4 x world, world <= 16)", "");
+    if (misaligned16(d_square_avg) || (grad_multicast & 15) || (param_multicast & 15))
+        return set_error(IDL_EINVAL, "idl_rmsprop_allreduce_step: misaligned square_avg / multicast address%s", "");
     PeerPtrs g, p;
     for (int r = 0; r < MAX_PEERS; ++r) { g.p[r] = nullptr; p.p[r] = nullptr; }
     for (int r = 0; r < world; ++r) {

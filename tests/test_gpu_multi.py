@@ -1,7 +1,9 @@
 """Two-rank NCCL test of the sharded path (needs >= 2 GPUs; skipped otherwise): scaler
 statistics merged over ranks == single-GPU statistics, sharded mimics identical to the
 unsharded ones (global sequence ids in the RNG), data-parallel training step (eager and CUDA-graphed, flat-gradient
-all-reduce), all-gathered predictions."""
+all-reduce), all-gathered predictions.  Every training step's optimiser update is checked bit for bit: this rank's slice of the new
+parameters and its RMSprop state == idl_rmsprop_step on the rank-order sum of every rank's gradient (symmetric memory: peer loads
+or NVLS multimem; with two ranks the sum has one rounding, so its order cannot matter) or on the NCCL-averaged gradient."""
 import os
 import sys
 
@@ -11,6 +13,31 @@ import pytest
 torch = pytest.importorskip("torch")
 pytestmark = pytest.mark.gpu
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+
+
+def _checked_step(tr, world):
+    """one training step; returns (loss, whether the optimiser's update of this rank's slice equals the reference update)"""
+    import torch.distributed as dist
+    from idelucs_b200 import _lib
+    lib = _lib.load()
+    P0, sq0 = tr._flat_param.clone(), tr._sq.clone()
+    loss = float(tr.step().item())
+    torch.cuda.synchronize()
+    if tr._mode == "symm":   # the kernel reads every rank's gradient and leaves it untouched
+        gs = [torch.empty_like(P0) for _ in range(world)]
+        dist.all_gather(gs, tr._flat_grad.clone())
+        total = torch.zeros_like(P0)
+        for g in gs:
+            total += g
+        lo, hi = tr.rank * tr._shard, (tr.rank + 1) * tr._shard
+        P, g, scale = P0[lo:hi].clone(), total[lo:hi].clone(), float(np.float32(1) / np.float32(world))
+    else:                    # NCCL: the flat gradient was averaged in place
+        lo, hi = 0, P0.numel()
+        P, g, scale = P0.clone(), tr._flat_grad.clone(), 1.0
+    sq = sq0.clone()
+    _lib.check(lib.idl_rmsprop_step(_lib.ptr(P), _lib.ptr(g), _lib.ptr(sq), hi - lo, tr.lr, tr.alpha, tr.eps, tr.weight_decay, scale,
+                                    _lib.stream_ptr()))
+    return loss, torch.equal(tr._flat_param[lo:hi], P) and torch.equal(tr._sq, sq)
 
 
 def _worker(rank, world, port, ret):
@@ -43,8 +70,9 @@ def _worker(rank, world, port, ret):
         ok = ok and bool((prof == pf[:, lo:hi]).float().mean() > 0.99)
     tr = ShardedTrainer(ss, k=k, n_clusters=4, n_mimics=6, batch_sz=64, seed=3, seq_id0=lo, world=world)
     graphed = tr.enable_cuda_graph()                            # step + flat-gradient all-reduce in one CUDA graph
-    losses = [float(tr.step().item()) for _ in range(4)]
-    ok = ok and all(np.isfinite(losses))
+    steps = [_checked_step(tr, world) for _ in range(4)]
+    ok = ok and all(np.isfinite(l) for l, _ in steps)
+    opt_ok = [o for _, o in steps]
     w = next(tr.net.parameters()).detach().clone()
     ws = [torch.empty_like(w) for _ in range(world)]
     dist.all_gather(ws, w)
@@ -52,9 +80,11 @@ def _worker(rank, world, port, ret):
     if rank == 0:
         ret["graph"] = bool(graphed)
         ret["graph_error"] = getattr(tr, "_graph_error", "")
+        ret["path"] = tr._mode + ("/multimem" if tr._mode == "symm" and tr._mc[0] else "/peer loads" if tr._mode == "symm" else "")
     tr._graph = None                                            # the same step eagerly
-    losses = [float(tr.step().item()) for _ in range(3)]
-    ok = ok and all(np.isfinite(losses))
+    steps = [_checked_step(tr, world) for _ in range(3)]
+    ok = ok and all(np.isfinite(l) for l, _ in steps)
+    opt_ok += [o for _, o in steps]
     w = next(tr.net.parameters()).detach().clone()
     dist.all_gather(ws, w)
     ok = ok and all(torch.equal(ws[0], x) for x in ws)
@@ -69,10 +99,19 @@ def _worker(rank, world, port, ret):
             out, lat_full = tr.net(xs)
         tr.net.train()
         ok = ok and torch.allclose(lat_full, lat, rtol=1e-4, atol=1e-4) and bool((out.argmax(1) == preds).float().mean() > 0.99)
-    t = torch.tensor([1.0 if ok else 0.0], device=dev)
+    # the same checks on the NCCL path (all-reduce + idl_rmsprop_step), graphed and eager
+    trn = ShardedTrainer(ss, k=k, n_clusters=4, n_mimics=6, batch_sz=64, seed=3, seq_id0=lo, world=world, use_symmetric_memory=False)
+    graphed_nccl = trn.enable_cuda_graph()
+    opt_nccl = [_checked_step(trn, world)[1] for _ in range(2)]
+    trn._graph = None
+    opt_nccl += [_checked_step(trn, world)[1] for _ in range(2)]
+    t = torch.tensor([1.0 if ok else 0.0, 1.0 if all(opt_ok) else 0.0, 1.0 if all(opt_nccl) and graphed_nccl and trn._mode == "nccl" else 0.0],
+                     device=dev)
     dist.all_reduce(t, op=dist.ReduceOp.MIN)
     if rank == 0:
-        ret["ok"] = bool(t.item() == 1.0)
+        ret["ok"] = bool(t[0].item() == 1.0)
+        ret["optimizer"] = (opt_ok, bool(t[1].item() == 1.0))
+        ret["optimizer_nccl"] = (opt_nccl, bool(t[2].item() == 1.0))
     dist.destroy_process_group()
 
 
@@ -84,5 +123,8 @@ def test_two_gpu_sharding():
     mgr = mp.Manager()
     ret = mgr.dict()
     mp.spawn(_worker, args=(2, 29700 + os.getpid() % 200, ret), nprocs=2, join=True)
+    print("optimiser path:", ret["path"])
     assert ret["ok"]
     assert ret["graph"], ret["graph_error"]
+    assert ret["optimizer"][1], (ret["path"], ret["optimizer"][0])       # per step on rank 0: eager after the four graphed ones
+    assert ret["optimizer_nccl"][1], ret["optimizer_nccl"][0]
