@@ -24,8 +24,8 @@ def _iid_device(z1, z2, lamb, EPS, want_grad=True, want_joint=False, grad_scale=
                 dz1=None, dz2=None):
     """IIC loss of float32 contiguous CUDA [B, C] tensors (may be the two halves of one stacked tensor): (loss, joint, dz1, dz2).
     C <= 16: one launch (idl_iid_loss_scaled: register-resident / single-CTA kernels).  Larger C (the 200 output units of the
-    embedding path): S = z1^T z2, dz1 = z2 dS, dz2 = z1 dS as three small strict-fp32 GEMMs around idl_iid_joint_algebra — 20 us
-    instead of 52 us for the cooperative tiled kernel the C ABI's idl_iid_loss uses on its own."""
+    embedding path): S = z1^T z2, dz1 = z2 dS, dz2 = z1 dS as three small strict-fp32 GEMMs around idl_iid_joint_algebra (the C
+    ABI's idl_iid_loss runs the same algebra between two contraction kernels of its own)."""
     lib = _lib.load()
     B, C = z1.shape
     dev = z1.device

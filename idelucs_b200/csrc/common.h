@@ -11,10 +11,6 @@ int set_error(int code, const char* fmt, const char* a = "", long long b = 0);
 void note_launch();
 // IDL_EINVAL naming `who` unless 0 <= row_begin <= row_end <= n (hdbscan.cu; the row ranges of the all-pairs entry points)
 int check_rows(const char* who, int64_t n, int64_t row_begin, int64_t row_end);
-// IIC loss for C <= 16 in one ordinary CTA (train_ops.cu)
-constexpr int IID_SMALL_MAXC = 16;
-int iid_loss_small_launch(const float* d_z1, const float* d_z2, int B, int C, float lamb, float eps, float* d_loss, float* d_joint, float* d_dz1,
-                          float* d_dz2, void* stream, float gscale, float loss_w, const float* d_add, float add_w);
 }  // namespace idl
 
 #define IDL_CUDA_CHECK(expr)                                                                             \

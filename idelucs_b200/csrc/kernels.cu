@@ -1,5 +1,5 @@
 // idelucs_b200 — sm_100a kernels K1 (pack), K2/K3 (k-mer profile + mimic variants), K4 (scaler)
-// and the C ABI of include/idelucs_b200.h for them.  K5 (IIC loss) lives in iid_loss.cu.
+// and the C ABI of include/idelucs_b200.h for them.  K5 (IIC loss) lives in train_ops.cu.
 //
 // Design (DESIGN.md §4): one CTA owns one sequence at a time.  It builds the CLEAN 4^k
 // histogram once in shared memory (rolling k-mer index from 2-bit packed bases read with

@@ -7,8 +7,9 @@
 //                       weights W = (P + P^T - 2 Y) / (2B T) written over the similarity in place; the normalisation's
 //                       backward.  Four launches of ours + two GEMMs instead of ~25 framework kernels and three mask gathers;
 //                       fixed-order reductions (run-to-run identical)
-//   * iid_loss_small    the IIC loss (LossFunctions.py:20-62) for C <= 16 clusters in ONE ordinary CTA (no cooperative launch,
-//                       no grid barriers): the headline configuration has C = 5, i.e. a 5 x 5 joint
+//   * idl_iid_loss      the IIC loss (LossFunctions.py:20-62) and its gradient: C <= 16 clusters in ONE ordinary CTA (the
+//                       headline configuration has C = 5, i.e. a 5 x 5 joint); above that two contraction kernels around the
+//                       launches of idl_iid_joint_algebra, the C x C algebra the Python layer calls between cuBLAS GEMMs
 //   * idl_rmsprop_step  torch.optim.RMSprop's update (alpha, eps, weight_decay; no momentum, not centred — what
 //                       idelucs/models.py:86 constructs) on a flat parameter shard in one elementwise pass, so that a
 //                       data-parallel step can reduce-scatter the gradient, update 1/N of the parameters per rank and
@@ -628,10 +629,10 @@ static void iid_reg_launch(const float* z1, const float* z2, int B, float lamb, 
 // ---------------------------------------------------------------------------------------------------------------
 // IIC loss from a given S2 = S + S^T, S = z1^T z2 (any C): the C x C algebra of LossFunctions.py:28-44, :59-60 and its derivative.
 // For large C (C = 200 of the embedding path) the contractions around it (S = z1^T z2, dz1 = z2 dS, dz2 = z1 dS) are small dense
-// GEMMs and stay library calls issued by the caller, like InfoNCE's; these kernels replace the cooperative tiled kernel (three
-// grid barriers, 52 us at C = 200) on that path.  Four dependent launches, warp <-> row of the (symmetrised: coalesced row reads
-// only) joint, the few global scalars (T, loss, <A, P>) re-derived by every warp from per-row partials in a fixed order — a single
-// CTA doing the same work takes 65 us (instruction-bound on one SM).
+// GEMMs and stay library calls issued by the caller, like InfoNCE's (idl_iid_loss issues them as the two kernels below).  Four
+// dependent launches, warp <-> row of the (symmetrised: coalesced row reads only) joint, the few global scalars (T, loss, <A, P>)
+// re-derived by every warp from per-row partials in a fixed order — a single CTA doing the same work takes 65 us (instruction-bound
+// on one SM).
 // scratch: 6 C floats = rowsum | marg | gvec | lgm | rowterm | rowap
 // ---------------------------------------------------------------------------------------------------------------
 constexpr int IA_NT = 256, IA_RPB = IA_NT / 32;
@@ -716,8 +717,93 @@ __global__ void __launch_bounds__(IA_NT) iid_alg_grad_kernel(const float* __rest
     }
 }
 
-// C <= 16: called by idl_iid_loss (iid_loss.cu)
-int iid_loss_small_launch(const float* d_z1, const float* d_z2, int B, int C, float lamb, float eps, float* d_loss, float* d_joint, float* d_dz1,
+// ---------------------------------------------------------------------------------------------------------------
+// IIC loss, 16 < C <= 256, through the C ABI: the contractions around the algebra kernels above as two tiled kernels of our own,
+// S2 = S + S^T with S = z1^T z2 before them and dz1 = z2 dS, dz2 = z1 dS after them.  Every thread sums its entries in a fixed
+// order (no float atomics), so the results are run-to-run identical.
+// ---------------------------------------------------------------------------------------------------------------
+constexpr int IC_T = 16;             // tile edge
+constexpr int IC_NT = IC_T * IC_T;   // threads per CTA
+constexpr int IC_BR = 64;            // batch rows staged per step
+constexpr int IID_MAXC = 256;        // idl_iid_loss_max_clusters()
+
+// CTA <-> tile pair (I, J), I <= J, enumerated row by row; thread (ti, tj) sums S_ij and S_ji for i = 16 I + ti, j = 16 J + tj and
+// stores S_ij + S_ji to both (i, j) and (j, i), so S2 is exactly symmetric (a diagonal tile stores from its upper triangle only)
+__global__ void __launch_bounds__(IC_NT) iid_s2_kernel(const float* __restrict__ z1, const float* __restrict__ z2, int B, int C, int nt,
+                                                       float* __restrict__ S2) {
+    __shared__ float sA[4][IC_BR][IC_T];   // z1[:, I] z2[:, J] z1[:, J] z2[:, I]
+    const int tid = threadIdx.x, ti = tid / IC_T, tj = tid % IC_T;
+    int I = 0, rem = blockIdx.x;
+    while (rem >= nt - I) { rem -= nt - I; ++I; }
+    const int J = I + rem;
+    const int I0 = I * IC_T, J0 = J * IC_T;
+    float a0 = 0.f, a1 = 0.f, b0 = 0.f, b1 = 0.f;
+    for (int r0 = 0; r0 < B; r0 += IC_BR) {
+        __syncthreads();
+#pragma unroll
+        for (int q = 0; q < IC_BR * IC_T / IC_NT; ++q) {
+            const int idx = tid + q * IC_NT, row = idx / IC_T, col = idx % IC_T;
+            const int b = r0 + row;
+            const bool ci = b < B && I0 + col < C, cj = b < B && J0 + col < C;
+            sA[0][row][col] = ci ? z1[(size_t)b * C + I0 + col] : 0.f;
+            sA[3][row][col] = ci ? z2[(size_t)b * C + I0 + col] : 0.f;
+            sA[1][row][col] = cj ? z2[(size_t)b * C + J0 + col] : 0.f;
+            sA[2][row][col] = cj ? z1[(size_t)b * C + J0 + col] : 0.f;
+        }
+        __syncthreads();
+#pragma unroll 8
+        for (int r = 0; r < IC_BR; r += 2) {
+            a0 = fmaf(sA[0][r][ti], sA[1][r][tj], a0);
+            b0 = fmaf(sA[2][r][tj], sA[3][r][ti], b0);
+            a1 = fmaf(sA[0][r + 1][ti], sA[1][r + 1][tj], a1);
+            b1 = fmaf(sA[2][r + 1][tj], sA[3][r + 1][ti], b1);
+        }
+    }
+    const int i = I0 + ti, j = J0 + tj;
+    if (i < C && j < C && (I != J || ti <= tj)) {
+        const float s = (a0 + a1) + (b0 + b1);
+        S2[(size_t)i * C + j] = s;
+        S2[(size_t)j * C + i] = s;
+    }
+}
+
+// CTA <-> 64 rows x 16 columns of dz1 = z2 dS (blockIdx.z = 0) or dz2 = z1 dS (blockIdx.z = 1; a NULL output is skipped); thread
+// (ti, tj) sums rows ti, ti + 16, ... of column tj over j in increasing order
+__global__ void __launch_bounds__(IC_NT) iid_dz_kernel(const float* __restrict__ z1, const float* __restrict__ z2, const float* __restrict__ dS, int B,
+                                                       int C, float* __restrict__ dz1, float* __restrict__ dz2) {
+    float* out = blockIdx.z == 0 ? dz1 : dz2;
+    if (!out) return;
+    const float* zo = blockIdx.z == 0 ? z2 : z1;
+    __shared__ float sZ[IC_BR][IC_T];   // zo[r0 .., j0 ..]
+    __shared__ float sD[IC_T][IC_T];    // dS[j0 .., c0 ..]
+    const int tid = threadIdx.x, ti = tid / IC_T, tj = tid % IC_T;
+    const int r0 = blockIdx.x * IC_BR, c0 = blockIdx.y * IC_T;
+    float acc[IC_BR / IC_T] = {};
+    for (int j0 = 0; j0 < C; j0 += IC_T) {
+        __syncthreads();
+#pragma unroll
+        for (int q = 0; q < IC_BR * IC_T / IC_NT; ++q) {
+            const int idx = tid + q * IC_NT, row = idx / IC_T, col = idx % IC_T;
+            sZ[row][col] = (r0 + row < B && j0 + col < C) ? zo[(size_t)(r0 + row) * C + j0 + col] : 0.f;
+        }
+        sD[ti][tj] = (j0 + ti < C && c0 + tj < C) ? dS[(size_t)(j0 + ti) * C + c0 + tj] : 0.f;
+        __syncthreads();
+#pragma unroll
+        for (int jj = 0; jj < IC_T; ++jj) {
+            const float d = sD[jj][tj];
+#pragma unroll
+            for (int q = 0; q < IC_BR / IC_T; ++q) acc[q] = fmaf(sZ[ti + q * IC_T][jj], d, acc[q]);
+        }
+    }
+#pragma unroll
+    for (int q = 0; q < IC_BR / IC_T; ++q) {
+        const int b = r0 + ti + q * IC_T;
+        if (b < B && c0 + tj < C) out[(size_t)b * C + c0 + tj] = acc[q];
+    }
+}
+
+// C <= 16 (idl_iid_loss_scaled)
+static int iid_loss_small_launch(const float* d_z1, const float* d_z2, int B, int C, float lamb, float eps, float* d_loss, float* d_joint, float* d_dz1,
                           float* d_dz2, void* stream, float gscale, float loss_w, const float* d_add, float add_w) {
     cudaStream_t st = (cudaStream_t)stream;
     if (C <= 8) {
@@ -814,6 +900,43 @@ int idl_iid_joint_algebra(const float* d_S2, int C, float lamb, float eps, float
     }
     IDL_CUDA_CHECK(cudaGetLastError());
     return IDL_OK;
+}
+
+int idl_iid_loss_max_clusters(void) { return IID_MAXC; }
+
+size_t idl_iid_loss_workspace_bytes(int C) {
+    if (C < 1 || C > IID_MAXC) return 0;
+    if (C <= IS_MAXC) return sizeof(float) * (3 + 2 * IID_MAXC + C * C) + 64;   // unused by the single-CTA kernels: the size this has always returned
+    return sizeof(float) * (2 * (size_t)C * C + 6 * (size_t)C);                  // S2 | dS | the algebra's scratch
+}
+
+int idl_iid_loss_scaled(const float* d_z1, const float* d_z2, int B, int C, float lamb, float eps, float grad_scale, float loss_weight,
+                        const float* d_add, float add_weight, float* d_loss, float* d_joint, float* d_dz1, float* d_dz2, void* d_workspace,
+                        size_t workspace_bytes, void* stream) {
+    if (!d_z1 || !d_z2 || !d_workspace || B < 1 || C < 1) return set_error(IDL_EINVAL, "idl_iid_loss: bad argument%s", "");
+    if (C > IID_MAXC) return set_error(IDL_EUNSUPPORTED, "idl_iid_loss: n_clusters > 256 not supported%s (got %lld)", "", C);
+    if (workspace_bytes < idl_iid_loss_workspace_bytes(C)) return set_error(IDL_EINVAL, "idl_iid_loss: workspace too small%s", "");
+    if (C <= IS_MAXC)
+        return iid_loss_small_launch(d_z1, d_z2, B, C, lamb, eps, d_loss, d_joint, d_dz1, d_dz2, stream, grad_scale, loss_weight, d_add, add_weight);
+    cudaStream_t st = (cudaStream_t)stream;
+    float* S2 = reinterpret_cast<float*>(d_workspace);
+    float* dS = S2 + (size_t)C * C;
+    float* scratch = dS + (size_t)C * C;
+    const int nt = (C + IC_T - 1) / IC_T;
+    const bool grad = d_dz1 || d_dz2;
+    iid_s2_kernel<<<nt * (nt + 1) / 2, IC_NT, 0, st>>>(d_z1, d_z2, B, C, nt, S2); note_launch();
+    const int rc = idl_iid_joint_algebra(S2, C, lamb, eps, grad_scale, loss_weight, d_add, add_weight, d_loss, d_joint, grad ? dS : nullptr, scratch,
+                                         stream);
+    if (rc != IDL_OK || !grad) return rc;
+    iid_dz_kernel<<<dim3((B + IC_BR - 1) / IC_BR, nt, 2), IC_NT, 0, st>>>(d_z1, d_z2, dS, B, C, d_dz1, d_dz2); note_launch();
+    IDL_CUDA_CHECK(cudaGetLastError());
+    return IDL_OK;
+}
+
+int idl_iid_loss(const float* d_z1, const float* d_z2, int B, int C, float lamb, float eps, float* d_loss, float* d_joint, float* d_dz1, float* d_dz2,
+                 void* d_workspace, size_t workspace_bytes, void* stream) {
+    return idl_iid_loss_scaled(d_z1, d_z2, B, C, lamb, eps, 1.0f, 1.0f, nullptr, 0.0f, d_loss, d_joint, d_dz1, d_dz2, d_workspace, workspace_bytes,
+                               stream);
 }
 
 int idl_relu_dropout_forward(const float* d_parts, int n_parts, const float* d_bias, int64_t M, int N, float p, uint64_t seed, const int64_t* d_step,

@@ -242,8 +242,9 @@ int idl_normalize_counts(const int32_t* d_counts, int64_t n, int R, double* d_ou
  * unclamped — compute_joint's return value); d_dz1, d_dz2 float32 [B, C] = dLoss/dz.
  * C <= idl_iid_loss_max_clusters().  d_workspace: idl_iid_loss_workspace_bytes(C) bytes of
  * scratch (fixed-order partial sums; no float atomics, results are run-to-run identical).
- * C <= 16 (every configuration of Example/ALL_RESULTS.tsv): one ordinary CTA.  C > 16: one cooperative launch, the device
- * must be able to co-schedule ceil(C/16)*(ceil(C/16)+1)/2 CTAs of 256 threads (136 at C = 256; a B200 has 148 SMs). */
+ * C <= 16 (every configuration of Example/ALL_RESULTS.tsv): one ordinary CTA.  C > 16: S2 = S + S^T (S = z1^T z2) into
+ * the workspace, the launches of idl_iid_joint_algebra on it, then dz1 = z2 dS and dz2 = z1 dS (the workspace holds S2, dS and
+ * the algebra's scratch). */
 int idl_iid_loss_max_clusters(void);
 size_t idl_iid_loss_workspace_bytes(int C);
 int idl_iid_loss(const float* d_z1, const float* d_z2, int B, int C, float lamb, float eps, float* d_loss,

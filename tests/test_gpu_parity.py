@@ -551,7 +551,7 @@ def test_weighted_training_loss_and_seeded_gradients():
     """train_losses_and_grads (idl_nce_softmax_xent_scaled + idl_iid_loss_scaled: the weights of idelucs/models.py:128 inside the
     kernels, the combined loss written by the IIC kernel) == (1 - w) info_nce + w IID_loss of the reference formulation in
     float64 and its autograd gradients — register kernel (C <= 8; one and several rows per thread), single-CTA kernel (C <= 16),
-    tiled kernel (C = 200), odd batch sizes (the scalar weights kernel)"""
+    GEMM route (C = 200), odd batch sizes (the scalar weights kernel)"""
     from idelucs_b200.LossFunctions import train_losses_and_grads, train_losses
     torch.manual_seed(11)
     for B, C, w, lamb in ((512, 5, 0.25, 2.8), (96, 3, 0.25, 2.8), (700, 5, 0.4, 2.5), (1300, 8, 0.25, 2.8), (333, 7, 0.1, 1.0), (512, 2, 0.9, 2.8),
@@ -571,9 +571,10 @@ def test_weighted_training_loss_and_seeded_gradients():
         assert l2.item() == loss.item() and torch.equal(az, dz) and torch.equal(ah, dh)
 
 
-def test_iid_tiled_kernel_equals_gemm_route_and_oracle():
+def test_iid_abi_route_equals_gemm_route_and_oracle():
     """C > 16: the Python layer issues the three contractions as GEMMs around idl_iid_joint_algebra; the C ABI's own idl_iid_loss
-    keeps the cooperative tiled kernel.  Both against the oracle's closed form (loss, joint, gradients), incl. the weighting."""
+    issues them as its two contraction kernels around the same algebra.  Both against the oracle's closed form (loss, joint,
+    gradients), incl. the weighting; the C ABI's joint is exactly symmetric and a second call repeats every output bit for bit."""
     import ctypes
     from idelucs_b200 import _lib
     from idelucs_b200.LossFunctions import _iid_device, _ws
@@ -592,7 +593,7 @@ def test_iid_tiled_kernel_equals_gemm_route_and_oracle():
         assert abs(loss.item() - (0.25 * wl + 0.75 * 0.5)) < 1e-5, (B, C)
         np.testing.assert_allclose(joint.cpu().numpy(), wj, rtol=1e-4, atol=1e-9)
         assert np.abs(d1.cpu().numpy() - 0.25 * wd1).max() < 1e-4 * 0.25 * m and np.abs(d2.cpu().numpy() - 0.25 * wd2).max() < 1e-4 * 0.25 * m
-        # the C ABI on its own (tiled kernel)
+        # the C ABI on its own (contraction kernels)
         l2 = torch.empty((), device="cuda"); j2 = torch.empty((C, C), device="cuda"); e1 = torch.empty_like(z1); e2 = torch.empty_like(z2)
         ws = _ws(z1.device, C)
         _lib.check(lib.idl_iid_loss_scaled(_lib.ptr(z1), _lib.ptr(z2), B, C, lamb, sys.float_info.epsilon, 0.25, 0.25, _lib.ptr(add), 0.75, _lib.ptr(l2),
@@ -600,6 +601,11 @@ def test_iid_tiled_kernel_equals_gemm_route_and_oracle():
         assert abs(l2.item() - (0.25 * wl + 0.75 * 0.5)) < 1e-5, (B, C)
         np.testing.assert_allclose(j2.cpu().numpy(), wj, rtol=1e-4, atol=1e-9)
         assert np.abs(e1.cpu().numpy() - 0.25 * wd1).max() < 1e-4 * 0.25 * m and np.abs(e2.cpu().numpy() - 0.25 * wd2).max() < 1e-4 * 0.25 * m
+        assert torch.equal(j2, j2.t()), (B, C)
+        l3 = torch.empty_like(l2); j3 = torch.empty_like(j2); f1 = torch.empty_like(e1); f2 = torch.empty_like(e2)
+        _lib.check(lib.idl_iid_loss_scaled(_lib.ptr(z1), _lib.ptr(z2), B, C, lamb, sys.float_info.epsilon, 0.25, 0.25, _lib.ptr(add), 0.75, _lib.ptr(l3),
+                                           _lib.ptr(j3), _lib.ptr(f1), _lib.ptr(f2), _lib.ptr(ws), ws.numel(), _lib.stream_ptr()))
+        assert torch.equal(l3, l2) and torch.equal(j3, j2) and torch.equal(f1, e1) and torch.equal(f2, e2), (B, C)
 
 
 def test_trainer_forward_backward_equals_plain_module():

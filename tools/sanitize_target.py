@@ -1,6 +1,6 @@
 """Small invocation of every hand-written kernel family, for compute-sanitizer (racecheck / synccheck / memcheck):
 prepare pass + producer/consumer kernel (TMA bulk copies, mbarriers), generic kernel (short + int32 long path), chunked
-long-genome path, IIC loss (single-CTA and cooperative), fused InfoNCE, RMSprop.  Results are compared with the generic
+long-genome path, IIC loss (single-CTA kernels, GEMM route, the C ABI's contraction kernels), fused InfoNCE, RMSprop.  Results are compared with the generic
 kernel so that a sanitizer-clean run is also a correct one."""
 import os
 import sys
@@ -39,7 +39,7 @@ def main():
         assert torch.equal(a, b)
         print("long ok")
     if which in ("all", "loss"):
-        for B, C in ((96, 5), (700, 8), (96, 12), (96, 40)):   # register kernel (one / several rows per thread), single-CTA kernel, tiled kernel
+        for B, C in ((96, 5), (700, 8), (96, 12), (96, 40)):   # register kernel (one / several rows per thread), single-CTA kernel, GEMM route
             z1 = torch.softmax(torch.randn(B, C, device="cuda"), 1).requires_grad_(True)
             z2 = torch.softmax(torch.randn(B, C, device="cuda"), 1).requires_grad_(True)
             IID_loss(z1, z2, lamb=2.8).backward()
@@ -55,7 +55,7 @@ def main():
         lib = _lib.load()
         p, g, v = torch.randn(1000, device="cuda"), torch.randn(1000, device="cuda"), torch.zeros(1000, device="cuda")
         _lib.check(lib.idl_rmsprop_step(_lib.ptr(p), _lib.ptr(g), _lib.ptr(v), 1000, 1e-3, 0.99, 1e-8, 0.01, 1.0, _lib.stream_ptr()))
-        # the C ABI's own tiled kernel (the Python layer takes the GEMM route above 16 clusters)
+        # the C ABI's own contraction kernels around the algebra kernels (the Python layer takes the GEMM route above 16 clusters)
         from idelucs_b200.LossFunctions import _ws
         z1 = torch.softmax(torch.randn(96, 40, device="cuda"), 1); z2 = torch.softmax(torch.randn(96, 40, device="cuda"), 1)
         lo = torch.empty((), device="cuda"); d1 = torch.empty_like(z1); d2 = torch.empty_like(z2); ws = _ws(z1.device, 40)
