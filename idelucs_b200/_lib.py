@@ -72,6 +72,13 @@ PROTOTYPES = {
     "idl_pair_selection": (c_int, [c_void_p, c_int, c_i64, c_void_p, c_void_p, c_void_p]),
     "idl_rmsprop_step": (c_int, [c_void_p, c_void_p, c_void_p, c_i64, c_float, c_float, c_float, c_float, c_float, c_void_p]),
     "idl_rmsprop_allreduce_step": (c_int, [c_void_p, c_void_p, c_u64, c_u64, c_void_p, c_i64, c_int, c_int, c_float, c_float, c_float, c_float, c_void_p]),
+    "idl_sgd_step": (c_int, [c_void_p, c_void_p, c_void_p, c_i64, c_float, c_float, c_float, c_void_p, c_float, c_void_p]),
+    "idl_adam_step": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_i64, c_float, c_double, c_double, c_float, c_float, c_void_p, c_float,
+                              c_void_p]),
+    "idl_sgd_allreduce_step": (c_int, [c_void_p, c_void_p, c_u64, c_u64, c_void_p, c_i64, c_int, c_int, c_float, c_float, c_float, c_void_p,
+                                       c_void_p]),
+    "idl_adam_allreduce_step": (c_int, [c_void_p, c_void_p, c_u64, c_u64, c_void_p, c_void_p, c_i64, c_int, c_int, c_float, c_double, c_double,
+                                        c_float, c_float, c_void_p, c_void_p]),
     "idl_fasta_scan": (c_int, [c_void_p, c_i64, ctypes.POINTER(c_i64), ctypes.POINTER(c_i64)]),
     "idl_fasta_extract": (c_int, [c_void_p, c_i64, c_i64, c_void_p, c_i64, c_void_p, c_void_p, c_void_p]),
     "idl_iid_loss_max_clusters": (c_int, []),

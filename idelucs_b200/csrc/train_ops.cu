@@ -14,9 +14,12 @@
 //                       idelucs/models.py:86 constructs) on a flat parameter shard in one elementwise pass, so that a
 //                       data-parallel step can reduce-scatter the gradient, update 1/N of the parameters per rank and
 //                       all-gather them
+//   * idl_sgd_step / idl_adam_step  the other two optimisers of idelucs/models.py:86-99 (SGD with momentum, Adam), the step
+//                       number read from device memory; the *_allreduce_step variants of all three share one NVLink kernel body
 #include <cuda_runtime.h>
 #include <math.h>
 #include <stdint.h>
+#include <stdio.h>
 
 #include "common.h"
 #include "core.cuh"
@@ -397,11 +400,87 @@ __global__ void rmsprop_kernel(float* __restrict__ p, const float* __restrict__ 
 }
 
 // ---------------------------------------------------------------------------------------------------------------
-// Data-parallel optimiser step as ONE kernel over NVLink peer memory: gradient all-reduce (mean) + RMSprop + parameter
+// The other two optimisers of idelucs/models.py:86-99 as per-element updates, shared by the single-rank kernel below and the
+// all-reduce kernel: update(g, p, s) takes the (scaled) gradient, the parameter and the optimiser state s[kStates] of one element
+// and returns the new parameter.  load() runs once per thread before the first element: the step number t (1-based) is read
+// from device memory, so a replayed CUDA graph keeps counting without a host argument.
+//   SGD  (torch.optim.SGD(lr, momentum, weight_decay), dampening 0, no Nesterov): d = g + wd p; buf = d at t = 1, else
+//        momentum buf + d; p -= lr buf
+//   Adam (torch.optim.Adam(lr, betas, eps, weight_decay), no amsgrad): g += wd p; m = m + (1 - b1)(g - m);
+//        v = b2 v + (1 - b2) g^2; p -= (lr / (1 - b1^t)) m / (sqrt(v) / sqrt(1 - b2^t) + eps)
+// ---------------------------------------------------------------------------------------------------------------
+struct RmspropUpdate {
+    static constexpr int kStates = 1;
+    float lr, alpha, eps, wd;
+    __device__ __forceinline__ void load() {}
+    __device__ __forceinline__ float update(float g, float p, float (&s)[1]) const {
+        const float gg = fmaf(wd, p, g);
+        const float vv = fmaf(1.0f - alpha, gg * gg, alpha * s[0]);
+        s[0] = vv;
+        return p - lr * (gg / (sqrtf(vv) + eps));
+    }
+};
+
+struct SgdUpdate {
+    static constexpr int kStates = 1;
+    float lr, momentum, wd;
+    const long long* step;
+    bool first;
+    __device__ __forceinline__ void load() { first = *step <= 1; }
+    __device__ __forceinline__ float update(float g, float p, float (&s)[1]) const {
+        const float d = fmaf(wd, p, g);
+        const float b = first ? d : __fadd_rn(__fmul_rn(momentum, s[0]), d);   // (torch's mul_ then add_: two roundings)
+        s[0] = b;
+        return p - lr * b;
+    }
+};
+
+struct AdamUpdate {   // (the betas in double, as torch holds them: 1 - 0.999f is 1.3e-5 away from 1 - 0.999)
+    static constexpr int kStates = 2;
+    float lr, eps, wd;
+    double beta1, beta2;
+    const long long* step;
+    float c1, b2, c2, step_size, bc2_sqrt;
+    __device__ __forceinline__ void load() {   // the bias corrections in double, as torch computes them on the host
+        const double t = (double)*step;
+        c1 = (float)(1.0 - beta1);
+        b2 = (float)beta2;
+        c2 = (float)(1.0 - beta2);
+        step_size = (float)((double)lr / (1.0 - pow(beta1, t)));
+        bc2_sqrt = (float)sqrt(1.0 - pow(beta2, t));
+    }
+    __device__ __forceinline__ float update(float g, float p, float (&s)[2]) const {
+        const float gg = fmaf(wd, p, g);
+        const float m = s[0] + c1 * (gg - s[0]);
+        const float v = fmaf(c2 * gg, gg, __fmul_rn(s[1], b2));   // (torch's mul_(beta2) then addcmul_)
+        s[0] = m; s[1] = v;
+        return p - step_size * (m / (sqrtf(v) / bc2_sqrt + eps));
+    }
+};
+
+constexpr int MAX_STATES = 2;
+struct StatePtrs { float* s[MAX_STATES]; };
+
+// single rank: one elementwise pass over a flat buffer (any alignment)
+template <class Op>
+__global__ void opt_step_kernel(float* __restrict__ p, const float* __restrict__ g, StatePtrs st, long long n, float gscale, Op op) {
+    op.load();
+    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) {
+        float s[Op::kStates];
+#pragma unroll
+        for (int k = 0; k < Op::kStates; ++k) s[k] = st.s[k][i];
+        p[i] = op.update(g[i] * gscale, p[i], s);
+#pragma unroll
+        for (int k = 0; k < Op::kStates; ++k) st.s[k][i] = s[k];
+    }
+}
+
+// ---------------------------------------------------------------------------------------------------------------
+// Data-parallel optimiser step as ONE kernel over NVLink peer memory: gradient all-reduce (mean) + the update of Op + parameter
 // broadcast.  Gradients and parameters live in symmetric buffers (the same allocation mapped by every rank).  Rank r owns the
 // slice [r * shard, (r + 1) * shard): it reads the SUM of every rank's gradient slice — one multimem.ld_reduce per 16 bytes when
 // the buffers have an NVLS multicast mapping (the NVSwitch adds the eight operands), else one load per peer in rank order —
-// applies the RMSprop update to its slice of the parameters and stores the new values into EVERY rank's parameter buffer
+// applies the update to its slice of the parameters and stores the new values into EVERY rank's parameter buffer
 // (multimem.st, or one store per peer).  Per GPU that is 1/N of the gradient bytes in and 1/N of the parameter bytes out,
 // no staging buffers, no separate optimiser pass, and every replica receives bit-identical parameters (one writer per slice).
 // The caller brackets the launch with cross-rank barriers (gradients complete before, parameters visible after).
@@ -424,14 +503,15 @@ __device__ __forceinline__ void multimem_st(float* mc_addr, float4 v) {
 // are 1 MB per rank at 8 GPUs — so the loads of a thread must overlap each other.
 constexpr int AR_U = 4;
 
-__global__ void __launch_bounds__(256) rmsprop_allreduce_kernel(const PeerPtrs grads, const PeerPtrs params, const float* grad_mc, float* param_mc,
-                                                                  float* __restrict__ sq, long long shard, int rank, int world, float lr, float alpha,
-                                                                  float eps, float wd) {
+template <class Op>
+__global__ void __launch_bounds__(256) allreduce_step_kernel(const PeerPtrs grads, const PeerPtrs params, const float* grad_mc, float* param_mc,
+                                                               const StatePtrs st, long long shard, int rank, int world, Op op) {
+    op.load();
     const long long base = (long long)rank * shard;
     const float inv_world = 1.0f / (float)world;
     const long long units = shard / 4, stride = (long long)gridDim.x * blockDim.x;
     for (long long i0 = (long long)blockIdx.x * blockDim.x + threadIdx.x; i0 < units; i0 += stride * AR_U) {
-        float4 g[AR_U], p[AR_U], v[AR_U];
+        float4 g[AR_U], p[AR_U], v[Op::kStates][AR_U];
 #pragma unroll
         for (int u = 0; u < AR_U; ++u) {
             const long long i4 = i0 + u * stride;
@@ -447,7 +527,8 @@ __global__ void __launch_bounds__(256) rmsprop_allreduce_kernel(const PeerPtrs g
                     }
                 }
                 p[u] = *reinterpret_cast<const float4*>(params.p[rank] + idx);
-                v[u] = reinterpret_cast<const float4*>(sq)[i4];
+#pragma unroll
+                for (int k = 0; k < Op::kStates; ++k) v[k][u] = reinterpret_cast<const float4*>(st.s[k])[i4];
             }
         }
 #pragma unroll
@@ -455,15 +536,18 @@ __global__ void __launch_bounds__(256) rmsprop_allreduce_kernel(const PeerPtrs g
             const long long i4 = i0 + u * stride;
             if (i4 < units) {
                 const long long idx = base + i4 * 4;
-                float* gp = &g[u].x; float* pp = &p[u].x; float* vp = &v[u].x;
+                float* gp = &g[u].x; float* pp = &p[u].x;
 #pragma unroll
                 for (int e = 0; e < 4; ++e) {
-                    const float gg = fmaf(wd, pp[e], gp[e] * inv_world);
-                    const float vv = fmaf(1.0f - alpha, gg * gg, alpha * vp[e]);
-                    vp[e] = vv;
-                    pp[e] = pp[e] - lr * (gg / (sqrtf(vv) + eps));
+                    float s[Op::kStates];
+#pragma unroll
+                    for (int k = 0; k < Op::kStates; ++k) s[k] = (&v[k][u].x)[e];
+                    pp[e] = op.update(gp[e] * inv_world, pp[e], s);
+#pragma unroll
+                    for (int k = 0; k < Op::kStates; ++k) (&v[k][u].x)[e] = s[k];
                 }
-                reinterpret_cast<float4*>(sq)[i4] = v[u];
+#pragma unroll
+                for (int k = 0; k < Op::kStates; ++k) reinterpret_cast<float4*>(st.s[k])[i4] = v[k][u];
                 if (param_mc) {
                     multimem_st(param_mc + idx, p[u]);
                 } else {
@@ -846,6 +930,54 @@ using namespace idl;
 // the float4 kernels below need 16-byte aligned buffers (a torch view at an odd storage offset is not): rejected, not faulted on
 static bool misaligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) != 0; }
 
+// single-rank SGD / Adam: one thread per element, up to 8 CTAs per SM
+template <class Op>
+static int opt_step_launch(float* d_param, const float* d_grad, StatePtrs st, int64_t n, float grad_scale, Op op, void* stream) {
+    if (n == 0) return IDL_OK;
+    long long grid = (n + 255) / 256;
+    if (grid > 148 * 8) grid = 148 * 8;
+    opt_step_kernel<Op><<<(unsigned)grid, 256, 0, (cudaStream_t)stream>>>(d_param, d_grad, st, n, grad_scale, op); note_launch();
+    IDL_CUDA_CHECK(cudaGetLastError());
+    return IDL_OK;
+}
+
+// the argument checks and the launch of the three *_allreduce_step entry points; `who` names the entry point in the error text,
+// `state` its state buffers
+template <class Op>
+static int allreduce_step_launch(const char* who, const char* state, const uint64_t* h_grad_peers, const uint64_t* h_param_peers,
+                                 uint64_t grad_multicast, uint64_t param_multicast, StatePtrs st, int64_t n_total, int rank, int world, Op op,
+                                 void* stream) {
+    bool null_state = false, odd_state = false;
+    for (int k = 0; k < Op::kStates; ++k) { null_state |= !st.s[k]; odd_state |= misaligned16(st.s[k]); }
+    if (!h_grad_peers || !h_param_peers || null_state || world < 1 || world > MAX_PEERS || rank < 0 || rank >= world || n_total <= 0 ||
+        n_total % (4LL * world) != 0)
+        return set_error(IDL_EINVAL, "%s: bad argument (n_total must be a multiple of 4 x world, world <= 16)", who);
+    if (odd_state || (grad_multicast & 15) || (param_multicast & 15)) {
+        char msg[128];
+        snprintf(msg, sizeof msg, "%s: misaligned %s / multicast address", who, state);
+        return set_error(IDL_EINVAL, "%s", msg);
+    }
+    PeerPtrs g, p;
+    for (int r = 0; r < MAX_PEERS; ++r) { g.p[r] = nullptr; p.p[r] = nullptr; }
+    for (int r = 0; r < world; ++r) {
+        g.p[r] = reinterpret_cast<float*>((uintptr_t)h_grad_peers[r]);
+        p.p[r] = reinterpret_cast<float*>((uintptr_t)h_param_peers[r]);
+        if (!g.p[r] || !p.p[r] || (h_grad_peers[r] & 15) || (h_param_peers[r] & 15)) return set_error(IDL_EINVAL, "%s: null / misaligned peer pointer", who);
+    }
+    const long long shard = n_total / world;
+    long long grid = (shard / 4 + 256 * AR_U - 1) / (256 * AR_U);
+    if (grid > 148) grid = 148;   // measured on 2 and 8 B200s (tools/symm_probe.py): more CTAs do not move the NVLS-bound kernel
+    if (grid < 1) grid = 1;
+    allreduce_step_kernel<Op><<<(unsigned)grid, 256, 0, (cudaStream_t)stream>>>(g, p, reinterpret_cast<const float*>((uintptr_t)grad_multicast),
+                                                                                 reinterpret_cast<float*>((uintptr_t)param_multicast), st, shard, rank,
+                                                                                 world, op); note_launch();
+    IDL_CUDA_CHECK(cudaGetLastError());
+    return IDL_OK;
+}
+
+// the step counter the SGD / Adam kernels read: an int64 in device memory, so 8-byte aligned
+static bool bad_step(const int64_t* d_step) { return !d_step || (reinterpret_cast<uintptr_t>(d_step) & 7) != 0; }
+
 extern "C" {
 
 int idl_nce_normalize(const float* d_h, int n2, int D, float* d_fn, float* d_inv_norm, void* stream) {
@@ -1006,27 +1138,42 @@ int idl_rmsprop_step(float* d_param, const float* d_grad, float* d_square_avg, i
 int idl_rmsprop_allreduce_step(const uint64_t* h_grad_peers, const uint64_t* h_param_peers, uint64_t grad_multicast, uint64_t param_multicast,
                                float* d_square_avg, int64_t n_total, int rank, int world, float lr, float alpha, float eps, float weight_decay,
                                void* stream) {
-    if (!h_grad_peers || !h_param_peers || !d_square_avg || world < 1 || world > MAX_PEERS || rank < 0 || rank >= world || n_total <= 0 ||
-        n_total % (4LL * world) != 0)
-        return set_error(IDL_EINVAL, "idl_rmsprop_allreduce_step: bad argument%s (n_total must be a multiple of 4 x world, world <= 16)", "");
-    if (misaligned16(d_square_avg) || (grad_multicast & 15) || (param_multicast & 15))
-        return set_error(IDL_EINVAL, "idl_rmsprop_allreduce_step: misaligned square_avg / multicast address%s", "");
-    PeerPtrs g, p;
-    for (int r = 0; r < MAX_PEERS; ++r) { g.p[r] = nullptr; p.p[r] = nullptr; }
-    for (int r = 0; r < world; ++r) {
-        g.p[r] = reinterpret_cast<float*>((uintptr_t)h_grad_peers[r]);
-        p.p[r] = reinterpret_cast<float*>((uintptr_t)h_param_peers[r]);
-        if (!g.p[r] || !p.p[r] || (h_grad_peers[r] & 15) || (h_param_peers[r] & 15)) return set_error(IDL_EINVAL, "idl_rmsprop_allreduce_step: null / misaligned peer pointer%s", "");
-    }
-    const long long shard = n_total / world;
-    long long grid = (shard / 4 + 256 * AR_U - 1) / (256 * AR_U);
-    if (grid > 148) grid = 148;   // measured on 2 and 8 B200s (tools/symm_probe.py): more CTAs do not move the NVLS-bound kernel
-    if (grid < 1) grid = 1;
-    rmsprop_allreduce_kernel<<<(unsigned)grid, 256, 0, (cudaStream_t)stream>>>(g, p, reinterpret_cast<const float*>((uintptr_t)grad_multicast),
-                                                                               reinterpret_cast<float*>((uintptr_t)param_multicast), d_square_avg, shard,
-                                                                               rank, world, lr, alpha, eps, weight_decay); note_launch();
-    IDL_CUDA_CHECK(cudaGetLastError());
-    return IDL_OK;
+    return allreduce_step_launch("idl_rmsprop_allreduce_step", "square_avg", h_grad_peers, h_param_peers, grad_multicast, param_multicast,
+                                 StatePtrs{{d_square_avg, nullptr}}, n_total, rank, world, RmspropUpdate{lr, alpha, eps, weight_decay}, stream);
+}
+
+int idl_sgd_step(float* d_param, const float* d_grad, float* d_momentum_buf, int64_t n, float lr, float momentum, float weight_decay,
+                 const int64_t* d_step, float grad_scale, void* stream) {
+    if (!d_param || !d_grad || !d_momentum_buf || n < 0) return set_error(IDL_EINVAL, "idl_sgd_step: bad argument%s", "");
+    if (bad_step(d_step)) return set_error(IDL_EINVAL, "idl_sgd_step: null / misaligned step counter%s (int64 in device memory)", "");
+    return opt_step_launch(d_param, d_grad, StatePtrs{{d_momentum_buf, nullptr}}, n, grad_scale,
+                           SgdUpdate{lr, momentum, weight_decay, reinterpret_cast<const long long*>(d_step), false}, stream);
+}
+
+int idl_adam_step(float* d_param, const float* d_grad, float* d_exp_avg, float* d_exp_avg_sq, int64_t n, float lr, double beta1, double beta2,
+                  float eps, float weight_decay, const int64_t* d_step, float grad_scale, void* stream) {
+    if (!d_param || !d_grad || !d_exp_avg || !d_exp_avg_sq || n < 0) return set_error(IDL_EINVAL, "idl_adam_step: bad argument%s", "");
+    if (bad_step(d_step)) return set_error(IDL_EINVAL, "idl_adam_step: null / misaligned step counter%s (int64 in device memory)", "");
+    return opt_step_launch(d_param, d_grad, StatePtrs{{d_exp_avg, d_exp_avg_sq}}, n, grad_scale,
+                           AdamUpdate{lr, eps, weight_decay, beta1, beta2, reinterpret_cast<const long long*>(d_step), 0.f, 0.f, 0.f, 0.f, 0.f}, stream);
+}
+
+int idl_sgd_allreduce_step(const uint64_t* h_grad_peers, const uint64_t* h_param_peers, uint64_t grad_multicast, uint64_t param_multicast,
+                           float* d_momentum_buf, int64_t n_total, int rank, int world, float lr, float momentum, float weight_decay,
+                           const int64_t* d_step, void* stream) {
+    if (bad_step(d_step)) return set_error(IDL_EINVAL, "idl_sgd_allreduce_step: null / misaligned step counter%s (int64 in device memory)", "");
+    return allreduce_step_launch("idl_sgd_allreduce_step", "momentum_buffer", h_grad_peers, h_param_peers, grad_multicast, param_multicast,
+                                 StatePtrs{{d_momentum_buf, nullptr}}, n_total, rank, world,
+                                 SgdUpdate{lr, momentum, weight_decay, reinterpret_cast<const long long*>(d_step), false}, stream);
+}
+
+int idl_adam_allreduce_step(const uint64_t* h_grad_peers, const uint64_t* h_param_peers, uint64_t grad_multicast, uint64_t param_multicast,
+                            float* d_exp_avg, float* d_exp_avg_sq, int64_t n_total, int rank, int world, float lr, double beta1, double beta2, float eps,
+                            float weight_decay, const int64_t* d_step, void* stream) {
+    if (bad_step(d_step)) return set_error(IDL_EINVAL, "idl_adam_allreduce_step: null / misaligned step counter%s (int64 in device memory)", "");
+    return allreduce_step_launch("idl_adam_allreduce_step", "exp_avg / exp_avg_sq", h_grad_peers, h_param_peers, grad_multicast, param_multicast,
+                                 StatePtrs{{d_exp_avg, d_exp_avg_sq}}, n_total, rank, world,
+                                 AdamUpdate{lr, eps, weight_decay, beta1, beta2, reinterpret_cast<const long long*>(d_step), 0.f, 0.f, 0.f, 0.f, 0.f}, stream);
 }
 
 }  // extern "C"

@@ -180,11 +180,14 @@ class SeqSet(object):
         return self
 
     @classmethod
-    def from_fasta(cls, fname, device=None):
+    def from_fasta(cls, fname, device=None, rows=None):
         """Parse once with the native scanner, one H2D copy of the flat pinned bytes, pack on the device.  Records
         whose sequence lines hold interior whitespace (deleted by check_sequence, utils.py:45) take the host
-        compaction path of from_sequences."""
+        compaction path of from_sequences.  rows = (lo, hi): pack only records lo .. hi-1 (one rank's shard)."""
         names, flat, byte_off = read_fasta_native(fname)
+        if rows is not None:
+            lo, hi = rows
+            flat, byte_off, names = flat[int(byte_off[lo]):int(byte_off[hi])], byte_off[lo:hi + 1] - byte_off[lo], names[lo:hi]
         header_error = None
         for i, h in enumerate(names):
             try:

@@ -3,7 +3,7 @@ k=6, n_mimics=50, batch_sz=512, sharded over 1/2/4/8 B200).
 
 Each rank owns a contiguous shard of the packed sequences, regenerates its pair batches on the fly with the mimic kernel (selection
 mode — the 1.6 TB x_train of the reference never exists) and runs the reference's training step (idelucs/models.py:113-143: two
-forwards, (1-w) InfoNCE + w IIC loss, backward, RMSprop) as ONE CUDA graph on two streams:
+forwards, (1-w) InfoNCE + w IIC loss, backward, RMSprop or the SGD / Adam of `optimizer=`) as ONE CUDA graph on two streams:
 
   * every dense contraction of the encoder stays a PyTorch / cuBLAS GEMM in strict fp32, issued in the shape that fills the GPU for
     this batch (_FirstLinear / _FlatLinear: inner-dimension splits as batched GEMMs, gradients written straight into a flat buffer);
@@ -21,6 +21,10 @@ from . import featurise as ft
 from .LossFunctions import train_losses_and_grads
 from .PytorchUtils import NetLinear
 from .models import weights_init
+
+OPTIMIZERS = {"RMSprop": 1, "SGD": 1, "Adam": 2}   # the optimisers of idelucs/models.py:86-99 -> state buffers per parameter
+SGD_MOMENTUM = 0.9
+ADAM_BETAS = (0.9, 0.999)
 
 
 def _relu_dropout_fwd(parts, n_parts, bias, M, N, drop):
@@ -172,9 +176,13 @@ class ShardedTrainer(object):
     The parameters of the network are views into one flat buffer, so the optimiser and the collectives see one tensor."""
 
     def __init__(self, seqset, k=6, n_clusters=5, n_mimics=50, batch_sz=512, lamb=2.8, weight=0.25, lr=1e-3, seed=0,
-                 seq_id0=0, world=1, materialize_bytes=0, alpha=0.99, eps=1e-8, weight_decay=0.01, use_symmetric_memory=True,
-                 overlap_featurise_with="forward"):
+                 seq_id0=0, world=1, materialize_bytes=0, alpha=0.99, eps=1e-8, weight_decay=None, use_symmetric_memory=True,
+                 overlap_featurise_with="forward", optimizer="RMSprop"):
         from .utils import PairBatchLoader
+        if optimizer not in OPTIMIZERS:
+            raise ValueError("optimizer must be one of %s, got %r" % (", ".join(OPTIMIZERS), optimizer))
+        if weight_decay is None:   # idelucs/models.py:86-99: RMSprop and SGD with weight_decay=0.01, Adam without
+            weight_decay = 0.0 if optimizer == "Adam" else 0.01
         self.dev = seqset.device
         self.world = world
         self.rank = dist.get_rank() if world > 1 else 0
@@ -222,7 +230,11 @@ class ShardedTrainer(object):
         if world > 1:   # replicas must start identical whatever the RNG state of the rank was
             dist.broadcast(self._flat_param, src=0)
         self._shard = (n + pad) // world if self._mode == "symm" else n + pad
-        self._sq = torch.zeros(self._shard, dtype=torch.float32, device=self.dev)
+        # optimiser state of this rank's slice: RMSprop's square average (_sq), SGD's momentum buffer, Adam's two moments
+        self.optimizer = optimizer
+        self._state = [torch.zeros(self._shard, dtype=torch.float32, device=self.dev) for _ in range(OPTIMIZERS[optimizer])]
+        self._sq = self._state[0] if optimizer == "RMSprop" else None
+        self._loss_sum = torch.zeros((), dtype=torch.float32, device=self.dev)   # sum of the step losses since epoch_loss()
         self.lr, self.alpha, self.eps, self.weight_decay = lr, alpha, eps, weight_decay
         self.overlap_featurise_with = overlap_featurise_with
         self.lamb, self.weight, self.batch_sz = lamb, weight, batch_sz
@@ -248,24 +260,68 @@ class ShardedTrainer(object):
         mc_p = int(getattr(self._hp, "multicast_ptr", 0) or 0)
         self._mc = (mc_g, mc_p) if (mc_g and mc_p) else (0, 0)
 
-    # ---- optimiser: torch.optim.RMSprop's arithmetic on flat buffers ----
+    # ---- optimiser: torch.optim.RMSprop's / SGD's / Adam's arithmetic on flat buffers ----
     def _optimizer_step(self):
         from . import _lib
         lib = _lib.load()
+        st = [_lib.ptr(t) for t in self._state]
+        step = _lib.ptr(self._step_no)   # (SGD's first step and Adam's bias corrections: the counter the step incremented)
         with torch.cuda.device(self.dev):
             if self._mode == "symm":
-                # ONE kernel: mean of every rank's gradient slice (NVLS multimem.ld_reduce, or peer loads) -> RMSprop on this rank's
+                # ONE kernel: mean of every rank's gradient slice (NVLS multimem.ld_reduce, or peer loads) -> the update of this rank's
                 # slice -> new parameters stored into every rank's buffer; symmetric-memory barriers (5 us each) on both sides
+                peers = (self._gp, self._pp, self._mc[0], self._mc[1])
+                n, r, w = self._flat_grad.numel(), self.rank, self.world
                 self._hg.barrier(channel=0)
-                _lib.check(lib.idl_rmsprop_allreduce_step(self._gp, self._pp, self._mc[0], self._mc[1], _lib.ptr(self._sq),
-                                                          self._flat_grad.numel(), self.rank, self.world, self.lr, self.alpha, self.eps,
-                                                          self.weight_decay, _lib.stream_ptr()))
+                if self.optimizer == "RMSprop":
+                    rc = lib.idl_rmsprop_allreduce_step(*peers, *st, n, r, w, self.lr, self.alpha, self.eps, self.weight_decay, _lib.stream_ptr())
+                elif self.optimizer == "SGD":
+                    rc = lib.idl_sgd_allreduce_step(*peers, *st, n, r, w, self.lr, SGD_MOMENTUM, self.weight_decay, step, _lib.stream_ptr())
+                else:
+                    rc = lib.idl_adam_allreduce_step(*peers, *st, n, r, w, self.lr, *ADAM_BETAS, self.eps, self.weight_decay, step,
+                                                     _lib.stream_ptr())
+                _lib.check(rc)
                 self._hp.barrier(channel=0)
                 return
             if self._mode == "nccl":
                 dist.all_reduce(self._flat_grad, op=dist.ReduceOp.AVG)
-            _lib.check(lib.idl_rmsprop_step(_lib.ptr(self._flat_param), _lib.ptr(self._flat_grad), _lib.ptr(self._sq), self._shard, self.lr,
-                                            self.alpha, self.eps, self.weight_decay, 1.0, _lib.stream_ptr()))
+            p, g = _lib.ptr(self._flat_param), _lib.ptr(self._flat_grad)
+            if self.optimizer == "RMSprop":
+                rc = lib.idl_rmsprop_step(p, g, *st, self._shard, self.lr, self.alpha, self.eps, self.weight_decay, 1.0, _lib.stream_ptr())
+            elif self.optimizer == "SGD":
+                rc = lib.idl_sgd_step(p, g, *st, self._shard, self.lr, SGD_MOMENTUM, self.weight_decay, step, 1.0, _lib.stream_ptr())
+            else:
+                rc = lib.idl_adam_step(p, g, *st, self._shard, self.lr, *ADAM_BETAS, self.eps, self.weight_decay, step, 1.0, _lib.stream_ptr())
+            _lib.check(rc)
+
+    def reinit(self, seed):
+        """A fresh voter (idelucs/__main__.py:106-109): new Kaiming-normal weights and zero biases (models.weights_init, drawn on
+        rank 0 from `seed` and broadcast).  The optimiser state and the step counter are kept, as the reference keeps its
+        optimiser between voters; every buffer stays in place, so a captured CUDA graph stays valid."""
+        if self.rank == 0:
+            with torch.random.fork_rng(devices=[self.dev]):
+                torch.manual_seed(seed)
+                self.net.apply(weights_init)   # (in place: the parameters are views into the flat buffer)
+        if self.world > 1:
+            dist.broadcast(self._flat_param, src=0)
+
+    def reset_optimizer(self):
+        """zero the optimiser state and the step counter: the state of a fresh torch optimiser (after the warm-up steps of
+        enable_cuda_graph, before the first voter)"""
+        for t in self._state:
+            t.zero_()
+        self._step_no.zero_()
+        self._loss_sum.zero_()
+
+    def epoch_loss(self, n_steps):
+        """the mean loss of the n_steps steps since the last call, as contrastive_training_epoch divides it (idelucs/models.py:
+        137-143: the sum over the epoch over the index of its last batch, n_steps - 1), averaged over the ranks; read once per
+        epoch (one synchronisation), then the accumulator restarts"""
+        s = self._loss_sum.clone()
+        self._loss_sum.zero_()
+        if self.world > 1:
+            dist.all_reduce(s, op=dist.ReduceOp.AVG)
+        return float((s / float(n_steps - 1)).item()) if n_steps > 1 else float((s / torch.zeros_like(s)).item())
 
     def enable_cuda_graph(self, warmup=11):
         """Capture the whole step (both streams) in ONE CUDA graph: the step is launch-bound, so replaying a graph removes the
@@ -379,6 +435,9 @@ class ShardedTrainer(object):
         # (1 - w) InfoNCE + w IIC (models.py:128) and its gradients with respect to z and h straight from the fused kernels (the
         # weights ride inside them); the MLP's backward pass is seeded with those — no framework kernel between forward and backward
         loss, dz, dh = train_losses_and_grads(z, h, self.lamb, self.weight, 0.85)
+        self._side.wait_stream(main)          # (the epoch's loss sum: a one-element add beside the backward pass, off the main stream)
+        with torch.cuda.stream(self._side):
+            self._loss_sum.add_(loss)
         torch.autograd.backward((z, h), (dz, dh))
         if late:
             self._side.wait_stream(main)

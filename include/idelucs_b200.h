@@ -324,6 +324,29 @@ int idl_rmsprop_allreduce_step(const uint64_t* h_grad_peers, const uint64_t* h_p
                                float* d_square_avg, int64_t n_total, int rank, int world, float lr, float alpha, float eps, float weight_decay,
                                void* stream);
 
+/* The other two optimisers of idelucs/models.py:86-99 on a flat float32 shard, one elementwise pass each.  d_step points to the
+ * 1-based number of the step being taken (int64 in device memory, 8-byte aligned): it is read by the kernel, so a replayed CUDA
+ * graph keeps counting with the counter incremented on the device before the call.  g = grad * grad_scale + weight_decay * p.
+ *   idl_sgd_step   torch.optim.SGD(lr, momentum, weight_decay), dampening 0, no Nesterov: buf = g at step 1, else
+ *                  buf = momentum buf + g; p -= lr buf  (d_momentum_buf: n floats)
+ *   idl_adam_step  torch.optim.Adam(lr, (beta1, beta2), eps, weight_decay), no amsgrad: m = m + (1 - beta1)(g - m);
+ *                  v = beta2 v + (1 - beta2) g^2; p -= lr / (1 - beta1^t) m / (sqrt(v) / sqrt(1 - beta2^t) + eps), the bias
+ *                  corrections in double; the betas are doubles, as torch holds them (1 - beta2 rounded from a float 0.999 is
+ *                  1.3e-5 off)  (d_exp_avg, d_exp_avg_sq: n floats each) */
+int idl_sgd_step(float* d_param, const float* d_grad, float* d_momentum_buf, int64_t n, float lr, float momentum, float weight_decay,
+                 const int64_t* d_step, float grad_scale, void* stream);
+int idl_adam_step(float* d_param, const float* d_grad, float* d_exp_avg, float* d_exp_avg_sq, int64_t n, float lr, double beta1, double beta2,
+                  float eps, float weight_decay, const int64_t* d_step, float grad_scale, void* stream);
+
+/* idl_rmsprop_allreduce_step with the SGD / Adam update: the same NVLink reduction and broadcast, the same argument rules (the
+ * state buffers hold n_total / world floats each and are 16-byte aligned), the gradient mean taking the place of grad * grad_scale. */
+int idl_sgd_allreduce_step(const uint64_t* h_grad_peers, const uint64_t* h_param_peers, uint64_t grad_multicast, uint64_t param_multicast,
+                           float* d_momentum_buf, int64_t n_total, int rank, int world, float lr, float momentum, float weight_decay,
+                           const int64_t* d_step, void* stream);
+int idl_adam_allreduce_step(const uint64_t* h_grad_peers, const uint64_t* h_param_peers, uint64_t grad_multicast, uint64_t param_multicast,
+                            float* d_exp_avg, float* d_exp_avg_sq, int64_t n_total, int rank, int world, float lr, double beta1, double beta2, float eps,
+                            float weight_decay, const int64_t* d_step, void* stream);
+
 /* F1 — FASTA ingest on the host (SURVEY §8f rank 1).  Replaces the record loop of kmersFasta
  * (idelucs/utils.py:229-261), which the reference re-runs on every pass (n_mimics + 1 times per training run,
  * once more per predict): '#' lines skipped (:230); a '>' line closes the running record only while its id is
