@@ -1581,6 +1581,11 @@ static int profiles_impl(const ProfCall& c) {
     if (c.n_items <= 0) return IDL_OK;
     // (canonical rows are written one element at a time: any stride)
     if (c.out_stride % 4 != 0 && !is_canon(c.out_kind)) return set_error(IDL_EINVAL, "idl_profiles: out_stride must be a multiple of 4%s", "");
+    if (!is_canon(c.out_kind)) {   // every kernel writes these rows as 16-byte vectors: a misaligned row would fault
+        bool aligned = ((uintptr_t)c.out & 15) == 0;
+        for (int s = 0; s < c.S && aligned; ++s) aligned = (c.out_off[s] & 3) == 0;
+        if (!aligned) return set_error(IDL_EINVAL, "idl_profiles: d_out must be 16-byte aligned and out_off multiples of 4%s", "");
+    }
 
     HostPlan hp;
     ProfParams p;
@@ -1629,9 +1634,8 @@ static int profiles_impl(const ProfCall& c) {
                  c.n_variants <= PC_MAXS && c.n_items >= 2LL * sm_count() && c.prep_size >= prep_bytes(c.n_items);
     if (pc_ok) {
         if (hp.has_explicit || !hp.randn_small || hp.n_bern > PC_DENSE || hp.n_ent > PC_LIST || hp.n_ent * PC_K > PC_REM) pc_ok = false;
-        // TMA bulk copies: 16-byte aligned rows
-        if (((uintptr_t)c.out & 15) || (c.out_stride & 3) || ((uintptr_t)c.codes & 15) || ((uintptr_t)c.nmask & 15) || ((uintptr_t)c.prep & 15)) pc_ok = false;
-        for (int v = 0; v < c.S && pc_ok; ++v) if (c.out_off[v] & 3) pc_ok = false;
+        // TMA bulk copies: 16-byte aligned sources (the output rows are, checked above)
+        if (((uintptr_t)c.codes & 15) || ((uintptr_t)c.nmask & 15) || ((uintptr_t)c.prep & 15)) pc_ok = false;
     }
     if (pc_ok) {
         p.prep = const_cast<void*>(c.prep);

@@ -182,7 +182,9 @@ def profiles(seqset, k, variants, out_kind=OUT_FREQ_F32, seed=0, out=None, out_o
              accumulate=False, status=None, prepared=None, chunked=None, max_long=None, cta_cap=0):
     """Run K2+K3.  Default output: tensor [S, n_items, 4^k] (variant-major) of the out_kind's
     dtype; [S, n_items, R] (R = canonical_width(k)) for the canonical kinds OUT_CANON_*.  See
-    include/idelucs_b200.h::idl_profiles for the argument meaning.  ``prepared`` (from ``prepare`` with the
+    include/idelucs_b200.h::idl_profiles for the argument meaning.  The standardised kinds equal IEEE float32 division by
+    ``scale`` when every scale is a finite, normal float (``Scaler`` guarantees that for frequency columns); a zero or
+    infinite scale, or a subnormal one whose reciprocal overflows, gives NaN instead.  ``prepared`` (from ``prepare`` with the
     same SeqSet / variants / seed / seq_id0) routes float32 outputs through idl_profiles_prepared (k = 6 fast path).  Sets with
     sequences of >= 65 536 bases go through idl_profiles_chunked (k = 6; chunked=False forces the generic kernel).  ``cta_cap`` > 0
     caps the generic kernel at that many CTAs per SM (room for a concurrent stream)."""

@@ -54,7 +54,10 @@ enum {
 enum {
     IDL_OUT_COUNTS_I32 = 0, /* raw window counts, no pseudocount (kmers.pyx:2-50) */
     IDL_OUT_FREQ_F32 = 1,   /* float32((count+pc)/sum)  (utils.py:242-250 then :353 astype) */
-    IDL_OUT_STD_F32 = 2,    /* (freq32 - mean32) / scale32  (utils.py:358-366 via sklearn) */
+    IDL_OUT_STD_F32 = 2,    /* (freq32 - mean32) / scale32  (utils.py:358-366 via sklearn): IEEE float32 division (subnormal quotients
+                             * included) when every scale32 is a finite, normal float, which idl_scaler_finalize guarantees for
+                             * frequency columns.  A zero or infinite scale, or a subnormal one whose reciprocal overflows, gives
+                             * NaN where IEEE division gives +-inf, 0 or a finite quotient */
     IDL_OUT_FREQ_F64 = 3,   /* float64 (count+pc)/sum  (utils.py:250) */
     /* canonical k-mer rows of kmersFasta(reduce=True) (utils.py:246-250): R = idl_revcomp_canonical(k) columns in its order;
      * each value is 8 + the matching frequency kind */
@@ -106,7 +109,8 @@ size_t idl_profiles_workspace_bytes(void);
  * Work items: n_items; item w processes sequence d_sidx[w] (or w when d_sidx is NULL) and,
  * for s in [0, S): variant slot d_sel[w*S+s] (or s when d_sel is NULL; then S must equal
  * n_variants).  Row (s, w) of the output is written at element offset
- * out_off[s] + w*out_stride of d_out (elements of the out_kind's type; multiples of 4).
+ * out_off[s] + w*out_stride of d_out (elements of the out_kind's type; multiples of 4 and d_out 16-byte aligned: rows are
+ * written as 16-byte vectors, IDL_EINVAL otherwise).
  * The RNG sequence id of an item is seq_id0 + its sequence index.
  * d_edit_off / d_edits: CSR edit lists for IDL_KIND_EXPLICIT variants (entry = pos<<3 | val,
  * val 0..3 = set A/C/G/T, 4 = set N; position-sorted and unique per list; positions < 2^29, which also bounds the length of
@@ -159,7 +163,9 @@ int idl_profile_stats(const uint32_t* d_codes, const uint32_t* d_nmask, const in
  * variants, seed and pseudocount: its k = 6 producer/consumer kernel loads the prepared deltas instead of generating the
  * mutations again.  The buffer carries a stamp of what it was prepared for; on a mismatch (or for the few items the prepare
  * pass flags: longer than 20 480 bases, on-chip list overflows) the generic kernel computes the rows — results are identical
- * either way.  d_status int32[n_items] must be zero on entry of each call and is zero again afterwards. */
+ * either way.  The stamp identifies the sequences and the items by address (d_codes, d_sidx), not by content: rewriting
+ * the packed sequences or the item list in place between the two calls is not noticed.  d_status int32[n_items] must be
+ * zero on entry of each call and is zero again afterwards. */
 size_t idl_prepare_bytes(int64_t n_items);
 int idl_profiles_prepare(const uint32_t* d_codes, const uint32_t* d_nmask, const int64_t* d_chunk_off, const int32_t* d_len,
                          int64_t n_seqs_total, const int32_t* d_sidx, int64_t n_items, int64_t seq_id0, int k,

@@ -55,6 +55,7 @@ POINTERS = set("codes nmask chunk_off len sidx sel edit_off edits out mean scale
 NULL = "idl_profiles: null pointer"
 WS_SMALL = "idl_profiles: workspace too small (need {ws} bytes)"
 CUDA = "<cuda>"   # any CUDA runtime error: the request got past validation
+ALIGN = "idl_profiles: d_out must be 16-byte aligned and out_off multiples of 4"
 
 # (id, entry point, arguments that differ from BASE / PER_ENTRY, (return code, error text or CUDA or None))
 CASES = [
@@ -95,6 +96,10 @@ CASES = [
     ("n_items_negative", "idl_profiles", dict(n_items=-5, out_stride=3), (OK, None)),
     ("n_items_0_still_checks_k", "idl_profiles", dict(n_items=0, k=7), (EUNSUPPORTED, "idl_profiles: k must be in 1..6 (got 7)")),
     ("out_stride_not_multiple_of_4", "idl_profiles", dict(out_stride=4098), (EINVAL, "idl_profiles: out_stride must be a multiple of 4")),
+    ("out_misaligned", "idl_profiles", dict(out=68), (EINVAL, ALIGN)),
+    ("out_8_aligned_f64", "idl_profiles", dict(out=72, out_kind=FREQ_F64), (EINVAL, ALIGN)),
+    ("out_off_not_multiple_of_4", "idl_profiles", dict(out_off=[0, 0, 2, 0]), (EINVAL, ALIGN)),
+    ("out_off_multiple_of_4", "idl_profiles", dict(out_off=[4, 8, 12, 4096]), (ECUDA, CUDA)),
     ("bad_kind_6", "idl_profiles", dict(variants=[(CLEAN, 0.0, 0.0, 0), (6, 0.0, 0.0, 0)]), (EINVAL, "idl_profiles: bad variant kind 6")),
     ("bad_kind_negative", "idl_profiles", dict(variants=[(-1, 0.0, 0.0, 0)]), (EINVAL, "idl_profiles: bad variant kind -1")),
     ("p1_above_1", "idl_profiles", dict(variants=[(TRANSITION, 1.5, 0.0, 0)]), (EINVAL, "idl_profiles: p1 out of range")),
@@ -122,6 +127,7 @@ CASES = [
     ("accumulate_freq", "idl_profiles_chunked", dict(accumulate=1), (EINVAL, "idl_profiles: accumulate only for counts")),
     ("bad_kind", "idl_profiles_chunked", dict(variants=[(9, 0.0, 0.0, 0)]), (EINVAL, "idl_profiles: bad variant kind 9")),
     ("n_items_0", "idl_profiles_chunked", dict(n_items=0), (OK, None)),
+    ("out_misaligned", "idl_profiles_chunked", dict(out=84, out_kind=COUNTS_I32), (EINVAL, ALIGN)),
 
     ("valid", "idl_profiles_prepared", {}, (ECUDA, CUDA)),
     ("valid_std", "idl_profiles_prepared", dict(out_kind=STD_F32, mean=DEV, scale=DEV), (ECUDA, CUDA)),
@@ -135,6 +141,8 @@ CASES = [
     ("std_without_scale", "idl_profiles_prepared", dict(out_kind=STD_F32, mean=DEV), (EINVAL, "idl_profiles: mean/scale required")),
     ("explicit", "idl_profiles_prepared", dict(variants=[(EXPLICIT, 0.0, 0.0, 0)]), (EINVAL, "idl_profiles: explicit variant without edit lists")),
     ("n_items_0", "idl_profiles_prepared", dict(n_items=0), (OK, None)),
+    ("out_misaligned", "idl_profiles_prepared", dict(out=68), (EINVAL, ALIGN)),
+    ("out_off_not_multiple_of_4", "idl_profiles_prepared", dict(out_off=[0, 0, 0, 4098]), (EINVAL, ALIGN)),
 
     ("valid", "idl_profiles_prepare", {}, (ECUDA, CUDA)),
     ("valid_without_statistics", "idl_profiles_prepare", dict(partials=None, part_n=None, max_parts=0, n_parts=None), (ECUDA, CUDA)),
