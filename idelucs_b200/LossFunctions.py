@@ -138,6 +138,91 @@ def train_losses_and_grads(z, h, lamb, weight, temperature=0.85, EPS=sys.float_i
     return loss, dz, dh
 
 
+class GlobalBatchLoss(object):
+    """train_losses_and_grads of the GLOBAL batch for one rank of a data-parallel step: W ranks of b pairs each, the loss of the
+    B = W b pairs together (idelucs/models.py:128 on the batch one GPU would train on), the gradients of this rank's rows.
+
+    Global row order: [true rows of rank 0 .. W-1 ; modified rows of rank 0 .. W-1].  Two buffers per rank are read by the others:
+      send1 = [S2_r = z1_r^T z2_r + its transpose (C x C, padded to 4) | fn_r, the normalised latent [2b, D]]
+      send2 = [G_r^T fn_r [2B, D] | the 2b row losses of InfoNCE (padded to 4)]
+    ``set_peers`` gives the device addresses of every rank's send1 / send2 (symmetric memory, or the slots of all-gathered copies).
+    A step is ``stage1(z, h)`` (writes send1), exchange, ``stage2()`` (writes send2), exchange, ``stage3()`` -> (loss, dz, dh).
+    The loss is the same on every rank; dz and dh are multiplied by W, because the optimiser averages the ranks' gradients and the
+    update must be that of the gradient of the global loss.  All cross-rank sums run in rank order (no float atomics)."""
+
+    def __init__(self, rank, world, b, C, D, device, lamb, weight, temperature=0.85, EPS=sys.float_info.epsilon, send=None):
+        self.rank, self.world, self.b, self.C, self.D = rank, world, b, C, D
+        self.lamb, self.weight, self.temperature, self.EPS = lamb, weight, temperature, EPS
+        B = world * b
+        self.n_s2 = C * C + (-C * C) % 4
+        self.len1, self.len2 = self.buffer_sizes(world, b, C, D)
+        f32 = dict(dtype=torch.float32, device=device)
+        self.send1, self.send2 = send if send is not None else (torch.zeros(self.len1, **f32), torch.zeros(self.len2, **f32))
+        assert self.send1.numel() >= self.len1 and self.send2.numel() >= self.len2
+        self.s2 = self.send1[:C * C]
+        self.fn = self.send1[self.n_s2:self.n_s2 + 2 * b * D].view(2 * b, D)
+        self.prod = self.send2[:2 * B * D].view(2 * B, D)
+        self.rowloss = self.send2[2 * B * D:2 * B * D + 2 * b]
+        self.inv_norm = torch.empty(2 * b, **f32)
+        self.fn_all = torch.empty((2 * B, D), **f32)
+        self.ws = torch.empty(_lib.load().idl_iid_loss_workspace_bytes(C), dtype=torch.uint8, device=device)
+
+    @staticmethod
+    def buffer_sizes(world, b, C, D):
+        """floats of send1 and send2 (each a multiple of 4, so that slots of an all-gathered copy stay 16-byte aligned)"""
+        return C * C + (-C * C) % 4 + 2 * b * D + (-2 * b * D) % 4, 2 * world * b * D + 2 * b + (-2 * b) % 4
+
+    def set_peers(self, addr1, addr2):
+        """device addresses (ints, rank order) at which this process reads every rank's send1 / send2"""
+        W = self.world
+        self._p_s2 = (ctypes.c_uint64 * W)(*addr1)
+        self._p_fn = (ctypes.c_uint64 * W)(*[a + 4 * self.n_s2 for a in addr1])
+        self._p_prod = (ctypes.c_uint64 * W)(*addr2)
+
+    def stage1(self, z, h):
+        """this rank's partial joint and normalised latent into send1"""
+        lib = _lib.load()
+        b, C = self.b, self.C
+        self._z = z.detach().contiguous().float()
+        hh = h.detach().contiguous().float()
+        with torch.cuda.device(hh.device):
+            st = _lib.stream_ptr()
+            _lib.check(lib.idl_iid_partial_s2(_lib.ptr(self._z[:b]), _lib.ptr(self._z[b:]), b, C, _lib.ptr(self.s2), st))
+            _lib.check(lib.idl_nce_normalize(_lib.ptr(hh), 2 * b, self.D, _lib.ptr(self.fn), _lib.ptr(self.inv_norm), st))
+
+    def stage2(self):
+        """(every rank's send1 readable) fn_all, this rank's row block of the similarity -> (1 - w) W G_r, its local term
+        G_r fn_all, and G_r^T fn_r with the row losses into send2"""
+        lib = _lib.load()
+        b, D, W = self.b, self.D, self.world
+        with torch.cuda.device(self.fn.device):
+            st = _lib.stream_ptr()
+            _lib.check(lib.idl_nce_gather_rows(self._p_fn, W, b, D, _lib.ptr(self.fn_all), st))
+            sim = torch.mm(self.fn, self.fn_all.t())   # [2b, 2B]: this rank's rows only
+            _lib.check(lib.idl_nce_softmax_xent_rows(_lib.ptr(sim), b, self.rank, W, float(self.temperature), float((1.0 - self.weight) * W),
+                                                     _lib.ptr(self.rowloss), st))
+            self._local = torch.mm(sim, self.fn_all)
+            torch.mm(sim.t(), self.fn, out=self.prod)
+
+    def stage3(self):
+        """(every rank's send2 readable) (loss, dz, dh) of this rank's rows"""
+        lib = _lib.load()
+        b, C, D, W = self.b, self.C, self.D, self.world
+        dev = self.fn.device
+        nce = torch.empty((), dtype=torch.float32, device=dev)
+        loss = torch.empty((), dtype=torch.float32, device=dev)
+        dh = torch.empty((2 * b, D), dtype=torch.float32, device=dev)
+        dz = torch.empty_like(self._z)
+        with torch.cuda.device(dev):
+            st = _lib.stream_ptr()
+            _lib.check(lib.idl_nce_normalize_backward_global(_lib.ptr(self._local), 1, self._p_prod, W, _lib.ptr(self.fn), _lib.ptr(self.inv_norm),
+                                                             b, D, self.rank, _lib.ptr(dh), _lib.ptr(nce), st))
+            _lib.check(lib.idl_iid_global_finish(self._p_s2, W, _lib.ptr(self._z[:b]), _lib.ptr(self._z[b:]), b, C, float(self.lamb), float(self.EPS),
+                                                 float(self.weight * W), float(self.weight), _lib.ptr(nce), float(1.0 - self.weight), _lib.ptr(loss),
+                                                 _lib.ptr(dz[:b]), _lib.ptr(dz[b:]), _lib.ptr(self.ws), self.ws.numel(), st))
+        return loss, dz, dh
+
+
 class _InfoNCE(torch.autograd.Function):
     """fused CUDA form: value and gradient with respect to the stacked latent, computed together in the forward"""
 

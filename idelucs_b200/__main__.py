@@ -4,7 +4,8 @@ majority vote over voters (k-means on one-hot votes, utils.py:582-602) or HDBSCA
 --n_clusters=0 (the ``hdbscan`` package if importable, else scikit-learn's algorithm with its all-pairs work on the GPU,
 ``hdbscan.hdbscan_device``), metrics (silhouette on the GPU, ``metrics.silhouette_score_device``) and TSV output:
 assignments.tsv and metrics.tsv under Results/<fasta stem>/<time>/.  ``--gpus N`` (N >= 2) trains data-parallel on N GPUs with
-train.ShardedTrainer's graph-captured step (run_gpus); the tail is the same."""
+train.ShardedTrainer's graph-captured step (run_gpus), with --global_batch_loss on the losses of the global batch; the tail is the
+same."""
 import argparse
 import os
 import sys
@@ -158,7 +159,7 @@ def _rank_main(rank, world, port, args):
     steps = -(-(len(ft.mimic_schedule(args["n_mimics"])) - 1) * n_total // args["batch_sz"])
     tr = ShardedTrainer(ss, k=args["k"], n_clusters=n_clusters, n_mimics=args["n_mimics"], batch_sz=args["batch_sz"] // world,
                         lamb=args["lambda"], weight=args["weight"], lr=args["lr"], seed=0, seq_id0=lo, world=world,
-                        optimizer=args["optimizer"])
+                        optimizer=args["optimizer"], global_batch_loss=args.get("global_batch_loss", False))
     tr.enable_cuda_graph()
     tr.reset_optimizer()   # (the capture's warm-up steps trained the network: start from a fresh optimiser)
     predictions, latent = [], None
@@ -206,8 +207,12 @@ def main(argv=None):
     parser.add_argument("--plot", action="store", type=bool, default=False)
     parser.add_argument("--gpus", action="store", type=int, default=argparse.SUPPRESS,
                         help="train data-parallel on this many GPUs (default 1); --batch_sz stays the global batch")
+    parser.add_argument("--global_batch_loss", action="store_true", default=argparse.SUPPRESS,
+                        help="with --gpus N >= 2: evaluate both losses on the global batch (the ranks exchange the IIC joint and the "
+                             "InfoNCE latents), as one GPU does, instead of on each GPU's batch_sz / N pairs")
     args = vars(parser.parse_args(argv))
     gpus = args.pop("gpus", 1)
+    global_batch_loss = args.pop("global_batch_loss", False)   # (one GPU already trains on the global batch)
     print("\nTraining Parameters:")
     for key in args:
         print(f"{key} \t -> {args[key]}")
@@ -231,6 +236,9 @@ def main(argv=None):
     if gpus > torch.cuda.device_count():
         parser.error(f"--gpus {gpus}: only {torch.cuda.device_count()} CUDA devices are visible")
     print(f"gpus \t -> {gpus}")
+    if global_batch_loss:
+        print("global_batch_loss \t -> True")
+        args["global_batch_loss"] = True
     run_gpus(args, gpus)
 
 

@@ -66,6 +66,13 @@ PROTOTYPES = {
     "idl_nce_softmax_xent_scaled": (c_int, [c_void_p, c_int, c_float, c_float, c_void_p, c_void_p, c_void_p, c_void_p]),
     "idl_nce_normalize_backward": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_void_p, c_void_p]),
     "idl_nce_normalize_backward_parts": (c_int, [c_void_p, c_int, c_void_p, c_void_p, c_int, c_int, c_void_p, c_void_p]),
+    "idl_iid_partial_s2": (c_int, [c_void_p, c_void_p, c_int, c_int, c_void_p, c_void_p]),
+    "idl_iid_global_finish": (c_int, [c_void_p, c_int, c_void_p, c_void_p, c_int, c_int, c_float, c_float, c_float, c_float, c_void_p, c_float,
+                                      c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]),
+    "idl_nce_gather_rows": (c_int, [c_void_p, c_int, c_int, c_int, c_void_p, c_void_p]),
+    "idl_nce_softmax_xent_rows": (c_int, [c_void_p, c_int, c_int, c_int, c_float, c_float, c_void_p, c_void_p]),
+    "idl_nce_normalize_backward_global": (c_int, [c_void_p, c_int, c_void_p, c_int, c_void_p, c_void_p, c_int, c_int, c_int, c_void_p, c_void_p,
+                                                  c_void_p]),
     "idl_relu_dropout_forward": (c_int, [c_void_p, c_int, c_void_p, c_i64, c_int, c_float, c_u64, c_void_p, ctypes.c_uint32, c_void_p, c_void_p]),
     "idl_relu_dropout_backward": (c_int, [c_void_p, c_void_p, c_i64, c_float, c_void_p, c_void_p]),
     "idl_sum_parts_bias": (c_int, [c_void_p, c_int, c_void_p, c_i64, c_int, c_void_p, c_void_p]),

@@ -923,6 +923,190 @@ static int iid_loss_small_launch(const float* d_z1, const float* d_z2, int B, in
     return IDL_OK;
 }
 
+// ---------------------------------------------------------------------------------------------------------------
+// Global-batch losses of the data-parallel step: W ranks of b pairs each train on the loss of the B = W b pairs together.  The
+// global stacked batch is [true rows of rank 0 .. W-1 ; modified rows of rank 0 .. W-1]: rank r's local row q is global row
+// r b + q (q < b) or B + r b + (q - b).  What one rank needs of the others is read through peer addresses (symmetric memory, or
+// the slots of an all-gathered tensor), always summed in rank order, so every rank computes the same bits without float atomics.
+// ---------------------------------------------------------------------------------------------------------------
+__device__ __forceinline__ int global_row(int q, int b, int rank, int B) { return q < b ? rank * b + q : B + rank * b + (q - b); }
+
+// s + element i of every rank's buffer, added in rank order.  The table is indexed with compile-time ranks only, so the kernel
+// parameter is not copied to local memory.
+__device__ __forceinline__ float rank_order_sum(const PeerPtrs& t, int world, size_t i, float s) {
+#pragma unroll
+    for (int r = 0; r < MAX_PEERS; ++r)
+        if (r < world) s += t.p[r][i];
+    return s;
+}
+
+// IIC, C <= 16: S2 = sum over the ranks' partials S2_r (rank order), the C x C algebra of iid_loss_small_kernel on it, and this
+// rank's gradients dz1 = z2 dS, dz2 = z1 dS — ONE CTA, thread <-> joint entry
+constexpr int IG_NT = 512;
+__global__ void __launch_bounds__(IG_NT) iid_global_small_kernel(const PeerPtrs s2, int world, const float* __restrict__ z1, const float* __restrict__ z2,
+                                                                 int B, int C, float lamb, float eps, float gscale, float loss_w,
+                                                                 const float* __restrict__ add, float add_w, float* __restrict__ loss,
+                                                                 float* __restrict__ dz1, float* __restrict__ dz2) {
+    __shared__ float Pm[IS_MAXC][IS_MAXC + 1], dS[IS_MAXC][IS_MAXC + 1];
+    __shared__ float marg[IS_MAXC], gvec[IS_MAXC];
+    __shared__ float red[IG_NT / 32][2];
+    __shared__ float sT, sgp;
+    const int tid = threadIdx.x, lane = tid & 31, w = tid >> 5;
+    const int np = C * C;
+    const int pi = tid < np ? tid / C : 0, pj = tid < np ? tid - pi * C : 0;
+    float ssym = 0.f;
+    if (tid < np) {
+        ssym = 0.5f * rank_order_sum(s2, world, tid, 0.f);   // (S + S^T) / 2 (LossFunctions.py:59)
+    }
+    const float t = warp_total(ssym);
+    if (lane == 0) red[w][0] = t;
+    __syncthreads();
+    if (tid == 0) { float T = 0.f; for (int g = 0; g < IG_NT / 32; ++g) T += red[g][0]; sT = T; }
+    __syncthreads();
+    const float T = sT;
+    const float P = ssym / T;   // normalise (:60)
+    if (tid < np) Pm[pi][pj] = P;
+    __syncthreads();
+    if (tid < C) {   // marginals before clamping, the clamp's correction (:28-38)
+        float m = 0.f, c = 0.f;
+        for (int j = 0; j < C; ++j) { const float v = Pm[tid][j]; m += v; if (v < eps) c += eps - v; }
+        marg[tid] = m;
+        gvec[tid] = m < eps ? 0.f : lamb * (m + c) / m;
+    }
+    __syncthreads();
+    float term = 0.f, A = 0.f;
+    if (tid < np) {   // clamp, entropy terms (:36-44) and the pieces of the gradient
+        const bool cl = P < eps;
+        const float Pc = cl ? eps : P;
+        const float mi = marg[pi], mj = marg[pj];
+        const float inner = logf(Pc) - lamb * logf(mj < eps ? eps : mj) - lamb * logf(mi < eps ? eps : mi);
+        term = -Pc * inner;
+        A = cl ? 0.f : (-inner - 1.f);
+    }
+    const float tt = warp_total(term), ap = warp_total(A * P);
+    if (lane == 0) { red[w][0] = tt; red[w][1] = ap; }
+    __syncthreads();
+    if (tid == 0) {
+        float l = 0.f, gp = 0.f;
+        for (int g = 0; g < IG_NT / 32; ++g) { l += red[g][0]; gp += red[g][1]; }
+        for (int i = 0; i < C; ++i) gp += 2.f * gvec[i] * marg[i];
+        if (loss) *loss = add ? loss_w * l + add_w * (*add) : loss_w * l;
+        sgp = gp;
+    }
+    __syncthreads();
+    if (tid < np) dS[pi][pj] = gscale * (A + gvec[pi] + gvec[pj] - sgp) / T;   // dL/dSsym (symmetric), times the caller's weight
+    __syncthreads();
+    for (int q = tid; q < B * C; q += IG_NT) {
+        const int b = q / C, c = q - b * C;
+        float a1 = 0.f, a2 = 0.f;
+        for (int j = 0; j < C; ++j) {
+            const float d = dS[c][j];
+            a1 = fmaf(z2[(size_t)b * C + j], d, a1);
+            a2 = fmaf(z1[(size_t)b * C + j], d, a2);
+        }
+        if (dz1) dz1[q] = a1;
+        if (dz2) dz2[q] = a2;
+    }
+}
+
+// IIC, C > 16: S2 = sum over the ranks' partials (rank order) into the workspace, for idl_iid_joint_algebra
+__global__ void __launch_bounds__(256) iid_s2_sum_kernel(const PeerPtrs s2, int world, int n, float* __restrict__ out) {
+    const int i = blockIdx.x * 256 + threadIdx.x;
+    if (i >= n) return;
+    out[i] = rank_order_sum(s2, world, i, 0.f);
+}
+
+// fn of every rank ([2b, D] each, local row order) -> fn_all [2B, D] in global row order
+__global__ void __launch_bounds__(256) nce_gather_rows_kernel(const PeerPtrs fn, int b, int B, int D, float* __restrict__ out) {
+    const long long n = 2LL * B * D;
+    for (long long idx = (long long)blockIdx.x * 256 + threadIdx.x; idx < n; idx += (long long)gridDim.x * 256) {
+        const int g = (int)(idx / D), d = (int)(idx - (long long)g * D);
+        const int side = g >= B ? 1 : 0, rem = g - side * B;
+        const int r = rem / b, q = rem - r * b + side * b;
+        const float* src = fn.p[0];
+#pragma unroll
+        for (int k = 1; k < MAX_PEERS; ++k)
+            if (k == r) src = fn.p[k];
+        out[idx] = src[(size_t)q * D + d];
+    }
+}
+
+// Row block [2b, 2B] of the global similarity (rows: this rank's, columns: fn_all) -> in place grad_scale G_r with
+// G = (P - Y) / (2B T): P_ij = exp(S_ij / T - lse_i) for j != i (0 on the global diagonal), Y the positive pairs.  The whole
+// gradient of the global InfoNCE is (G + G^T) fn, i.e. the W of nce_weights_kernel, split by rows.  rowloss[q] = lse - S_pos / T.
+// Warp <-> row; |S / T| <= 1 / T, so exp needs no running maximum (as nce_lse_kernel).
+__global__ void __launch_bounds__(NCE_NT) nce_rows_kernel(float* __restrict__ S, int b, int rank, int B, float inv_t, float c,
+                                                          float* __restrict__ rowloss) {
+    const int lane = threadIdx.x & 31;
+    const int q = blockIdx.x * NCE_RB + (threadIdx.x >> 5);
+    if (q >= 2 * b) return;
+    const int n = 2 * B;
+    const int gi = global_row(q, b, rank, B);
+    const int pos = gi < B ? gi + B : gi - B;
+    float* row = S + (size_t)q * n;
+    float sum = 0.f;
+    for (int j = lane; j < n; j += 32)
+        if (j != gi) sum += __expf(row[j] * inv_t);
+    sum = warp_total(sum);   // (xor tree: every lane holds the same bits)
+    const float lse = logf(sum);
+    if (lane == 0) rowloss[q] = lse - row[pos] * inv_t;
+    __syncwarp();
+    for (int j = lane; j < n; j += 32) {
+        float v = 0.f;
+        if (j != gi) {
+            v = __expf(row[j] * inv_t - lse);
+            if (j == pos) v -= 1.f;
+        }
+        row[j] = c * v;
+    }
+}
+
+// dh of this rank's rows through F.normalize: dfn = (sum of the local parts G_r fn_all, index order) + (sum over the ranks, rank
+// order, of row gi of G_r'^T fn_r'); dh = inv_norm (dfn - fn (fn . dfn)).  Block 0 also writes the global InfoNCE loss: the ranks'
+// row losses (stored behind each product) summed rank by rank, over 2B.
+__global__ void __launch_bounds__(NCE_NT) nce_normalize_backward_global_kernel(const float* __restrict__ parts, int n_parts, const PeerPtrs prod,
+                                                                                int world, const float* __restrict__ fn,
+                                                                                const float* __restrict__ inv_norm, int b, int D, int rank,
+                                                                                float* __restrict__ dh, float* __restrict__ loss) {
+    const int lane = threadIdx.x & 31;
+    const int q = blockIdx.x * NCE_RB + (threadIdx.x >> 5);
+    const int B = world * b;
+    if (blockIdx.x == 0 && threadIdx.x < 32 && loss) {
+        const size_t off = (size_t)2 * B * D;
+        float tot = 0.f;
+#pragma unroll
+        for (int r = 0; r < MAX_PEERS; ++r) {
+            if (r >= world) break;
+            float t = 0.f;
+            for (int i = lane; i < 2 * b; i += 32) t += prod.p[r][off + i];
+            tot += warp_total(t);
+        }
+        if (lane == 0) *loss = tot / (float)(2 * B);
+    }
+    if (q >= 2 * b) return;
+    const int gi = global_row(q, b, rank, B);
+    const size_t part = (size_t)2 * b * D;
+    const float inv = inv_norm[q];
+    float g[4];
+    float dot = 0.f;
+#pragma unroll
+    for (int k = 0; k < 4; ++k) {
+        const int d = lane + 32 * k;
+        g[k] = 0.f;
+        if (d < D) {
+            for (int p = 0; p < n_parts; ++p) g[k] += parts[p * part + (size_t)q * D + d];
+            g[k] = rank_order_sum(prod, world, (size_t)gi * D + d, g[k]);
+            dot = fmaf(fn[(size_t)q * D + d], g[k], dot);
+        }
+    }
+    dot = warp_total(dot);
+#pragma unroll
+    for (int k = 0; k < 4; ++k) {
+        const int d = lane + 32 * k;
+        if (d < D) dh[(size_t)q * D + d] = inv * (g[k] - fn[(size_t)q * D + d] * dot);
+    }
+}
+
 }  // namespace idl
 
 using namespace idl;
@@ -1174,6 +1358,97 @@ int idl_adam_allreduce_step(const uint64_t* h_grad_peers, const uint64_t* h_para
     return allreduce_step_launch("idl_adam_allreduce_step", "exp_avg / exp_avg_sq", h_grad_peers, h_param_peers, grad_multicast, param_multicast,
                                  StatePtrs{{d_exp_avg, d_exp_avg_sq}}, n_total, rank, world,
                                  AdamUpdate{lr, eps, weight_decay, beta1, beta2, reinterpret_cast<const long long*>(d_step), 0.f, 0.f, 0.f, 0.f, 0.f}, stream);
+}
+
+// ---- global-batch losses (see the kernels above) ----
+
+// the `world` float buffers of a host peer table; false when one is null or not 4-byte aligned
+static bool peer_floats(const uint64_t* h_peers, int world, PeerPtrs& out) {
+    for (int r = 0; r < MAX_PEERS; ++r) out.p[r] = nullptr;
+    for (int r = 0; r < world; ++r) {
+        if (!h_peers[r] || (h_peers[r] & 3)) return false;
+        out.p[r] = reinterpret_cast<float*>((uintptr_t)h_peers[r]);
+    }
+    return true;
+}
+
+// b rows per rank, world ranks, D columns: 1 <= world <= 16, b >= 1, and the [2B, D] / [2b, 2B] operands indexable with int rows
+static bool bad_rows(int b, int world, int64_t width) { return world < 1 || world > MAX_PEERS || b < 1 || 2LL * b * world * width > INT32_MAX; }
+
+int idl_iid_partial_s2(const float* d_z1, const float* d_z2, int B, int C, float* d_S2, void* stream) {
+    if (!d_z1 || !d_z2 || !d_S2 || B < 1 || C < 1 || C > IID_MAXC)
+        return set_error(IDL_EINVAL, "idl_iid_partial_s2: bad argument%s (B >= 1, 1 <= C <= 256)", "");
+    const int nt = (C + IC_T - 1) / IC_T;
+    iid_s2_kernel<<<nt * (nt + 1) / 2, IC_NT, 0, (cudaStream_t)stream>>>(d_z1, d_z2, B, C, nt, d_S2); note_launch();
+    IDL_CUDA_CHECK(cudaGetLastError());
+    return IDL_OK;
+}
+
+int idl_iid_global_finish(const uint64_t* h_s2_peers, int world, const float* d_z1, const float* d_z2, int B, int C, float lamb, float eps,
+                          float grad_scale, float loss_weight, const float* d_add, float add_weight, float* d_loss, float* d_dz1, float* d_dz2,
+                          void* d_workspace, size_t workspace_bytes, void* stream) {
+    if (!h_s2_peers || !d_z1 || !d_z2 || !d_workspace || world < 1 || world > MAX_PEERS || B < 1 || C < 1 || C > IID_MAXC)
+        return set_error(IDL_EINVAL, "idl_iid_global_finish: bad argument%s (world 1..16, B >= 1, 1 <= C <= 256)", "");
+    if (workspace_bytes < idl_iid_loss_workspace_bytes(C)) return set_error(IDL_EINVAL, "idl_iid_global_finish: workspace too small%s", "");
+    PeerPtrs s2;
+    if (!peer_floats(h_s2_peers, world, s2)) return set_error(IDL_EINVAL, "idl_iid_global_finish: null / misaligned peer pointer%s", "");
+    cudaStream_t st = (cudaStream_t)stream;
+    if (C <= IS_MAXC) {
+        iid_global_small_kernel<<<1, IG_NT, 0, st>>>(s2, world, d_z1, d_z2, B, C, lamb, eps, grad_scale, loss_weight, d_add, add_weight, d_loss, d_dz1,
+                                                     d_dz2); note_launch();
+        IDL_CUDA_CHECK(cudaGetLastError());
+        return IDL_OK;
+    }
+    float* S2 = reinterpret_cast<float*>(d_workspace);
+    float* dS = S2 + (size_t)C * C;
+    float* scratch = dS + (size_t)C * C;
+    const bool grad = d_dz1 || d_dz2;
+    iid_s2_sum_kernel<<<(C * C + 255) / 256, 256, 0, st>>>(s2, world, C * C, S2); note_launch();
+    const int rc = idl_iid_joint_algebra(S2, C, lamb, eps, grad_scale, loss_weight, d_add, add_weight, d_loss, nullptr, grad ? dS : nullptr, scratch,
+                                         stream);
+    if (rc != IDL_OK || !grad) return rc;
+    const int nt = (C + IC_T - 1) / IC_T;
+    iid_dz_kernel<<<dim3((B + IC_BR - 1) / IC_BR, nt, 2), IC_NT, 0, st>>>(d_z1, d_z2, dS, B, C, d_dz1, d_dz2); note_launch();
+    IDL_CUDA_CHECK(cudaGetLastError());
+    return IDL_OK;
+}
+
+int idl_nce_gather_rows(const uint64_t* h_fn_peers, int world, int b, int D, float* d_fn_all, void* stream) {
+    if (!h_fn_peers || !d_fn_all || D < 1 || bad_rows(b, world, D))
+        return set_error(IDL_EINVAL, "idl_nce_gather_rows: bad argument%s (world 1..16, b >= 1, D >= 1, 2 b world D < 2^31)", "");
+    PeerPtrs fn;
+    if (!peer_floats(h_fn_peers, world, fn)) return set_error(IDL_EINVAL, "idl_nce_gather_rows: null / misaligned peer pointer%s", "");
+    const long long n = 2LL * b * world * D;
+    long long grid = (n + 255) / 256;
+    if (grid > 148 * 4) grid = 148 * 4;
+    nce_gather_rows_kernel<<<(unsigned)grid, 256, 0, (cudaStream_t)stream>>>(fn, b, b * world, D, d_fn_all); note_launch();
+    IDL_CUDA_CHECK(cudaGetLastError());
+    return IDL_OK;
+}
+
+int idl_nce_softmax_xent_rows(float* d_sim, int b, int rank, int world, float temperature, float grad_scale, float* d_rowloss, void* stream) {
+    if (!d_sim || !d_rowloss || !(temperature > 0.f) || rank < 0 || rank >= world || bad_rows(b, world, 2LL * b * world))
+        return set_error(IDL_EINVAL, "idl_nce_softmax_xent_rows: bad argument%s (world 1..16, 0 <= rank < world, b >= 1, 4 b^2 world^2 < 2^31)", "");
+    const float inv_t = 1.0f / temperature;
+    const int B = b * world;
+    nce_rows_kernel<<<(2 * b + NCE_RB - 1) / NCE_RB, NCE_NT, 0, (cudaStream_t)stream>>>(d_sim, b, rank, B, inv_t, grad_scale * inv_t / (float)(2 * B),
+                                                                                       d_rowloss); note_launch();
+    IDL_CUDA_CHECK(cudaGetLastError());
+    return IDL_OK;
+}
+
+int idl_nce_normalize_backward_global(const float* d_dfn_parts, int n_parts, const uint64_t* h_prod_peers, int world, const float* d_fn,
+                                      const float* d_inv_norm, int b, int D, int rank, float* d_dh, float* d_loss, void* stream) {
+    if (!d_dfn_parts || !h_prod_peers || !d_fn || !d_inv_norm || !d_dh || n_parts < 1 || D < 1 || D > 128 || rank < 0 || rank >= world ||
+        bad_rows(b, world, D + 1))
+        return set_error(IDL_EINVAL, "idl_nce_normalize_backward_global: bad argument%s (world 1..16, 0 <= rank < world, b >= 1, 1 <= D <= 128)", "");
+    PeerPtrs prod;
+    if (!peer_floats(h_prod_peers, world, prod)) return set_error(IDL_EINVAL, "idl_nce_normalize_backward_global: null / misaligned peer pointer%s", "");
+    nce_normalize_backward_global_kernel<<<(2 * b + NCE_RB - 1) / NCE_RB, NCE_NT, 0, (cudaStream_t)stream>>>(d_dfn_parts, n_parts, prod, world, d_fn,
+                                                                                                           d_inv_norm, b, D, rank, d_dh, d_loss);
+    note_launch();
+    IDL_CUDA_CHECK(cudaGetLastError());
+    return IDL_OK;
 }
 
 }  // extern "C"

@@ -18,7 +18,7 @@ import torch
 import torch.distributed as dist
 
 from . import featurise as ft
-from .LossFunctions import train_losses_and_grads
+from .LossFunctions import GlobalBatchLoss, train_losses_and_grads
 from .PytorchUtils import NetLinear
 from .models import weights_init
 
@@ -173,11 +173,13 @@ class ShardedTrainer(object):
       side stream  pair batch t+1 regenerated from the packed sequences (selection mode of idl_profiles, one CTA per SM) under the
                    small kernels of the middle of the step, the first layer's bias gradient beside its weight-gradient GEMM, the
                    hand-over of the batch beside the optimiser.
-    The parameters of the network are views into one flat buffer, so the optimiser and the collectives see one tensor."""
+    The parameters of the network are views into one flat buffer, so the optimiser and the collectives see one tensor.
+    With several ranks and global_batch_loss=True the losses are those of all ranks' pairs together (_global_losses); by default,
+    and always at one rank, each rank's losses are those of its own batch_sz pairs."""
 
     def __init__(self, seqset, k=6, n_clusters=5, n_mimics=50, batch_sz=512, lamb=2.8, weight=0.25, lr=1e-3, seed=0,
                  seq_id0=0, world=1, materialize_bytes=0, alpha=0.99, eps=1e-8, weight_decay=None, use_symmetric_memory=True,
-                 overlap_featurise_with="forward", optimizer="RMSprop"):
+                 overlap_featurise_with="forward", optimizer="RMSprop", global_batch_loss=False):
         from .utils import PairBatchLoader
         if optimizer not in OPTIMIZERS:
             raise ValueError("optimizer must be one of %s, got %r" % (", ".join(OPTIMIZERS), optimizer))
@@ -203,6 +205,10 @@ class ShardedTrainer(object):
         pad = (-n) % (4 * world)
         self._mode = "single"
         self._flat_param = self._flat_grad = None
+        # global_batch_loss (several ranks): the step's losses are those of the world * batch_sz pairs together, exchanged between
+        # the ranks (LossFunctions.GlobalBatchLoss); at one rank the local batch already is the global one
+        self._gsizes = GlobalBatchLoss.buffer_sizes(world, batch_sz, n_clusters, net.layers[3].out_features) if world > 1 and global_batch_loss else None
+        self._gloss = None
         if world > 1 and use_symmetric_memory:
             try:
                 self._setup_symmetric(n + pad)
@@ -216,6 +222,8 @@ class ShardedTrainer(object):
         if self._mode != "symm":
             self._flat_param = torch.zeros(n + pad, dtype=torch.float32, device=self.dev)
             self._flat_grad = torch.zeros(n + pad, dtype=torch.float32, device=self.dev)
+        if self._gsizes is not None:
+            self._setup_global_loss(batch_sz, n_clusters, net.layers[3].out_features, lamb, weight)
         o = 0
         for p in params:
             self._flat_param[o:o + p.numel()].copy_(p.data.reshape(-1))
@@ -259,6 +267,40 @@ class ShardedTrainer(object):
         mc_g = int(getattr(self._hg, "multicast_ptr", 0) or 0)
         mc_p = int(getattr(self._hp, "multicast_ptr", 0) or 0)
         self._mc = (mc_g, mc_p) if (mc_g and mc_p) else (0, 0)
+        if self._gsizes is not None:   # the two buffers of the global-batch loss every rank reads
+            self._gsend = [symm.empty(n, dtype=torch.float32, device=self.dev) for n in self._gsizes]
+            self._gh = [symm.rendezvous(t, grp) for t in self._gsend]
+            for t in self._gsend:
+                t.zero_()
+
+    def _setup_global_loss(self, b, C, D, lamb, weight):
+        """GlobalBatchLoss of this rank: its send buffers are symmetric memory (peers read them in place after a barrier) or, with
+        NCCL, local tensors all-gathered into one copy per rank"""
+        if self._mode == "symm":
+            gl = GlobalBatchLoss(self.rank, self.world, b, C, D, self.dev, lamb, weight, send=self._gsend)
+            gl.set_peers(*[[int(a) for a in h.buffer_ptrs] for h in self._gh])
+        else:
+            gl = GlobalBatchLoss(self.rank, self.world, b, C, D, self.dev, lamb, weight)
+            self._gathered = [torch.zeros(self.world * n, dtype=torch.float32, device=self.dev) for n in self._gsizes]
+            gl.set_peers(*[[g.data_ptr() + 4 * n * r for r in range(self.world)] for g, n in zip(self._gathered, self._gsizes)])
+        self._gloss = gl
+
+    def _global_losses(self, z, h):
+        """LossFunctions.GlobalBatchLoss's three stages with the exchanges between them: (loss, dz, dh) of this rank's rows.
+        Symmetric memory: one barrier after each rank wrote send1 (partial joint, normalised latent) and one after send2
+        (G_r^T fn_r, row losses); peers then read both in place.  No barrier is needed before a rank overwrites them in the next
+        step: every peer's last read (stage 3) precedes, in its stream order, its arrival at the optimiser's first barrier, and
+        this rank writes again only after passing that barrier.  NCCL: each buffer is all-gathered instead."""
+        gl = self._gloss
+        gl.stage1(z, h)
+        for k, send in enumerate((gl.send1, gl.send2)):
+            if self._mode == "symm":
+                self._gh[k].barrier(channel=0)
+            else:
+                dist.all_gather_into_tensor(self._gathered[k], send)
+            if k == 0:
+                gl.stage2()
+        return gl.stage3()
 
     # ---- optimiser: torch.optim.RMSprop's / SGD's / Adam's arithmetic on flat buffers ----
     def _optimizer_step(self):
@@ -434,7 +476,10 @@ class ShardedTrainer(object):
         z, h = self._tail(d1)
         # (1 - w) InfoNCE + w IIC (models.py:128) and its gradients with respect to z and h straight from the fused kernels (the
         # weights ride inside them); the MLP's backward pass is seeded with those — no framework kernel between forward and backward
-        loss, dz, dh = train_losses_and_grads(z, h, self.lamb, self.weight, 0.85)
+        if self._gloss is not None:
+            loss, dz, dh = self._global_losses(z, h)
+        else:
+            loss, dz, dh = train_losses_and_grads(z, h, self.lamb, self.weight, 0.85)
         self._side.wait_stream(main)          # (the epoch's loss sum: a one-element add beside the backward pass, off the main stream)
         with torch.cuda.stream(self._side):
             self._loss_sum.add_(loss)

@@ -293,6 +293,34 @@ int idl_nce_normalize_backward(const float* d_dfn, const float* d_fn, const floa
 int idl_nce_normalize_backward_parts(const float* d_dfn_parts, int n_parts, const float* d_fn, const float* d_inv_norm, int n2, int D,
                                      float* d_dh, void* stream);
 
+/* Global-batch loss of the data-parallel step: W = world ranks of b pairs each compute (1 - w) InfoNCE + w IIC of the B = W b pairs
+ * together, the loss one GPU computes on the whole batch.  The global stacked batch is [true rows of rank 0 .. W-1 ; modified rows
+ * of rank 0 .. W-1]: local row q of rank r (its own stacked [2b, .] batch) is global row r b + q for q < b, else B + r b + (q - b).
+ * What a rank needs of the others is read through HOST arrays of `world` device addresses (entry r = rank r's buffer: symmetric
+ * memory, or the slots of an all-gathered tensor), always summed in rank order, so every rank computes the same bits.  The caller
+ * synchronises the ranks between writing a buffer and the peers' reads of it.
+ *   idl_iid_partial_s2           d_S2 [C, C] = S + S^T with S = z1^T z2 over this rank's b pairs (fixed order, exactly symmetric)
+ *   idl_iid_global_finish        S2 = sum of the ranks' partials; the IIC loss and this rank's dz1 = z2 dS, dz2 = z1 dS, weighted and
+ *                                combined like idl_iid_loss_scaled.  C <= 16: one kernel; larger C: the sum into the workspace,
+ *                                idl_iid_joint_algebra on it, one contraction kernel.  d_workspace: idl_iid_loss_workspace_bytes(C)
+ *   idl_nce_gather_rows          d_fn_all [2B, D] in global row order from every rank's normalised latent fn [2b, D]
+ *   idl_nce_softmax_xent_rows    d_sim [2b, 2B] = fn fn_all^T on entry (this rank's rows); overwritten IN PLACE by grad_scale G_r,
+ *                                G = (P - Y) / (2B T) (P the self-masked softmax rows, Y the positive pairs, G + G^T = the W of
+ *                                idl_nce_softmax_xent); d_rowloss[2b] = each row's cross-entropy
+ *   idl_nce_normalize_backward_global  dh of this rank's rows: dfn = (sum of n_parts local parts [n_parts, 2b, D] of G_r fn_all) +
+ *                                (row gi of sum over the ranks of G_r'^T fn_r'), then the normalisation's backward.  Every peer
+ *                                buffer holds [2B, D] of G_r'^T fn_r' followed by that rank's 2b row losses; d_loss (optional)
+ *                                receives their sum over 2B, the global InfoNCE loss.  D <= 128.
+ * world <= 16; peer addresses 4-byte aligned. */
+int idl_iid_partial_s2(const float* d_z1, const float* d_z2, int B, int C, float* d_S2, void* stream);
+int idl_iid_global_finish(const uint64_t* h_s2_peers, int world, const float* d_z1, const float* d_z2, int B, int C, float lamb, float eps,
+                          float grad_scale, float loss_weight, const float* d_add, float add_weight, float* d_loss, float* d_dz1, float* d_dz2,
+                          void* d_workspace, size_t workspace_bytes, void* stream);
+int idl_nce_gather_rows(const uint64_t* h_fn_peers, int world, int b, int D, float* d_fn_all, void* stream);
+int idl_nce_softmax_xent_rows(float* d_sim, int b, int rank, int world, float temperature, float grad_scale, float* d_rowloss, void* stream);
+int idl_nce_normalize_backward_global(const float* d_dfn_parts, int n_parts, const uint64_t* h_prod_peers, int world, const float* d_fn,
+                                      const float* d_inv_norm, int b, int D, int rank, float* d_dh, float* d_loss, void* stream);
+
 /* ReLU + Dropout(p) of the encoder (idelucs/PytorchUtils.py:36-44) fused with the tail of the Linear before it, one pass each way.
  * forward: v = sum over the n_parts partial products d_parts[n_parts, M, N] (n_parts = 1: a plain activation matrix) + d_bias[N]
  * (NULL: none); d_out = (v > 0 and kept) ? v / (1 - p) : 0.  The keep decision of an element in training step *d_step (device
